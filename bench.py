@@ -7,6 +7,7 @@
                                                                  else the oracle port), same metric / config
   python bench.py --workload amazon                              BASELINE configs[3] shape (133 table rows, 1 image, 70 tokens)
   python bench.py --workload generate                            BASELINE configs[4]: beam-4 generation, 64 businesses
+  python bench.py --dump-outputs DIR                             also write what the last timed step computed to DIR/*.npy
 
 Default workload = BASELINE.json configs[1]: one step = forward + backward (+ bucketed gradient all-reduce when N > 1)
 + fused clip/AdamW of `MultimodalSum.forward` over 16 synthetic Yelp-shaped businesses per GPU (9 reviews x 128-token frame
@@ -45,7 +46,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the Amazon / generation workloads appended to the default run")
     ap.add_argument("--cpu-seconds", type=float, default=240.0, help="time budget of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy: training workloads "
+                         "loss, grads and params (fixed per-tensor samples, see sampled_parameters); generate generated_ids")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs records the CUDA path (--impl b200)")
     a.workload = a.workload or a.dataset or "yelp"
     if a.businesses is None:
         a.businesses = 64 if a.workload == "generate" else 16
@@ -117,14 +125,6 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------ reference arm / cpu baseline
-def _reference_tree():
-    """The unmodified reference, when a copy is reachable (the build container; never on the GPU box)."""
-    for cand in (os.environ.get("MMSUM_REF"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.isdir(os.path.join(cand, "src", "transformer")):
-            return cand
-    return None
-
-
 def cpu_reference_steps(steps, warmup, budget_s, dataset="yelp"):
     """Time the reference's CPU implementation of the step (MultimodalSum.forward + backward as written: 9-pass loop, fp32,
     dropout 0.1, no optimizer — BASELINE.md §3) on the host cores.  One step = ONE business.  Runs the UNMODIFIED reference
@@ -138,11 +138,9 @@ def cpu_reference_steps(steps, warmup, budget_s, dataset="yelp"):
     amazon = dataset == "amazon"
     batch = make_batch(cfg, 1, seed=1, fixed_len=70 if amazon else 100, n_valid_imgs=1 if amazon else 10)
     kind, run = "port", None
-    ref = _reference_tree()
-    if ref is not None:
+    from oracle import ref_harness as RH
+    if RH.available():
         try:
-            os.environ["MMSUM_REF"] = ref
-            from oracle import ref_harness as RH
             model = RH.build_reference_model(cfg, sd, dtype=torch.float32, label_smoothing=0.1, dropout=0.1)
 
             def run():
@@ -151,7 +149,7 @@ def cpu_reference_steps(steps, warmup, budget_s, dataset="yelp"):
                 loss.backward()
             kind = "reference"
         except Exception as e:                                  # noqa: BLE001 — fall back to the port, say why
-            sys.stderr.write("reference tree at %s unusable (%s); timing the oracle port\n" % (ref, e))
+            sys.stderr.write("reference tree at %s unusable (%s); timing the oracle port\n" % (RH.REF_ROOT, e))
             run = None
     if run is None:
         from oracle import mmsum_oracle as OR
@@ -231,6 +229,50 @@ def _build_record():
     b = _lib.build_info()
     return {"library": os.path.relpath(b["path"], ROOT), "nvcc": b.get("nvcc"), "arch": b.get("arch"),
             "source_digest": (b.get("source_digest") or "")[:16], "matches_sources": b["matches_sources"]}
+
+
+DUMP_PER_TENSOR = 4096          # entries kept per parameter tensor: 566 BART-large tensors -> < 10 MB per array
+DUMP_LIMIT_BYTES = 64 << 20
+# The training step is not bitwise reproducible: the embedding / LayerNorm / column-sum gradient kernels
+# (multimodalsum_b200/csrc/rowwise.cu) accumulate with float atomicAdd, so the summation order varies between runs and the
+# difference carries through AdamW into later steps.  Two runs of the same build (default workload, --steps 10 --warmup 3,
+# one B200 at its 1000 W power limit) differed by 1.4e-2 in the relative L2 norm of grads.npy, 3e-7 in params.npy and 2e-6
+# in loss.npy.  params.npy and loss.npy are therefore the sharp comparisons between two builds; grads.npy only shows
+# differences well above that 1e-2 spread.
+
+
+def sampled_parameters(model):
+    """{"grads": ..., "params": ...}: for every parameter in `model.named_parameters()` order, its gradient and its (updated)
+    value at the same fixed entries — all of them for tensors of at most DUMP_PER_TENSOR entries, else DUMP_PER_TENSOR sorted
+    distinct flat indices drawn from a generator seeded with crc32(name), so a tensor's sample depends on its name and size
+    only — concatenated into one float32 array each."""
+    import zlib
+
+    import numpy as np
+    import torch
+    grads, params = [], []
+    for name, p in model.named_parameters():
+        g, w = p.grad.detach().reshape(-1), p.detach().reshape(-1)
+        if w.numel() > DUMP_PER_TENSOR:
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(w.numel(), DUMP_PER_TENSOR, replace=False))
+            idx = torch.from_numpy(idx).to(w.device)
+            g, w = g[idx], w[idx]
+        grads.append(g.float().cpu())
+        params.append(w.float().cpu())
+    return {"grads": torch.cat(grads).numpy(), "params": torch.cat(params).numpy()}
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float32 / float64 (at most DUMP_LIMIT_BYTES in all)."""
+    import numpy as np
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("outputs to dump take %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 class KernelTimer:
@@ -352,7 +394,7 @@ def run_train(args):
     barrier()
     t_start.record()
     for _ in range(args.steps):
-        step(resident)
+        loss = step(resident)
     t_end.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -360,6 +402,9 @@ def run_train(args):
     ms = max_over_ranks(t_start.elapsed_time(t_end))
     ms_per_step = ms / args.steps
     value = B * world / (ms_per_step / 1000.0)
+    if args.dump_outputs and rank == 0:
+        # what the caller holds after the last timed step: its loss, every .grad and the parameters AdamW updated
+        dump_outputs(args.dump_outputs, dict(loss=loss.detach().double().reshape(1).cpu().numpy(), **sampled_parameters(model)))
 
     # ---------------- instrumented steps (outside `value`): every C-ABI call bracketed with CUDA events
     n_inst = 2
@@ -516,6 +561,8 @@ def run_generate(args):
     clocks = sampler.stop() if rank == 0 else None
     launches = ops.LAUNCHES - launches0
     ms_per_step = max_over_ranks(s.elapsed_time(e)) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"generated_ids": out.cpu().numpy().astype("float64")})
     tokens = max_length - 1                       # decode steps of a full frame (random-init weights never finish early)
     value = B * world * tokens / (ms_per_step / 1e3)
     # memory encoding alone (encoder + table + image heads + 12 cross K|V projections)
@@ -613,6 +660,7 @@ def main():
         _free_gpu()
         a2 = copy.copy(args)
         a2.workload, a2.businesses, a2.steps, a2.no_cpu_baseline = "amazon", 16, min(args.steps, 5), True
+        a2.dump_outputs = None
         r = run_train(a2)
         if r is not None:
             sec["amazon_configs3"] = {k: r[k] for k in ("value", "unit", "ms_per_step", "n_gpus", "steps", "e2e", "config", "clocks", "tc_fraction_step")}
@@ -620,7 +668,7 @@ def main():
         if world == 1:
             _free_gpu()
             a3 = copy.copy(args)
-            a3.workload, a3.businesses, a3.steps = "generate", 64, 3
+            a3.workload, a3.businesses, a3.steps, a3.dump_outputs = "generate", 64, min(args.steps, 3), None
             r = run_generate(a3)
             if r is not None:
                 sec["generate_configs4"] = {k: r[k] for k in ("metric", "value", "unit", "ms_per_step", "steps", "e2e", "config", "clocks", "roofline")}

@@ -3,12 +3,12 @@ the MultimodalSum training step.  It is the checker for the CUDA path; only test
 and bench.py's cpu_baseline / --impl reference legs may import it.  The product path never does.
 
 Pinned against the reference itself: tests/golden/*.npz were produced by running the UNMODIFIED reference
-(/root/reference, through oracle/ref_harness.py) on synthetic weights/inputs from multimodalsum_b200.synth;
+(through oracle/ref_harness.py) on synthetic weights/inputs from multimodalsum_b200.synth;
 tests/test_oracle_golden.py checks this file against those vectors, tests/test_oracle_vs_reference.py against the
-live reference when /root/reference is present.  (The reference's own test-suite holds no vectors for this path —
-SURVEY.md §4.)
+live reference when a checkout of it is present (see oracle/ref_harness.py).  (The reference's own test-suite holds no
+vectors for this path — SURVEY.md §4.)
 
-All file:line citations are relative to /root/reference/src.  Every function takes the flat reference state_dict
+All file:line citations are relative to the reference's src/.  Every function takes the flat reference state_dict
 (`p`, keys of SURVEY App. B) so that no nn.Module of the reference is needed.  The algorithm is the AS-WRITTEN one:
 9 sequential leave-one-out decoder passes, K/V re-projected in every pass, logits materialised.
 """

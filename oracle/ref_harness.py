@@ -1,10 +1,11 @@
-"""TEST INFRASTRUCTURE — runs the UNMODIFIED reference (nc-ai/MultimodalSum) from /root/reference.
+"""TEST INFRASTRUCTURE — runs the UNMODIFIED reference (nc-ai/MultimodalSum) from a checkout of it.
 
-Only usable where /root/reference exists (the build container): used by tests/golden/make_golden.py to produce
-the committed golden vectors and by tests/test_oracle_vs_reference.py to pin oracle/mmsum_oracle.py.  Nothing on
-the product path, in the `-m gpu` tests, smoke() or bench.py imports this file.
+The checkout is not part of this repository.  It is found at $MMSUM_REF, else at oracle/_ref or baseline/_ref inside the
+repository (both git-ignored).  Used by tests/golden/make_golden.py to produce the committed golden vectors, by
+tests/test_oracle_vs_reference.py to pin oracle/mmsum_oracle.py, and by bench.py's CPU reference arm when present.
+Nothing on the product path, in the `-m gpu` tests or smoke() imports this file.
 
-Recipe (SURVEY.md §8c / App. G): put /root/reference/src on sys.path, stub the two imports that no longer exist
+Recipe (SURVEY.md §8c / App. G): put <checkout>/src on sys.path, stub the two imports that no longer exist
 (`apex.parallel.DistributedDataParallel`, `transformers.AdamW`), build `MultimodalSum` without its network-bound
 constructor, and call the reference's own `MultimodalSum.forward` (src/multimodal_train.py:124-163).  Only the image
 branch of `get_multimodal_outputs` (:188-192, which hard-codes a ResNet over [*,3,224,224]) is restated so pooled
@@ -18,11 +19,22 @@ import types
 import torch
 import torch.nn as nn
 
-REF_ROOT = os.environ.get("MMSUM_REF", "/root/reference")
+_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def find_reference():
+    """The first reference checkout among $MMSUM_REF, oracle/_ref and baseline/_ref, or None."""
+    for cand in (os.environ.get("MMSUM_REF"), os.path.join(_REPO, "oracle", "_ref"), os.path.join(_REPO, "baseline", "_ref")):
+        if cand and os.path.isdir(os.path.join(cand, "src", "transformer")):
+            return cand
+    return None
+
+
+REF_ROOT = find_reference()
 
 
 def available():
-    return os.path.isdir(os.path.join(REF_ROOT, "src", "transformer"))
+    return REF_ROOT is not None
 
 
 _mods = {}
@@ -32,7 +44,7 @@ def _import_reference():
     if _mods:
         return _mods
     if not available():
-        raise RuntimeError("reference tree not found at %s" % REF_ROOT)
+        raise RuntimeError("no reference checkout at $MMSUM_REF, oracle/_ref or baseline/_ref")
     sys.dont_write_bytecode = True
     src = os.path.join(REF_ROOT, "src")
     if src not in sys.path:

@@ -1,5 +1,6 @@
-"""Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference (/root/reference) on the
-synthetic weights/inputs of multimodalsum_b200.synth.  Run in the build container only:
+"""Generate the golden vectors under tests/golden/ by running the UNMODIFIED reference on the synthetic
+weights/inputs of multimodalsum_b200.synth.  Needs a checkout of the reference at $MMSUM_REF,
+oracle/_ref or baseline/_ref (see oracle/ref_harness.py):
 
     python tests/golden/make_golden.py [small|full|all]
 
@@ -119,7 +120,7 @@ def make_optimizer_golden():
     sd = make_state_dict(cfg, **c["sd"])
     grads = make_grads(cfg, **c["grads"])
     model = RH.build_reference_model(cfg, sd, dtype=torch.float32)
-    import train_utils as TU          # the reference's (RH put /root/reference/src on sys.path)
+    import train_utils as TU          # the reference's (RH put the checkout's src/ on sys.path)
     opt = TU.get_optimizer(c["lr"], c["no_decay"], model.named_parameters(), None)
     sched = TU.get_scheduler(argparse.Namespace(num_epochs=c["num_epochs"], warmup_ratio=c["warmup_ratio"]), c["t_epoch"], opt)
     named = dict(model.named_parameters())

@@ -198,6 +198,41 @@ def test_bench_reference_arm_prints_the_contract_line(monkeypatch, capsys):
     assert d["config"]["workload"] == bench.train_config(args, 1)["workload"] and d["config"]["workload"].startswith("BASELINE configs[1]")
 
 
+def test_bench_dump_outputs_samples_and_writes_float_arrays(monkeypatch, tmp_path):
+    """--dump-outputs: the same entries of every gradient / parameter on every run, written as float32 / float64 .npy files
+    within the size limit; --steps below 1 and a dump of the CPU reference arm are refused."""
+    import sys
+
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+
+    def model():
+        torch.manual_seed(3)
+        m = torch.nn.Sequential(torch.nn.Linear(100, 80), torch.nn.LayerNorm(80))
+        for p in m.parameters():
+            p.grad = torch.randn_like(p)
+        return m
+
+    a, b = bench.sampled_parameters(model()), bench.sampled_parameters(model())
+    n = bench.DUMP_PER_TENSOR + 80 + 80 + 80          # the 8000-entry weight is sampled, the small tensors are kept whole
+    assert set(a) == {"grads", "params"} and a["grads"].shape == a["params"].shape == (n,)
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    m = model()
+    w = m[0].weight.detach().reshape(-1).numpy()
+    assert np.isin(a["params"][:bench.DUMP_PER_TENSOR], w).all() and np.array_equal(a["params"][-80:], m[1].bias.detach().numpy())
+    bench.dump_outputs(str(tmp_path / "out"), dict(a, loss=np.array([1.5]), ids=np.arange(6).reshape(2, 3)))
+    got = {f: np.load(tmp_path / "out" / f) for f in sorted(os.listdir(tmp_path / "out"))}
+    assert sorted(got) == ["grads.npy", "ids.npy", "loss.npy", "params.npy"]
+    assert got["loss.npy"].dtype == np.float64 and got["ids.npy"].dtype == np.float32 and got["ids.npy"].tolist() == [[0, 1, 2], [3, 4, 5]]
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, np.float32)})
+
+
 def test_library_is_tied_to_the_sources_it_was_built_from(monkeypatch):
     """build() leaves a record (source digest, nvcc, flags) next to the library; loading a library whose record does not match
     csrc/ + include/ raises instead of running stale kernels (file mtimes do not survive the snapshot to the GPU box)."""

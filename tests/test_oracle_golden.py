@@ -1,5 +1,5 @@
 """Pin oracle/mmsum_oracle.py (the CPU restatement) against golden vectors produced by the UNMODIFIED reference
-(tests/golden/make_golden.py, run where /root/reference exists)."""
+(tests/golden/make_golden.py, run with a checkout of the reference present)."""
 import pytest
 import torch
 

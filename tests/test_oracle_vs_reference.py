@@ -1,5 +1,6 @@
-"""LIVE pin of the test infrastructure against the UNMODIFIED reference tree (skipped where /root/reference — or
-$MMSUM_REF — is absent, e.g. on the GPU box; the committed goldens carry the same pin there):
+"""LIVE pin of the test infrastructure against the UNMODIFIED reference tree (skipped unless a checkout of it is present
+at $MMSUM_REF, oracle/_ref or baseline/_ref; it is not part of this repository, and the committed goldens carry the
+same pin everywhere else):
   * oracle/mmsum_oracle.py vs the reference's own forward + backward (multimodal, text-only, img / table stages);
   * the golden files can be regenerated bit-for-bit (one case re-run);
   * checkpoint + optimizer-state interchange: what multimodalsum_b200.train_utils.save_checkpoint writes loads into the
@@ -15,7 +16,7 @@ from multimodalsum_b200.synth import ModelConfig, make_batch, make_state_dict
 from oracle import mmsum_oracle as OR
 from oracle import ref_harness as RH
 
-pytestmark = pytest.mark.skipif(not RH.available(), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not RH.available(), reason="needs a checkout of the unmodified reference ($MMSUM_REF, oracle/_ref or baseline/_ref)")
 
 SMALL = dict(encoder_layers=1, decoder_layers=2, ffn_dim=128, vocab_size=300, max_position_embeddings=128, dropout=0.0)
 

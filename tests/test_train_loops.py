@@ -139,6 +139,66 @@ def test_checkpoint_resume_round_trip(tmp_path):
         TU.load_checkpoint(m2, o2, s2, str(tmp_path / "c"))
 
 
+def test_checkpoint_files_match_the_reference_inventory(tmp_path):
+    """save_checkpoint writes what the reference's model, its stage sub-modules and its AdamW load (src/test.py:205,
+    src/multimodal_train.py:116-122, src/train_utils.py:79-97), checked against what the unmodified reference recorded in
+    tests/golden/adamw_small.npz: the names of its parameters, and which of them its own get_optimizer + AdamW updated
+    (quirk Q1: the no-decay group is empty, so those parameters carry no optimizer state).  A CPU-resident engine (arenas
+    only, no kernels) is enough to exercise the writers."""
+    from golden_util import load_optimizer_golden
+    from multimodalsum_b200.engine import StepEngine
+    from multimodalsum_b200.modules import MultimodalSum
+    gold = load_optimizer_golden()
+    cfg, sd, names, c = gold["cfg"], gold["sd"], gold["names"], gold["case"]
+    model = MultimodalSum(config=cfg)
+    model.load_state_dict(sd, strict=False)
+    eng = StepEngine(cfg, "cpu")
+    eng.bind(model.named_parameters())
+    object.__setattr__(model, "engine", eng)
+    opt = TU.get_optimizer(eng, c["lr"], c["no_decay"], model.named_parameters(), None, max_grad_norm=c["max_grad_norm"])
+    torch.manual_seed(0)
+    opt.m.normal_()
+    opt.v.uniform_()
+    opt.step_count = 2
+    sched = TU.LinearWarmupSchedule(opt, 2, 8)
+    for option in ("whole", "text", "img", "table"):
+        TU.save_checkpoint(model, opt, sched, 0, str(tmp_path / option), save_option=option)
+
+    def load(option, f="pytorch_model.bin"):
+        return torch.load(str(tmp_path / option / f))
+
+    # whole model: the reference's parameters, plus the entries of its state_dict that are not parameters of their own
+    # (the final_logits_bias buffer, and the token embedding that BART and the table encoder share under three more names)
+    shared = "bart_model.model.shared.weight"
+    aliases = {"bart_model.model.encoder.embed_tokens.weight", "bart_model.model.decoder.embed_tokens.weight",
+               "table_encoder.bart_embedding.weight"}
+    whole = load("whole")
+    assert set(whole) == set(names) | aliases | {"bart_model.final_logits_bias"}
+    for n, t in whole.items():
+        assert t.shape == sd[n].shape and torch.equal(t, sd[n]), n      # sd: the weights the reference loaded for the golden
+    assert all(torch.equal(whole[n], whole[shared]) for n in aliases)
+    # stage hand-offs: text -> bart_model, table -> table_encoder, img -> img_encoder
+    for option, prefix in (("text", "bart_model."), ("table", "table_encoder."), ("img", "img_encoder.")):
+        assert set(load(option)) == {n[len(prefix):] for n in whole if n.startswith(prefix)}, option
+    assert set(load("img")) == {"linear.weight"}
+    # training_state.bin: transformers-AdamW layout, state exactly for the parameters the reference's AdamW updated
+    state = load("whole", "training_state.bin")
+    assert state["epoch"] == 0 and state["scheduler"]["last_epoch"] == 0
+    updated = {n for n in names if gold["delta_norms"][n] > 0}
+    assert 0 < len(updated) < len(names)
+    groups = state["optimizer"]["param_groups"]
+    assert [g["weight_decay"] for g in groups] == [0.01, 0.0] and all(g["correct_bias"] for g in groups)
+    assert groups[0]["params"] == list(range(len(updated))) and groups[1]["params"] == []
+    order = [n for n, _ in model.named_parameters() if not any(nd in n for nd in c["no_decay"])]
+    assert set(order) == updated
+    st = state["optimizer"]["state"]
+    assert sorted(st) == groups[0]["params"]
+    for i, n in enumerate(order):
+        o, k = eng.offsets[n], sd[n].numel()
+        assert st[i]["step"] == 2 and st[i]["exp_avg"].shape == st[i]["exp_avg_sq"].shape == sd[n].shape, n
+        assert torch.equal(st[i]["exp_avg"].reshape(-1), opt.m[o:o + k]) and torch.equal(st[i]["exp_avg_sq"].reshape(-1), opt.v[o:o + k]), n
+
+
 class _StubModel(torch.nn.Module):
     """Stands in for the four stage modules on the CPU: records how it was called, returns a loss that depends on one tensor of
     the batch and on its parameters (so backward / clip / step do something)."""
