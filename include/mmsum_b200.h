@@ -87,8 +87,6 @@ typedef struct MmsumAttnArgs {
 } MmsumAttnArgs;
 int mmsum_attn_fwd(const MmsumAttnArgs* args, void* stream);
 int mmsum_attn_bwd(const MmsumAttnArgs* args, void* stream); /* dQ/DELTA pass, then dK/dV pass */
-/* A/B switch of the forward kernel: 0 = default (environment MMSUM_ATTN_FWD_V1 / _V2 may override), 1..3 = that version. */
-int mmsum_attn_set_fwd_variant(int32_t variant);
 /* Test aid: one CTA per SM fills its shared memory and all 512 tensor-memory columns with NaN bit patterns.  A kernel that
  * consumes stale on-chip state (0 * stale, unwritten accumulator columns) produces non-finite or run-dependent results when it
  * is launched after this one (tests/test_kernels_gpu.py::test_kernels_ignore_stale_onchip_state). */

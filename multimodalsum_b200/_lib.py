@@ -85,7 +85,7 @@ def lib():
 
 # every symbol include/mmsum_b200.h declares (tests/test_host_logic.py cross-checks this list against the header)
 EXPORTS = [
-    "mmsum_gemm_bf16", "mmsum_attn_fwd", "mmsum_attn_bwd", "mmsum_attn_set_fwd_variant", "mmsum_debug_poison",
+    "mmsum_gemm_bf16", "mmsum_attn_fwd", "mmsum_attn_bwd", "mmsum_debug_poison",
     "mmsum_cast_f32_bf16",
     "mmsum_embed_ln_fwd", "mmsum_embed_ln_bwd", "mmsum_add_ln_fwd", "mmsum_add_ln_bwd", "mmsum_colsum",
     "mmsum_gate_fwd", "mmsum_gate_bwd_u", "mmsum_gate_bwd_o", "mmsum_ce_fwd_bwd", "mmsum_prep_step",

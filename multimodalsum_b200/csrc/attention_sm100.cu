@@ -15,32 +15,15 @@
 // Shapes are the model's: 128 query positions per sequence (one UMMA M=128 tile), head_dim 64, <= 208 keys per entity,
 // so a whole entity's score tile lives in TMEM (128 lanes x <=208 fp32 columns) and no online-softmax rescaling is needed.
 //
-// forward, one CTA per (sequence, head), 192 threads:
-//   warp 0    TMA producer: Q once, then K_e / V_e per entity into a 2-stage smem ring (128B swizzle)
-//   warp 1    MMA issuer:   S_e = Q K_e^T -> TMEM (double buffered);  O_e = P_e V_e -> TMEM
-//   warps 2-5 softmax:      thread = query row; tcgen05.ld S, max, exp2, bf16 P -> swizzled smem (A operand of P V);
+// forward, one CTA per (sequence, head), 192 threads, two CTAs per SM:
+//   warp 0    TMA producer: Q once, then K_e / V_e per entity into one smem stage each (128B swizzle)
+//   warp 1    MMA issuer:   S_e = Q K_e^T -> TMEM;  O_e = P_e V_e -> TMEM (A operand P_e read from TMEM)
+//   warps 2-5 softmax:      thread = query row; tcgen05.ld S, exp2, bf16 P back over the scores in TMEM;
 //                           reads O_e back and accumulates (1/n)(1/l_e) O_e in registers; writes the modality outputs
 #include <cstdlib>
 #include <type_traits>
 #include "common.cuh"
 #include "../../include/mmsum_b200.h"
-
-// compile-time experiment switches (tools/ab_variants.sh builds one library per setting for same-box A/B timing)
-#ifndef MMSUM_DQ_PREFETCH
-#define MMSUM_DQ_PREFETCH 1
-#endif
-#ifndef MMSUM_DQ_PACKED
-#define MMSUM_DQ_PACKED 0
-#endif
-#ifndef MMSUM_TAIL16
-#define MMSUM_TAIL16 1     // forward v3 / dQ: the last 16 score columns of an entity with n16 % 32 == 16 are not processed as a
-#endif                     // full 32-column chunk (no exp2 / TMEM traffic for columns that do not exist)
-#ifndef MMSUM_FWD_ONEPASS
-#define MMSUM_FWD_ONEPASS 1 // forward v3: one pass over the scores with a lazily raised reference instead of a row-max pass first
-#endif
-#ifndef MMSUM_DKV_TS
-#define MMSUM_DKV_TS 1     // dK/dV kernel: P^T / dS^T stay in tensor memory as the A operands of the dV / dK products
-#endif
 
 namespace mmsum {
 
@@ -51,7 +34,7 @@ static constexpr int kMaxEnt = 24;
 static constexpr float kLog2e = 1.4426950408889634f;
 static constexpr int kKVStageBytes = kMaxKeys * 128;   // 26624 = 26 * 1024
 static constexpr int kPBytes = 4 * SQ * 128;           // four 64-key atoms of [128 rows x 128 B]
-static constexpr uint32_t kColS0 = 0, kColS1 = 224, kColO = 448;
+static constexpr uint32_t kColS0 = 0;
 struct EntItem {
   int kv_row0;     // first KV row of the entity
   int nkeys;       // keys of the entity (Sk of its modality)
@@ -154,642 +137,13 @@ __device__ int build_ent_items(const MmsumAttnArgs& p, int qseq, EntItem* items,
   return __popc(bal);
 }
 
-// validity bitmask of the entity's keys: bit j of word w = key 32w + j may be attended
-__device__ __forceinline__ void key_bitmask(const MmsumAttnArgs& p, const EntItem& it, int lane, uint32_t (&words)[7]) {
-#pragma unroll
-  for (int w = 0; w < 7; ++w) {
-    const int j = w * 32 + lane;
-    bool ok = j < it.nkeys;
-    if (ok && p.key_valid != nullptr) ok = p.key_valid[(long long)it.kv_row0 + j] != 0;
-    words[w] = __ballot_sync(0xffffffffu, ok);
-  }
-}
-
-struct FwdSmem {
-  uint8_t q[2][SQ * 128];      // 2-deep only in head mode (one Q tile per item); otherwise stage 0 holds the CTA's Q
-  uint8_t k[2][kKVStageBytes];
-  uint8_t v[2][kKVStageBytes];
-  uint8_t p[kPBytes];
-  float red_max[2][4][SQ];
-  float red_sum[2][4][SQ];
-  uint32_t kmask[kMaxEnt][8];
-  EntItem items[kMaxEnt];
-  uint64_t q_full[2], q_empty[2], k_full[2], k_empty[2], v_full[2], v_empty[2], s_full[2], s_empty[2], p_full, mma2_done;
-  uint32_t tmem_slot;
-  int n_items;
-};
-
-__global__ void __launch_bounds__(kAttnThreads, 1)
-attn_fwd_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs p, const int head_mode) {
-  extern __shared__ uint8_t smem_raw[];
-  pdl_launch_dependents();
-  pdl_wait();   // launched with programmatic stream serialization: nothing global is touched before this point
-  // align inside the shared window with pointer arithmetic on the __shared__ array so the compiler keeps the
-  // shared address space (LDS/STS instead of generic LD/ST)
-  FwdSmem& sm = *reinterpret_cast<FwdSmem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // head mode (self-attention: one modality, one entity): the CTA owns a whole sequence and its items are the H heads,
-  // so the per-CTA set-up and the load / MMA / softmax latencies are amortised and overlapped over 16 items instead of
-  // being paid by 16 single-item CTAs.  Otherwise the CTA owns one (sequence, head) and its items are the entities.
-  const int tgt = head_mode ? (int)(blockIdx.x % p.R) : (int)(blockIdx.x % p.R);
-  const int h = head_mode ? 0 : (int)((blockIdx.x / p.R) % p.H);
-  const int biz = head_mode ? (int)(blockIdx.x / p.R) : (int)(blockIdx.x / (p.R * p.H));
-  const int qseq = biz * p.R + tgt;
-  const int qrow0 = qseq * SQ;
-  auto item_head = [&](int i) { return head_mode ? i : h; };
-
-  if (warp == 0) {
-    int n = build_ent_items(p, qseq, sm.items, lane);
-    if (head_mode) {                       // replicate the single entity once per head
-      __syncwarp();
-      if (n > 0) {
-        const EntItem it0 = sm.items[0];
-        __syncwarp();
-        if (lane < p.H) sm.items[lane] = it0;
-        n = p.H;
-      }
-    }
-    if (lane == 0) sm.n_items = n;
-  }
-  if (threadIdx.x == 32) {
-    for (int s = 0; s < 2; ++s) { mbar_init(&sm.q_full[s], 1); mbar_init(&sm.q_empty[s], 1); }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&sm.k_full[s], 1); mbar_init(&sm.k_empty[s], 1);
-      mbar_init(&sm.v_full[s], 1); mbar_init(&sm.v_empty[s], 1);
-      mbar_init(&sm.s_full[s], 1); mbar_init(&sm.s_empty[s], kSoftThreads);
-    }
-    mbar_init(&sm.p_full, kSoftThreads);
-    mbar_init(&sm.mma2_done, 1);
-    fence_barrier_init();
-    tma_prefetch_desc(&maps.q);
-  }
-  // V rows beyond an entity's key count are multiplied by P = 0: they must hold finite values, never stale NaN bits
-  for (int i = threadIdx.x; i < 2 * kKVStageBytes / 16; i += blockDim.x)
-    reinterpret_cast<uint4*>(sm.v[0])[i] = make_uint4(0, 0, 0, 0);
-  if (warp == 1) { tmem_alloc(&sm.tmem_slot, 512); tmem_relinquish(); }
-  fence_proxy_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = sm.tmem_slot;
-  const int n_items = sm.n_items;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      if (!head_mode) {
-        mbar_expect_tx(&sm.q_full[0], SQ * 128);
-        tma_load_2d(sm.q[0], &maps.q, &sm.q_full[0], p.q_col + h * HD, qrow0);
-      }
-      // K stages are released as soon as S = Q K^T has retired, V stages only after P V: two independent rings
-      for (int i = 0; i < n_items; ++i) {
-        const int st = i & 1;
-        if (head_mode) {                   // this item's Q tile (released by the same commit as its K stage)
-          mbar_wait(&sm.q_empty[st], ((i >> 1) & 1) ^ 1);
-          mbar_expect_tx(&sm.q_full[st], SQ * 128);
-          tma_load_2d(sm.q[st], &maps.q, &sm.q_full[st], p.q_col + i * HD, qrow0);
-        }
-        mbar_wait(&sm.k_empty[st], ((i >> 1) & 1) ^ 1);
-        const EntItem it = sm.items[i];
-        mbar_expect_tx(&sm.k_full[st], it.nkeys * 128);
-        TRACE(0, i);
-        tma_load_2d(sm.k[st], &maps.kv[it.mod], &sm.k_full[st], p.k_col + item_head(i) * HD, it.kv_row0);
-      }
-    } else if (lane == 1) {
-      for (int i = 0; i < n_items; ++i) {
-        const int st = i & 1;
-        mbar_wait(&sm.v_empty[st], ((i >> 1) & 1) ^ 1);
-        const EntItem it = sm.items[i];
-        mbar_expect_tx(&sm.v_full[st], it.nkeys * 128);
-        tma_load_2d(sm.v[st], &maps.kv[it.mod], &sm.v_full[st], p.v_col + item_head(i) * HD, it.kv_row0);
-      }
-    }
-  } else if (warp == 1) {
-    build_masks(p, sm.items, n_items, sm.kmask, 0, lane);
-    if (n_items > 0) {   // whole warp runs the issue loop; elect.sync picks the issuing lane per instruction
-      const uint64_t qdesc0 = umma_smem_desc_sw128(smem_u32(sm.q[0]), 16, 1024), qdesc1 = umma_smem_desc_sw128(smem_u32(sm.q[1]), 16, 1024);
-      const uint64_t kdesc0 = umma_smem_desc_sw128(smem_u32(sm.k[0]), 16, 1024), kdesc1 = umma_smem_desc_sw128(smem_u32(sm.k[1]), 16, 1024);
-      const uint64_t pdesc = umma_smem_desc_sw128(smem_u32(sm.p), 16, 1024);
-      const uint64_t vdesc0 = umma_smem_desc_sw128(smem_u32(sm.v[0]), 8192, 1024), vdesc1 = umma_smem_desc_sw128(smem_u32(sm.v[1]), 8192, 1024);
-      if (!head_mode) mbar_wait(&sm.q_full[0], 0);
-      auto issue_s = [&](int i) {
-        const int st = i & 1;
-        const EntItem it = sm.items[i];
-        if (head_mode) mbar_wait(&sm.q_full[st], (i >> 1) & 1);
-        const uint64_t qdesc = (head_mode && st) ? qdesc1 : qdesc0;
-        mbar_wait(&sm.k_full[st], (i >> 1) & 1);
-        if (lane == 0) TRACE(1, 2 * i);
-        mbar_wait(&sm.s_empty[st], ((i >> 1) & 1) ^ 1);
-        if (lane == 0) TRACE(1, 2 * i + 1);
-        tc_fence_after();
-        const uint32_t idesc = umma_idesc_bf16(128, it.n16, 0, 0);
-        const uint64_t kdesc = st ? kdesc1 : kdesc0;
-        const uint32_t dcol = tmem + (st ? kColS1 : kColS0);
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk)
-          umma_bf16_w(dcol, desc_adv(qdesc, kk * 32), desc_adv(kdesc, kk * 32), idesc, kk > 0);
-        umma_commit_w(&sm.s_full[st]);
-        umma_commit_w(&sm.k_empty[st]);
-        if (head_mode) umma_commit_w(&sm.q_empty[st]);
-      };
-      issue_s(0);
-      const uint32_t idesc_o = umma_idesc_bf16(128, HD, 0, 1);
-      for (int i = 0; i < n_items; ++i) {
-        if (i + 1 < n_items) issue_s(i + 1);
-        const int st = i & 1;
-        const EntItem it = sm.items[i];
-        mbar_wait(&sm.v_full[st], (i >> 1) & 1);
-        if (lane == 0) TRACE(2, 2 * i);
-        mbar_wait(&sm.p_full, i & 1);
-        if (lane == 0) TRACE(2, 2 * i + 1);
-        tc_fence_after();
-        const uint64_t vdesc = st ? vdesc1 : vdesc0;
-        const int nk = it.n16 >> 4;
-#pragma unroll
-        for (int kk = 0; kk < kMaxKeys / 16; ++kk)
-          if (kk < nk)
-            umma_bf16_w(tmem + kColO, desc_adv(pdesc, (kk >> 2) * (SQ * 128) + (kk & 3) * 32), desc_adv(vdesc, kk * 2048), idesc_o, kk > 0);
-        if (lane == 0) TRACE(4, 2 * i);
-        umma_commit_w(&sm.v_empty[st]);
-        umma_commit_w(&sm.mma2_done);
-#ifdef MMSUM_ATTN_TRACE
-        mbar_wait(&sm.mma2_done, i & 1);
-        if (lane == 0) TRACE(4, 2 * i + 1);
-#endif
-      }
-    }
-  } else {
-    // ===================== softmax / accumulate warps =====================
-    // thread = (query row, column group cg): score chunks cg and cg+4, output columns [16cg, 16cg+16)
-    const int q4 = warp & 3;
-    const int cg = (warp - 2) >> 2;
-    const int row = q4 * 32 + lane;
-    const uint32_t lane_off = (uint32_t)(q4 * 32) << 16;
-    const float sc = p.scale * kLog2e;
-    float acc[16];
-#pragma unroll
-    for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-    bf16* Og = reinterpret_cast<bf16*>(p.O);
-    auto flush = [&](int m, int head) {
-      bf16* dst = Og + p.mods[m].o_off + (long long)(qrow0 + row) * p.ldo + head * HD + cg * 16;
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        uint4 u;
-        u.x = pack_bf16(acc[j * 8 + 0], acc[j * 8 + 1]); u.y = pack_bf16(acc[j * 8 + 2], acc[j * 8 + 3]);
-        u.z = pack_bf16(acc[j * 8 + 4], acc[j * 8 + 5]); u.w = pack_bf16(acc[j * 8 + 6], acc[j * 8 + 7]);
-        *reinterpret_cast<uint4*>(dst + j * 8) = u;
-      }
-#pragma unroll
-      for (int i = 0; i < 16; ++i) acc[i] = 0.f;
-    };
-    auto add_o = [&](float wgt) {
-      uint32_t r[16];
-      tmem_ld_32x16(tmem + lane_off + kColO + cg * 16, r);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 16; ++i) acc[i] = fmaf(wgt, __uint_as_float(r[i]), acc[i]);
-    };
-    // finish the bookkeeping of the previous entity once all four column groups have published their partial sums
-    float msc_prev = 0.f, invn_prev = 0.f;
-    int ent_prev = 0, head_prev = h;
-    auto close_prev = [&](int par_prev) {
-      const float l = (sm.red_sum[par_prev][0][row] + sm.red_sum[par_prev][1][row]) +
-                      (sm.red_sum[par_prev][2][row] + sm.red_sum[par_prev][3][row]);
-      if (cg == 0)
-        p.LSE[(((long long)qseq * p.H + head_prev) * p.E_total + ent_prev) * SQ + row] = (l > 0.f) ? (msc_prev + __log2f(l)) : INFINITY;
-      return (l > 0.f) ? __fdividef(invn_prev, l) : 0.f;
-    };
-    int cur_mod = 0;
-    build_masks(p, sm.items, n_items, sm.kmask, warp - 1, lane);
-    for (int i = 0; i < n_items; ++i) {
-      const EntItem it = sm.items[i];
-      const int st = i & 1, par = i & 1;
-      const int nchunk = (it.n16 + 31) >> 5;
-      const bool has0 = cg < nchunk, has1 = cg + 4 < nchunk;
-      uint32_t w0 = has0 ? sm.kmask[i][cg] : 0u;
-      uint32_t w1 = has1 ? sm.kmask[i][cg + 4] : 0u;
-      if (p.causal) { w0 = causal_word(w0, row, cg); w1 = causal_word(w1, row, cg + 4); }
-      const float inv_n = p.inv_n ? p.inv_n[(long long)qseq * p.n_mod + it.mod] : 1.f;
-      const uint32_t scol = tmem + lane_off + (st ? kColS1 : kColS0);
-      if (threadIdx.x == 64) TRACE(3, 6 * i);
-      mbar_wait(&sm.s_full[st], (i >> 1) & 1);
-      if (threadIdx.x == 64) TRACE(3, 6 * i + 1);
-      tc_fence_after();
-      // max pass (one 32-column chunk in registers at a time; 4 softmax warps per scheduler hide the TMEM latency)
-      float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-      for (int t = 0; t < 2; ++t) {
-        const bool has = t == 0 ? has0 : has1;
-        const uint32_t wd = t == 0 ? w0 : w1;
-        if (has) {
-          uint32_t r[32];
-          tmem_ld_32x32(scol + (cg + 4 * t) * 32, r);
-          tmem_ld_wait();
-          if (wd == 0xffffffffu) {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) mx4[j & 3] = fmaxf(mx4[j & 3], __uint_as_float(r[j]));
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) mx4[j & 3] = ((wd >> j) & 1u) ? fmaxf(mx4[j & 3], __uint_as_float(r[j])) : mx4[j & 3];
-          }
-        }
-      }
-      sm.red_max[par][cg][row] = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      if (threadIdx.x == 64) TRACE(3, 6 * i + 2);
-      soft_bar();
-      if (threadIdx.x == 64) TRACE(3, 6 * i + 3);
-      const float mx = fmaxf(fmaxf(sm.red_max[par][0][row], sm.red_max[par][1][row]),
-                             fmaxf(sm.red_max[par][2][row], sm.red_max[par][3][row]));
-      const float msc = (mx == -INFINITY) ? 0.f : mx * sc;
-      // the previous entity's P V has finished: fold its output in; its P buffer / O accumulator are free again
-      if (i > 0) {
-        const float w_prev = close_prev(par ^ 1);
-        mbar_wait(&sm.mma2_done, (i - 1) & 1);
-        if (threadIdx.x == 64) TRACE(3, 6 * i + 4);
-        tc_fence_after();
-        add_o(w_prev);
-        if (head_mode) flush(0, i - 1);    // previous head's output is complete
-      }
-      while (cur_mod < it.mod) { flush(cur_mod, h); ++cur_mod; }
-      // exp pass: P = exp2(s*sc - m) -> bf16 into the swizzled A-operand tile; partial row sum
-      f32x2 l2[2] = {splat2(0.f), splat2(0.f)};     // packed fp32 pairs (FFMA2 / FADD2): issue slots are the limit
-      const f32x2 sc2 = splat2(sc), nmsc2 = splat2(-msc);
-#pragma unroll
-      for (int t = 0; t < 2; ++t) {
-        const bool has = t == 0 ? has0 : has1;
-        const uint32_t wd = t == 0 ? w0 : w1;
-        if (has) {
-          const int c = cg + 4 * t;
-          uint32_t r[32];
-          tmem_ld_32x32(scol + c * 32, r);
-          tmem_ld_wait();
-          // two copies of the loop (warp-uniform choice): predicated-off mask code would still take issue slots
-          auto exp_body = [&](auto tag) {
-            constexpr bool kFull = decltype(tag)::value;
-#pragma unroll
-            for (int j = 0; j < 32; j += 2) {
-              float a0, a1;
-              unpack2(fma2(pack2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), sc2, nmsc2), a0, a1);
-              float e0 = ex2(a0), e1 = ex2(a1);
-              if constexpr (!kFull) { e0 = ((wd >> j) & 1u) ? e0 : 0.f; e1 = ((wd >> (j + 1)) & 1u) ? e1 : 0.f; }
-              l2[(j >> 1) & 1] = add2(l2[(j >> 1) & 1], pack2(e0, e1));
-              r[j] = __float_as_uint(e0); r[j + 1] = __float_as_uint(e1);
-            }
-          };
-          if (__all_sync(0xffffffffu, wd == 0xffffffffu)) exp_body(std::true_type{}); else exp_body(std::false_type{});
-          uint8_t* atom = sm.p + row * 128 + (c >> 1) * (SQ * 128);
-#pragma unroll
-          for (int g8 = 0; g8 < 4; ++g8) {
-            uint4 u;
-            u.x = pack_bf16(__uint_as_float(r[g8 * 8 + 0]), __uint_as_float(r[g8 * 8 + 1]));
-            u.y = pack_bf16(__uint_as_float(r[g8 * 8 + 2]), __uint_as_float(r[g8 * 8 + 3]));
-            u.z = pack_bf16(__uint_as_float(r[g8 * 8 + 4]), __uint_as_float(r[g8 * 8 + 5]));
-            u.w = pack_bf16(__uint_as_float(r[g8 * 8 + 6]), __uint_as_float(r[g8 * 8 + 7]));
-            const int chunk = (c & 1) * 4 + g8;
-            *reinterpret_cast<uint4*>(atom + ((chunk ^ (row & 7)) << 4)) = u;
-          }
-        }
-      }
-      float l4[4];
-      unpack2(l2[0], l4[0], l4[1]);
-      unpack2(l2[1], l4[2], l4[3]);
-      sm.red_sum[par][cg][row] = (l4[0] + l4[1]) + (l4[2] + l4[3]);
-      if (threadIdx.x == 64) TRACE(3, 6 * i + 5);
-      tc_fence_before();
-      mbar_arrive(&sm.s_empty[st]);
-      fence_proxy_async_smem();
-      mbar_arrive(&sm.p_full);
-      msc_prev = msc; invn_prev = inv_n; ent_prev = it.ent; head_prev = item_head(i);
-    }
-    if (n_items > 0) {
-      soft_bar();                                   // partial sums of the last entity are visible
-      const float w_prev = close_prev((n_items - 1) & 1);
-      mbar_wait(&sm.mma2_done, (n_items - 1) & 1);
-      tc_fence_after();
-      add_o(w_prev);
-    }
-    if (head_mode) {
-      if (n_items > 0) flush(0, n_items - 1);
-      else for (int hh = 0; hh < p.H; ++hh) flush(0, hh);      // null entity: zero rows for every head
-    } else {
-      while (cur_mod < p.n_mod) { flush(cur_mod, h); ++cur_mod; }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { __syncwarp(); tc_fence_after(); tmem_dealloc(tmem, 512); }
-}
-
 // ----------------------------------------------------------------------------------------------
-// forward, version 2 — one thread per query row, two softmax groups ping-pong over the items, P never leaves TMEM
-//   * warps 2-5 own the even items, warps 6-9 the odd ones; a thread owns a whole score row, so row max / sum need no
-//     cross-warp exchange and there is no CTA-level barrier in the item loop — the two groups drift half an item apart and
-//     one group's exp2 (MUFU) phase overlaps the other's TMEM loads, max pass and MMA hand-offs;
-//   * P = exp2(.) is written back over its own score row in tensor memory as packed bf16 (tcgen05.st) and P V is issued with
-//     the A operand in TMEM (no 64 KB P tile, no smem store traffic, no proxy fence);
-//   * outputs: per-entity O is read out of TMEM by the owning thread and folded into 64 register accumulators; the two
-//     groups' partial sums of a modality are combined through smem at the (at most three) modality boundaries.
-// ----------------------------------------------------------------------------------------------
-static constexpr int kF2Threads = 64 + 8 * 32;
-struct Fwd2Smem {
-  uint8_t q[2][SQ * 128];
-  uint8_t k[2][kKVStageBytes];
-  uint8_t v[2][kKVStageBytes];
-  float oacc[HD][SQ];          // group B's partial output of the current modality (column-major: conflict-free)
-  uint32_t kmask[kMaxEnt][8];
-  EntItem items[kMaxEnt];
-  uint64_t q_full[2], q_empty[2], k_full[2], k_empty[2], v_full[2], v_empty[2], s_full[2], p_full[2], o_full[2], o_free;
-  uint32_t tmem_slot;
-  int n_items;
-};
-__device__ __forceinline__ void f2_mask_bar() { asm volatile("bar.sync 2, 288;" ::: "memory"); }   // warps 1..9
-__device__ __forceinline__ void f2_group_bar() { asm volatile("bar.sync 3, 256;" ::: "memory"); }  // warps 2..9
-__device__ __forceinline__ void f2_build_masks(const MmsumAttnArgs& p, EntItem* items, int n_items, uint32_t (*kmask)[8],
-                                               int w, int lane) {   // w = warp - 1 in [0, 9)
-  for (int idx = w; idx < n_items * 7; idx += 9) {
-    const int i = idx / 7, c = idx - i * 7;
-    const uint32_t wd = chunk_word(p, items[i], c, lane);
-    if (lane == 0) kmask[i][c] = wd;
-  }
-  f2_mask_bar();
-  const int i = w * 32 + lane;
-  if (i < n_items) {
-    int last = 0;
-#pragma unroll
-    for (int c = 0; c < 7; ++c) { const uint32_t wd = kmask[i][c]; if (wd) last = c * 32 + 32 - __clz(wd); }
-    const int n16 = (last + 15) & ~15;
-    items[i].n16 = n16 < 16 ? 16 : n16;
-  }
-  f2_mask_bar();
-}
-
-__global__ void __launch_bounds__(kF2Threads, 1)
-attn_fwd_tc2_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs p, const int head_mode) {
-  extern __shared__ uint8_t smem_raw[];
-  pdl_launch_dependents();
-  pdl_wait();   // launched with programmatic stream serialization: nothing global is touched before this point
-  Fwd2Smem& sm = *reinterpret_cast<Fwd2Smem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int tgt = blockIdx.x % p.R;
-  const int h = head_mode ? 0 : (int)((blockIdx.x / p.R) % p.H);
-  const int biz = head_mode ? (int)(blockIdx.x / p.R) : (int)(blockIdx.x / (p.R * p.H));
-  const int qseq = biz * p.R + tgt;
-  const int qrow0 = qseq * SQ;
-  auto item_head = [&](int i) { return head_mode ? i : h; };
-
-  if (warp == 0) {
-    int n = build_ent_items(p, qseq, sm.items, lane);
-    if (head_mode) {                       // replicate the single entity once per head
-      __syncwarp();
-      if (n > 0) {
-        const EntItem it0 = sm.items[0];
-        __syncwarp();
-        if (lane < p.H) sm.items[lane] = it0;
-        n = p.H;
-      }
-    }
-    if (lane == 0) sm.n_items = n;
-  }
-  if (threadIdx.x == 32) {
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(&sm.q_full[s], 1); mbar_init(&sm.q_empty[s], 1);
-      mbar_init(&sm.k_full[s], 1); mbar_init(&sm.k_empty[s], 1);
-      mbar_init(&sm.v_full[s], 1); mbar_init(&sm.v_empty[s], 1);
-      mbar_init(&sm.s_full[s], 1); mbar_init(&sm.p_full[s], 128); mbar_init(&sm.o_full[s], 1);
-    }
-    mbar_init(&sm.o_free, 128);
-    fence_barrier_init();
-    tma_prefetch_desc(&maps.q);
-  }
-  // V rows beyond an entity's key count are multiplied by P = 0: they must hold finite values, never stale NaN bits
-  for (int i = threadIdx.x; i < 2 * kKVStageBytes / 16; i += blockDim.x)
-    reinterpret_cast<uint4*>(sm.v[0])[i] = make_uint4(0, 0, 0, 0);
-  if (warp == 1) { tmem_alloc(&sm.tmem_slot, 512); tmem_relinquish(); }
-  fence_proxy_async_smem();
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = sm.tmem_slot;
-  const int n_items = sm.n_items;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      if (!head_mode) {
-        mbar_expect_tx(&sm.q_full[0], SQ * 128);
-        tma_load_2d(sm.q[0], &maps.q, &sm.q_full[0], p.q_col + h * HD, qrow0);
-      }
-      for (int i = 0; i < n_items; ++i) {
-        const int st = i & 1;
-        if (head_mode) {
-          mbar_wait(&sm.q_empty[st], ((i >> 1) & 1) ^ 1);
-          mbar_expect_tx(&sm.q_full[st], SQ * 128);
-          tma_load_2d(sm.q[st], &maps.q, &sm.q_full[st], p.q_col + i * HD, qrow0);
-        }
-        mbar_wait(&sm.k_empty[st], ((i >> 1) & 1) ^ 1);
-        const EntItem it = sm.items[i];
-        mbar_expect_tx(&sm.k_full[st], it.nkeys * 128);
-        tma_load_2d(sm.k[st], &maps.kv[it.mod], &sm.k_full[st], p.k_col + item_head(i) * HD, it.kv_row0);
-      }
-    } else if (lane == 1) {
-      for (int i = 0; i < n_items; ++i) {
-        const int st = i & 1;
-        mbar_wait(&sm.v_empty[st], ((i >> 1) & 1) ^ 1);
-        const EntItem it = sm.items[i];
-        mbar_expect_tx(&sm.v_full[st], it.nkeys * 128);
-        tma_load_2d(sm.v[st], &maps.kv[it.mod], &sm.v_full[st], p.v_col + item_head(i) * HD, it.kv_row0);
-      }
-    }
-  } else if (warp == 1) {
-    f2_build_masks(p, sm.items, n_items, sm.kmask, 0, lane);
-    if (n_items > 0) {   // whole warp runs the issue loop; elect.sync picks the issuing lane per instruction
-      const uint64_t qdesc0 = umma_smem_desc_sw128(smem_u32(sm.q[0]), 16, 1024), qdesc1 = umma_smem_desc_sw128(smem_u32(sm.q[1]), 16, 1024);
-      const uint64_t kdesc0 = umma_smem_desc_sw128(smem_u32(sm.k[0]), 16, 1024), kdesc1 = umma_smem_desc_sw128(smem_u32(sm.k[1]), 16, 1024);
-      const uint64_t vdesc0 = umma_smem_desc_sw128(smem_u32(sm.v[0]), 8192, 1024), vdesc1 = umma_smem_desc_sw128(smem_u32(sm.v[1]), 8192, 1024);
-      if (!head_mode) mbar_wait(&sm.q_full[0], 0);
-      auto issue_s = [&](int i) {
-        const int st = i & 1;
-        const EntItem it = sm.items[i];
-        if (head_mode) mbar_wait(&sm.q_full[st], (i >> 1) & 1);
-        mbar_wait(&sm.k_full[st], (i >> 1) & 1);
-        tc_fence_after();
-        const uint32_t idesc = umma_idesc_bf16(128, it.n16, 0, 0);
-        const uint64_t qdesc = (head_mode && st) ? qdesc1 : qdesc0, kdesc = st ? kdesc1 : kdesc0;
-        const uint32_t dcol = tmem + (st ? kColS1 : kColS0);
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk)
-          umma_bf16_w(dcol, desc_adv(qdesc, kk * 32), desc_adv(kdesc, kk * 32), idesc, kk > 0);
-        umma_commit_w(&sm.s_full[st]);
-        umma_commit_w(&sm.k_empty[st]);
-        if (head_mode) umma_commit_w(&sm.q_empty[st]);
-      };
-      issue_s(0);
-      if (n_items > 1) issue_s(1);
-      const uint32_t idesc_o = umma_idesc_bf16(128, HD, 0, 1);
-      for (int i = 0; i < n_items; ++i) {
-        const int st = i & 1;
-        const EntItem it = sm.items[i];
-        mbar_wait(&sm.v_full[st], (i >> 1) & 1);
-        mbar_wait(&sm.p_full[st], (i >> 1) & 1);            // P (bf16) now sits where the scores were
-        if (lane == 0) TRACE(1, 3 * i);
-        if (i > 0) mbar_wait(&sm.o_free, (i - 1) & 1);      // the previous entity's O has been read out
-        if (lane == 0) TRACE(1, 3 * i + 1);
-        tc_fence_after();
-        const uint64_t vdesc = st ? vdesc1 : vdesc0;
-        const uint32_t pcol = tmem + (st ? kColS1 : kColS0);
-        const int nk = it.n16 >> 4;
-#pragma unroll
-        for (int kk = 0; kk < kMaxKeys / 16; ++kk)
-          if (kk < nk) umma_bf16_ts_w(tmem + kColO, pcol + kk * 8, desc_adv(vdesc, kk * 2048), idesc_o, kk > 0);
-        if (lane == 0) TRACE(1, 3 * i + 2);
-        umma_commit_w(&sm.v_empty[st]);
-        umma_commit_w(&sm.o_full[st]);
-        if (i + 2 < n_items) issue_s(i + 2);                 // overwrites this score buffer: ordered after P V above
-      }
-    }
-  } else {
-    // ===================== softmax groups: thread = one query row of every second item =====================
-    const int g = (warp - 2) >> 2;
-    const int q4 = warp & 3;
-    const int row = q4 * 32 + lane;
-    const uint32_t lane_off = (uint32_t)(q4 * 32) << 16;
-    const float sc = p.scale * kLog2e;
-    float acc[HD];
-#pragma unroll
-    for (int i = 0; i < HD; ++i) acc[i] = 0.f;
-    bf16* Og = reinterpret_cast<bf16*>(p.O);
-    auto store_out = [&](int m, int head) {        // acc -> bf16 output row, then reset
-      bf16* dst = Og + p.mods[m].o_off + (long long)(qrow0 + row) * p.ldo + head * HD;
-#pragma unroll
-      for (int j = 0; j < HD / 8; ++j) {
-        uint4 u;
-        u.x = pack_bf16(acc[j * 8 + 0], acc[j * 8 + 1]); u.y = pack_bf16(acc[j * 8 + 2], acc[j * 8 + 3]);
-        u.z = pack_bf16(acc[j * 8 + 4], acc[j * 8 + 5]); u.w = pack_bf16(acc[j * 8 + 6], acc[j * 8 + 7]);
-        *reinterpret_cast<uint4*>(dst + j * 8) = u;
-      }
-#pragma unroll
-      for (int i = 0; i < HD; ++i) acc[i] = 0.f;
-    };
-    // modality boundary (entity mode): group B hands its partial sums to group A through smem
-    auto flush = [&](int m) {
-      if (g == 1) {
-#pragma unroll
-        for (int j = 0; j < HD; ++j) sm.oacc[j][row] = acc[j];
-#pragma unroll
-        for (int j = 0; j < HD; ++j) acc[j] = 0.f;
-      }
-      f2_group_bar();
-      if (g == 0) {
-#pragma unroll
-        for (int j = 0; j < HD; ++j) acc[j] += sm.oacc[j][row];
-        store_out(m, h);
-      }
-      f2_group_bar();
-    };
-    int cur_mod = 0;
-    f2_build_masks(p, sm.items, n_items, sm.kmask, warp - 1, lane);
-    for (int i = g; i < n_items; i += 2) {
-      const EntItem it = sm.items[i];
-      const int head = item_head(i);
-      const int nchunk = (it.n16 + 31) >> 5;
-      const float inv_n = p.inv_n ? p.inv_n[(long long)qseq * p.n_mod + it.mod] : 1.f;
-      if (!head_mode) { while (cur_mod < it.mod) { flush(cur_mod); ++cur_mod; } }
-      const uint32_t scol = tmem + lane_off + (g ? kColS1 : kColS0);
-      const bool tr = (lane == 0 && q4 == 2);   // warps 2 and 6
-      if (tr) TRACE(3 + g, 6 * (i >> 1));
-      mbar_wait(&sm.s_full[g], (i >> 1) & 1);
-      if (tr) TRACE(3 + g, 6 * (i >> 1) + 1);
-      tc_fence_after();
-      // (Tried and measured slower: 16-column pieces with the next tcgen05.ld in flight, and strictly alternating the two
-      //  groups' exp2 phases with a token — the ~200-clock TMEM load round trip, not MUFU contention, bounds a lone warp.)
-      // ---- row max ----
-      float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll 1
-      for (int c = 0; c < nchunk; ++c) {
-        uint32_t wd = sm.kmask[i][c];
-        if (p.causal) wd = causal_word(wd, row, c);
-        uint32_t r[32];
-        tmem_ld_32x32(scol + c * 32, r);
-        tmem_ld_wait();
-        if (__all_sync(0xffffffffu, wd == 0xffffffffu)) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) mx4[j & 3] = fmaxf(mx4[j & 3], __uint_as_float(r[j]));
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) mx4[j & 3] = ((wd >> j) & 1u) ? fmaxf(mx4[j & 3], __uint_as_float(r[j])) : mx4[j & 3];
-        }
-      }
-      const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      const float msc = (mx == -INFINITY) ? 0.f : mx * sc;
-      if (tr) TRACE(3 + g, 6 * (i >> 1) + 2);
-      // ---- P = exp2(s*sc - m) written back over the scores as packed bf16; row sum ----
-      f32x2 l2[2] = {splat2(0.f), splat2(0.f)};
-      const f32x2 sc2 = splat2(sc), nmsc2 = splat2(-msc);
-#pragma unroll 1
-      for (int c = 0; c < nchunk; ++c) {
-        uint32_t wd = sm.kmask[i][c];
-        if (p.causal) wd = causal_word(wd, row, c);
-        uint32_t r[32], pk[16];
-        tmem_ld_32x32(scol + c * 32, r);
-        tmem_ld_wait();
-        auto body = [&](auto tag) {
-          constexpr bool kFull = decltype(tag)::value;
-#pragma unroll
-          for (int j = 0; j < 32; j += 2) {
-            float a0, a1;
-            unpack2(fma2(pack2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), sc2, nmsc2), a0, a1);
-            float e0 = ex2(a0), e1 = ex2(a1);
-            if constexpr (!kFull) { e0 = ((wd >> j) & 1u) ? e0 : 0.f; e1 = ((wd >> (j + 1)) & 1u) ? e1 : 0.f; }
-            l2[(j >> 1) & 1] = add2(l2[(j >> 1) & 1], pack2(e0, e1));
-            pk[j >> 1] = pack_bf16(e0, e1);
-          }
-        };
-        if (__all_sync(0xffffffffu, wd == 0xffffffffu)) body(std::true_type{}); else body(std::false_type{});
-        tmem_st_32x16(scol + c * 16, pk);          // columns [16c, 16c+16) lie inside score chunks this thread has consumed
-      }
-      tmem_st_wait();
-      tc_fence_before();
-      mbar_arrive(&sm.p_full[g]);
-      if (tr) TRACE(3 + g, 6 * (i >> 1) + 3);
-      float l4[4];
-      unpack2(l2[0], l4[0], l4[1]);
-      unpack2(l2[1], l4[2], l4[3]);
-      const float l = (l4[0] + l4[1]) + (l4[2] + l4[3]);
-      p.LSE[(((long long)qseq * p.H + head) * p.E_total + it.ent) * SQ + row] = (l > 0.f) ? (msc + __log2f(l)) : INFINITY;
-      const float wgt = (l > 0.f) ? __fdividef(inv_n, l) : 0.f;
-      // ---- this entity's O = P V: fold into the register accumulators ----
-      mbar_wait(&sm.o_full[g], (i >> 1) & 1);
-      if (tr) TRACE(3 + g, 6 * (i >> 1) + 4);
-      tc_fence_after();
-#pragma unroll
-      for (int hh = 0; hh < 2; ++hh) {
-        uint32_t r[32];
-        tmem_ld_32x32(tmem + lane_off + kColO + hh * 32, r);
-        tmem_ld_wait();
-#pragma unroll
-        for (int j = 0; j < 32; ++j) acc[hh * 32 + j] = fmaf(wgt, __uint_as_float(r[j]), acc[hh * 32 + j]);
-      }
-      tc_fence_before();
-      mbar_arrive(&sm.o_free);
-      if (tr) TRACE(3 + g, 6 * (i >> 1) + 5);
-      if (head_mode) store_out(0, head);
-    }
-    if (head_mode) {
-      if (n_items == 0 && g == 0) for (int hh = 0; hh < p.H; ++hh) store_out(0, hh);   // null entity: zero rows for every head
-    } else {
-      while (cur_mod < p.n_mod) { flush(cur_mod); ++cur_mod; }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { __syncwarp(); tc_fence_after(); tmem_dealloc(tmem, 512); }
-}
-
-// ----------------------------------------------------------------------------------------------
-// forward, version 3 — two INDEPENDENT CTAs per SM instead of two coupled softmax groups in one CTA
-//   v2's two groups share one MMA warp that issues in order and ONE output accumulator: P V of item i+1 waits for the
-//   read-out of O_i, so the groups run almost serially (measured ~4.1 k clk per item against ~4.7 k for a single group).
-//   Here a CTA is a single chain (4 softmax warps, thread = query row; 256 TMEM columns; one Q / K / V stage, 69 KB smem) and
+// forward — two INDEPENDENT CTAs per SM
+//   A CTA is a single chain (4 softmax warps, thread = query row; 256 TMEM columns; one Q / K / V stage, 69 KB smem) and
 //   TWO such CTAs are resident per SM, each with its own MMA warp, score buffer and output accumulator; they interfere only
-//   through the shared pipes, and one CTA's set-up / tear-down overlaps the other's items.
+//   through the shared pipes, and one CTA's set-up / tear-down overlaps the other's items.  Two softmax groups coupled in one
+//   CTA would share one in-order MMA warp and ONE output accumulator: P V of item i+1 waits for the read-out of O_i, so the
+//   groups ran almost serially (measured ~4.1 k clk per item against ~4.7 k for a single group).
 //   TMEM columns: scores [0, 208); P (bf16) over the scores' lower half [0, 104); O at [192, 256) — it overlaps score columns
 //   only of 208-wide (image) entities, and only after their exp pass has consumed them.
 // ----------------------------------------------------------------------------------------------
@@ -976,14 +330,9 @@ attn_fwd_tc3_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs p
       mbar_wait(&sm.s_full, i & 1);
       tc_fence_after();
       // ---- row max ----
-#if MMSUM_TAIL16
-      const int nfull = it.n16 >> 5;                 // 32-column chunks; an odd 16-column tail is handled on its own
+      // 32-column chunks; an odd 16-column tail is handled on its own (no exp2 / TMEM traffic for columns that do not exist)
+      const int nfull = it.n16 >> 5;
       const bool tail = (it.n16 & 16) != 0;
-#else
-      const int nfull = (it.n16 + 31) >> 5;
-      const bool tail = false;
-#endif
-#if MMSUM_FWD_ONEPASS
       // One pass: every 32-column chunk is read from tensor memory ONCE.  P = exp2(s*sc - ref) where ref is an integer reference
       // in the scaled log2 domain that starts at ceil(max of the first chunk) and is raised only when a later chunk exceeds it
       // by more than kSlack — then the bf16 P columns already written and the row sum are rescaled by the exact power of two
@@ -1056,62 +405,6 @@ attn_fwd_tc3_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs p
       for (int c = 0; c < nfull; ++c) one_part(std::integral_constant<int, 32>{}, c);
       if (tail) one_part(std::integral_constant<int, 16>{}, nfull);
       const float msc = (ref == -INFINITY) ? 0.f : ref;
-#else
-      float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-      auto max_part = [&](auto ntag, int c) {
-        constexpr int NC = decltype(ntag)::value;
-        uint32_t wd = sm.kmask[i][c];
-        if (p.causal) wd = causal_word(wd, row, c);
-        constexpr uint32_t kAll = NC == 32 ? 0xffffffffu : 0xffffu;
-        wd &= kAll;
-        uint32_t r[NC];
-        if constexpr (NC == 32) tmem_ld_32x32(scol + c * 32, r); else tmem_ld_32x16(scol + c * 32, r);
-        tmem_ld_wait();
-        if (__all_sync(0xffffffffu, wd == kAll)) {
-#pragma unroll
-          for (int j = 0; j < NC; ++j) mx4[j & 3] = fmaxf(mx4[j & 3], __uint_as_float(r[j]));
-        } else {
-#pragma unroll
-          for (int j = 0; j < NC; ++j) mx4[j & 3] = ((wd >> j) & 1u) ? fmaxf(mx4[j & 3], __uint_as_float(r[j])) : mx4[j & 3];
-        }
-      };
-#pragma unroll 1
-      for (int c = 0; c < nfull; ++c) max_part(std::integral_constant<int, 32>{}, c);
-      if (tail) max_part(std::integral_constant<int, 16>{}, nfull);
-      const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-      const float msc = (mx == -INFINITY) ? 0.f : mx * sc;
-      // ---- P = exp2(s*sc - m) written back over the scores as packed bf16; row sum ----
-      f32x2 l2[2] = {splat2(0.f), splat2(0.f)};
-      const f32x2 sc2 = splat2(sc), nmsc2 = splat2(-msc);
-      auto exp_part = [&](auto ntag, int c) {
-        constexpr int NC = decltype(ntag)::value;
-        uint32_t wd = sm.kmask[i][c];
-        if (p.causal) wd = causal_word(wd, row, c);
-        constexpr uint32_t kAll = NC == 32 ? 0xffffffffu : 0xffffu;
-        wd &= kAll;
-        uint32_t r[NC], pk[NC / 2];
-        if constexpr (NC == 32) tmem_ld_32x32(scol + c * 32, r); else tmem_ld_32x16(scol + c * 32, r);
-        tmem_ld_wait();
-        auto body = [&](auto tag) {
-          constexpr bool kFull = decltype(tag)::value;
-#pragma unroll
-          for (int j = 0; j < NC; j += 2) {
-            float a0, a1;
-            unpack2(fma2(pack2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), sc2, nmsc2), a0, a1);
-            float e0 = ex2(a0), e1 = ex2(a1);
-            if constexpr (!kFull) { e0 = ((wd >> j) & 1u) ? e0 : 0.f; e1 = ((wd >> (j + 1)) & 1u) ? e1 : 0.f; }
-            l2[(j >> 1) & 1] = add2(l2[(j >> 1) & 1], pack2(e0, e1));
-            pk[j >> 1] = pack_bf16(e0, e1);
-          }
-        };
-        if (__all_sync(0xffffffffu, wd == kAll)) body(std::true_type{}); else body(std::false_type{});
-        // columns [16c, 16c + NC/2) lie inside score chunks this thread has consumed
-        if constexpr (NC == 32) tmem_st_32x16(scol + c * 16, pk); else tmem_st_32x8(scol + c * 16, pk);
-      };
-#pragma unroll 1
-      for (int c = 0; c < nfull; ++c) exp_part(std::integral_constant<int, 32>{}, c);
-      if (tail) exp_part(std::integral_constant<int, 16>{}, nfull);
-#endif
       tmem_st_wait();
       tc_fence_before();
       mbar_arrive(&sm.p_full);
@@ -1177,9 +470,9 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
   // shared address space (LDS/STS instead of generic LD/ST)
   BwdQSmem& sm = *reinterpret_cast<BwdQSmem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // head mode (self-attention, <= 128 keys): the CTA owns a whole sequence and its items are the H heads (see the forward
-  // kernel); each item then has its own Q / dA tiles (2-deep ring: stage 1 lives in the unused upper half of the dS
-  // region) and its own dQ, read out of TMEM one item later.
+  // head mode (self-attention, <= 128 keys): the CTA owns a whole sequence and its items are the H heads, so the per-CTA
+  // set-up and the load / MMA / softmax latencies are amortised over the heads; each item then has its own Q / dA tiles
+  // (2-deep ring: stage 1 lives in the unused upper half of the dS region) and its own dQ, read out of TMEM one item later.
   const int tgt = blockIdx.x % p.R;
   const int h = head_mode ? 0 : (int)((blockIdx.x / p.R) % p.H);
   const int biz = head_mode ? (int)(blockIdx.x / p.R) : (int)(blockIdx.x / (p.R * p.H));
@@ -1347,15 +640,13 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
       }
     };
     // LSE / 1/n of an item are fetched one item ahead: as plain loads at the top of the item their global latency (~500 clk)
-    // sat in front of pass 1 of every item
+    // would sit in front of pass 1 of every item
     auto lse_index = [&](int i) { return (((long long)qseq * p.H + item_head(i)) * p.E_total + sm.items[i].ent) * SQ + row; };
     float lse_nx = 0.f, invn_nx = 1.f;
-#if MMSUM_DQ_PREFETCH
     if (n_items > 0) {
       lse_nx = p.LSE[lse_index(0)];
       if (p.inv_n) invn_nx = p.inv_n[(long long)qseq * p.n_mod + sm.items[0].mod];
     }
-#endif
     for (int i = 0; i < n_items; ++i) {
       const EntItem it = sm.items[i];
       const int par = i & 1;
@@ -1366,17 +657,12 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
       wd[1] = has[1] ? sm.kmask[i][cg + 4] : 0u;
       if (p.causal) { wd[0] = causal_word(wd[0], row, cg); wd[1] = causal_word(wd[1], row, cg + 4); }
       const long long li = lse_index(i);
-#if MMSUM_DQ_PREFETCH
       const float lse = lse_nx;
       const float inv_n = invn_nx;
       if (i + 1 < n_items) {
         lse_nx = p.LSE[lse_index(i + 1)];
         if (p.inv_n) invn_nx = p.inv_n[(long long)qseq * p.n_mod + sm.items[i + 1].mod];
       }
-#else
-      const float lse = p.LSE[li];
-      const float inv_n = p.inv_n ? p.inv_n[(long long)qseq * p.n_mod + it.mod] : 1.f;
-#endif
       if (threadIdx.x == 64) TRACE(3, 5 * i);
       mbar_wait(&sm.sdp_full, i & 1);
       if (threadIdx.x == 64) TRACE(3, 5 * i + 1);
@@ -1387,12 +673,7 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
       // (entities of <= 4 chunks keep dP' in registers across the delta exchange and release both after pass 1), so
       // the next entity's Q K^T / dA V^T overlap this entity's softmax work.
       const float wgt = p.scale * inv_n;
-#if MMSUM_DQ_PACKED
-      f32x2 dl2[2] = {splat2(0.f), splat2(0.f)};
-      const f32x2 sc2 = splat2(sc), nlse2 = splat2(-lse), wgt2 = splat2(wgt);
-#else
       float dl4[4] = {0.f, 0.f, 0.f, 0.f};
-#endif
       // half = 16 score columns: bits [16*half, +16) of the chunk's mask word, packed P words [8*half, +8)
       auto pass1 = [&](const uint32_t w16, const uint32_t (&rs)[16], const uint32_t (&rd)[16], uint32_t (&pk)[8]) {
         // two copies of the loop (warp-uniform choice): predicated-off mask code would still take issue slots
@@ -1400,15 +681,10 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
           constexpr bool kFull = decltype(tag)::value;
 #pragma unroll
           for (int j = 0; j < 16; j += 2) {
-            // packed fp32 pairs (FFMA2): the softmax warps are issue-bound, two lanes per instruction count
-#if MMSUM_DQ_PACKED
-            float a0, a1;
-            unpack2(fma2(pack2(__uint_as_float(rs[j]), __uint_as_float(rs[j + 1])), sc2, nlse2), a0, a1);
-            float p0 = ex2(a0), p1 = ex2(a1);
-#else
+            // scalar FFMA: at this kernel's 96-register cap the pack / unpack moves of packed fp32 pairs cost more than the
+            // halved FFMA count saves
             float p0 = ex2(fmaf(__uint_as_float(rs[j]), sc, -lse));
             float p1 = ex2(fmaf(__uint_as_float(rs[j + 1]), sc, -lse));
-#endif
             float d0 = __uint_as_float(rd[j]), d1 = __uint_as_float(rd[j + 1]);
             // masked columns: the score tile's columns beyond n16 were never written by this entity's MMAs (stale tensor
             // memory, possibly NaN patterns), so both factors are SELECTED to zero — 0 * stale is not 0
@@ -1417,23 +693,14 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
               p0 = b0 ? p0 : 0.f; p1 = b1 ? p1 : 0.f;
               d0 = b0 ? d0 : 0.f; d1 = b1 ? d1 : 0.f;
             }
-#if MMSUM_DQ_PACKED
-            dl2[(j >> 1) & 1] = fma2(pack2(p0, p1), pack2(d0, d1), dl2[(j >> 1) & 1]);
-#else
             dl4[(j >> 1) & 3] = fmaf(p0, d0, dl4[(j >> 1) & 3]);
             dl4[(j >> 1) & 3] = fmaf(p1, d1, dl4[(j >> 1) & 3]);
-#endif
             pk[j >> 1] = pack_bf16(p0, p1);
           }
         };
         if (__all_sync(0xffffffffu, w16 == 0xffffu)) body(std::true_type{}); else body(std::false_type{});
       };
       auto exchange_delta = [&]() {
-#if MMSUM_DQ_PACKED
-        float dl4[4];
-        unpack2(dl2[0], dl4[0], dl4[1]);
-        unpack2(dl2[1], dl4[2], dl4[3]);
-#endif
         sm.red_delta[par][cg][row] = (dl4[0] + dl4[1]) + (dl4[2] + dl4[3]);
         if (threadIdx.x == 64) TRACE(3, 5 * i + 2);
         soft_bar();
@@ -1445,9 +712,6 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
       };
       auto pass2 = [&](const int c, const int half, const float dw, const uint32_t (&rd)[16], const uint32_t (&pk)[8]) {
         uint8_t* atom = sm.ds + row * 128 + (c >> 1) * (SQ * 128);
-#if MMSUM_DQ_PACKED
-        const f32x2 ndw2 = splat2(-dw);
-#endif
 #pragma unroll
         for (int g8 = 0; g8 < 2; ++g8) {
           uint32_t o[4];
@@ -1455,13 +719,7 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
           for (int e = 0; e < 4; ++e) {
             const float2 pr = unpack_bf16(pk[g8 * 4 + e]);
             const int j = g8 * 8 + 2 * e;
-#if MMSUM_DQ_PACKED
-            float s0, s1;
-            unpack2(mul2(pack2(pr.x, pr.y), fma2(pack2(__uint_as_float(rd[j]), __uint_as_float(rd[j + 1])), wgt2, ndw2)), s0, s1);
-            o[e] = pack_bf16(s0, s1);
-#else
             o[e] = pack_bf16(pr.x * fmaf(__uint_as_float(rd[j]), wgt, -dw), pr.y * fmaf(__uint_as_float(rd[j + 1]), wgt, -dw));
-#endif
           }
           const int chunk = (c & 1) * 4 + half * 2 + g8;
           *reinterpret_cast<uint4*>(atom + ((chunk ^ (row & 7)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
@@ -1469,11 +727,7 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
       };
       // 16-column halves beyond the entity's n16 (the tail of the last chunk when n16 % 32 == 16): the dQ product never reads
       // them, so they are neither loaded nor computed nor stored
-#if MMSUM_TAIL16
       const bool live[2][2] = {{cg * 32 < it.n16, cg * 32 + 16 < it.n16}, {(cg + 4) * 32 < it.n16, (cg + 4) * 32 + 16 < it.n16}};
-#else
-      const bool live[2][2] = {{has[0], has[0]}, {has[1], has[1]}};
-#endif
       if (nchunk <= 4) {
         uint32_t pk[2][8] = {}, rda[16] = {}, rdb[16] = {};
         if (live[0][0]) {
@@ -1571,7 +825,7 @@ attn_bwd_dq_tc_kernel(const __grid_constant__ AttnMaps maps, const MmsumAttnArgs
 // ----------------------------------------------------------------------------------------------
 // backward, part 2 — one CTA per (business, head, entity tile of <=128 keys): dK, dV summed over the consumer targets
 //   per target:  S^T = K Q^T and dP'^T = V dA^T into TMEM (keys on the lanes);
-//   Pn^T = inv_n * exp2(sc*S^T - LSE[q]);  dS^T = scale * Pn^T o (dP'^T - delta'[q]);  both -> bf16 smem;
+//   Pn^T = inv_n * exp2(sc*S^T - LSE[q]);  dS^T = scale * Pn^T o (dP'^T - delta'[q]);  both -> bf16 over their own TMEM columns;
 //   dV += Pn^T dA,  dK += dS^T Q  (TMEM accumulators over all targets)
 // ----------------------------------------------------------------------------------------------
 // Two CTAs share an SM (256 TMEM columns, ~100 KB smem, 320 threads each): one CTA's softmax phase overlaps the other's
@@ -1592,24 +846,16 @@ __host__ __device__ inline int mod_tiles(const MmsumAttnMod& md) {
   return mod_packed(md) ? (md.E * md.Sk + SQ - 1) / SQ : md.E * ((md.Sk + SQ - 1) / SQ);
 }
 
-#if MMSUM_DKV_TS
-static constexpr int kKvStages = 4;                 // Q / dA ring depth (the P^T / dS^T tiles no longer take shared memory)
-#else
-static constexpr int kKvStages = 2;
-#endif
+static constexpr int kKvStages = 4;                 // Q / dA ring depth (P^T / dS^T stay in TMEM, so smem has room for four)
 struct BwdKVSmem {
   uint8_t k[SQ * 128];
   uint8_t v[SQ * 128];
   uint8_t q[kKvStages][QH * 128];      // Q / dA rows of the step's 64 queries (ring)
   uint8_t da[kKvStages][QH * 128];
-#if !MMSUM_DKV_TS
-  uint8_t pt[SQ * 128];        // Pn^T  [128 keys][64 queries] bf16, K-major A operand
-  uint8_t dst[SQ * 128];       // dS^T
-#endif
   float lse[2][2][QH];         // raw LSE / DELTA rows of the current and the next step (cp.async staged), for the (up to)
   float dlt[2][2][QH];         // two entities a packed tile straddles
   float lg_invn[32];           // log2(1/n) of every target for this modality
-  uint64_t kv_full, kv_free, qd_full[kKvStages], qd_empty[kKvStages], sdp_full, sdp_empty, pds_full, pds_free;
+  uint64_t kv_full, kv_free, qd_full[kKvStages], qd_empty[kKvStages], sdp_full, pds_full, pds_free;
   uint32_t tmem_slot;
 };
 static constexpr uint32_t kColST = 0, kColDPT = 64, kColDK = 128, kColDV = 192;
@@ -1689,7 +935,7 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
   if (threadIdx.x == 0) {
     mbar_init(&sm.kv_full, 1); mbar_init(&sm.kv_free, 1);
     for (int s = 0; s < kKvStages; ++s) { mbar_init(&sm.qd_full[s], 1); mbar_init(&sm.qd_empty[s], 1); }
-    mbar_init(&sm.sdp_full, 1); mbar_init(&sm.sdp_empty, kKvSoftThreads);
+    mbar_init(&sm.sdp_full, 1);
     mbar_init(&sm.pds_full, kKvSoftThreads); mbar_init(&sm.pds_free, 1);
     fence_barrier_init();
   }
@@ -1726,9 +972,6 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
   } else if (warp == 1) {
     {   // whole warp runs the issue loop; elect.sync picks the issuing lane per instruction
       const uint64_t kdesc = umma_smem_desc_sw128(smem_u32(sm.k), 16, 1024), vdesc = umma_smem_desc_sw128(smem_u32(sm.v), 16, 1024);
-#if !MMSUM_DKV_TS
-      const uint64_t ptdesc = umma_smem_desc_sw128(smem_u32(sm.pt), 16, 1024), dstdesc = umma_smem_desc_sw128(smem_u32(sm.dst), 16, 1024);
-#endif
       // stage descriptors: the stages are QH*128 bytes apart, so stage st = stage 0 advanced by st * QH*128 bytes
       const uint64_t qdesc_k0 = umma_smem_desc_sw128(smem_u32(sm.q[0]), 16, 1024), qdesc_mn0 = umma_smem_desc_sw128(smem_u32(sm.q[0]), 8192, 1024);
       const uint64_t dadesc_k0 = umma_smem_desc_sw128(smem_u32(sm.da[0]), 16, 1024), dadesc_mn0 = umma_smem_desc_sw128(smem_u32(sm.da[0]), 8192, 1024);
@@ -1740,9 +983,6 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
         if (s % n_steps == 0) mbar_wait(&sm.kv_full, (s / n_steps) & 1);
         mbar_wait(&sm.qd_full[st], (s / kKvStages) & 1);
         if (lane == 0) TRACE(5, 4 * s);
-#if !MMSUM_DKV_TS
-        mbar_wait(&sm.sdp_empty, (s & 1) ^ 1);
-#endif
         if (lane == 0) TRACE(5, 4 * s + 1);
         tc_fence_after();
         const uint64_t qd = desc_adv(qdesc_k0, st * (QH * 128)), dd = desc_adv(dadesc_k0, st * (QH * 128));
@@ -1755,24 +995,17 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
         umma_commit_w(&sm.sdp_full);
         if (s % n_steps == n_steps - 1) umma_commit_w(&sm.kv_free);   // last reader of this head's K / V tiles
       };
-#if MMSUM_DKV_TS
       // P^T / dS^T overwrite the score columns they were computed from and feed the dV / dK products straight out of tensor
       // memory, so the next step's S^T / dP^T products can only follow this step's dV / dK (issue order = execution order):
       // one serial chain per CTA, the co-resident CTA fills the gaps.
       for (int s = 0; s < g_total; ++s) {
         issue_sdp(s);
-#else
-      issue_sdp(0);
-      for (int s = 0; s < g_total; ++s) {
-        if (s + 1 < g_total) issue_sdp(s + 1);
-#endif
         const int st = s % kKvStages;
         const uint32_t first = (s % n_steps == 0) ? 0u : 1u;     // first step of a head starts fresh dK / dV accumulators
         mbar_wait(&sm.pds_full, s & 1);
         if (lane == 0) TRACE(5, 4 * s + 2);
         tc_fence_after();
         const uint64_t qd = desc_adv(qdesc_mn0, st * (QH * 128)), dd = desc_adv(dadesc_mn0, st * (QH * 128));
-#if MMSUM_DKV_TS
         // k-step kk = 16 queries = 8 packed columns; queries 32cg + [0, 32) sit at columns 32cg + [0, 16) of their score tile
 #pragma unroll
         for (int kk = 0; kk < QH / 16; ++kk)   // contraction over the step's 64 queries
@@ -1780,14 +1013,6 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
 #pragma unroll
         for (int kk = 0; kk < QH / 16; ++kk)
           umma_bf16_ts_w(tmem + kColDK, tmem + kColDPT + (kk >> 1) * 32 + (kk & 1) * 8, desc_adv(qd, kk * 2048), idesc_o, (kk > 0) ? 1u : first);
-#else
-#pragma unroll
-        for (int kk = 0; kk < QH / 16; ++kk)   // contraction over the step's 64 queries
-          umma_bf16_w(tmem + kColDV, desc_adv(ptdesc, kk * 32), desc_adv(dd, kk * 2048), idesc_o, (kk > 0) ? 1u : first);
-#pragma unroll
-        for (int kk = 0; kk < QH / 16; ++kk)
-          umma_bf16_w(tmem + kColDK, desc_adv(dstdesc, kk * 32), desc_adv(qd, kk * 2048), idesc_o, (kk > 0) ? 1u : first);
-#endif
         if (lane == 0) TRACE(5, 4 * s + 3);
         umma_commit_w(&sm.qd_empty[st]);
         umma_commit_w(&sm.pds_free);
@@ -1803,10 +1028,6 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
     const float sc = p.scale * kLog2e;
     const int slot = (packed && key0 + row >= md.Sk) ? 1 : 0;  // which of the tile's two entities owns this key row
     const bool kvalid = (row < nkeys) && (slot ? ok_hi : ok_lo) && (p.key_valid == nullptr || p.key_valid[(long long)kvrow0 + row] != 0);
-#if !MMSUM_DKV_TS
-    uint8_t* patom = sm.pt + row * 128;
-    uint8_t* datom = sm.dst + row * 128;
-#endif
     auto lse_index = [&](int h, int s, int ent) {
       return (((long long)(biz * p.R + step_target(s)) * p.H + h) * p.E_total + md.ent_base + ent) * SQ + (s & 1) * QH + (sw * 32 + lane);
     };
@@ -1856,18 +1077,8 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
       tmem_ld_32x32(tmem + lane_off + kColST + cg * 32, rs);
       tmem_ld_32x32(tmem + lane_off + kColDPT + cg * 32, rd);
       tmem_ld_wait();
-#if !MMSUM_DKV_TS
-      // S^T / dP^T now live in registers: hand the TMEM columns back so the next step's products overlap this one
-      tc_fence_before();
-      mbar_arrive(&sm.sdp_empty);
-#endif
       if (threadIdx.x == 64) TRACE(6, 6 * s + 3);
       const f32x2 lg2 = splat2(lg), m1 = splat2(-1.f), sc2 = splat2(sc), scale2 = splat2(p.scale), nscale2 = splat2(-p.scale);
-      // the P^T / dS^T tiles of the previous step must have been consumed by its dV / dK products (they were issued
-      // while this step waited for its scores, so this wait is short; it lets every group be stored as it is formed)
-#if !MMSUM_DKV_TS
-      if (g > 0) mbar_wait(&sm.pds_free, (g - 1) & 1);
-#endif
       if (threadIdx.x == 64) TRACE(6, 6 * s + 4);
       // three copies of the loop (warp-uniform choice; predicated-off mask code would still take issue slots):
       //   0 = every score valid;  1 = per-element mask (causal);  2 = the thread's key row is valid or not as a whole (pad keys,
@@ -1902,28 +1113,18 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
           dso[e2] = pack_bf16(s0, s1);
           if constexpr (kMode == 2) { po[e2] = wd ? po[e2] : 0u; dso[e2] = wd ? dso[e2] : 0u; }
         }
-#if MMSUM_DKV_TS
         // packed bf16 pairs back over the thread's own score columns (4 words = 8 queries): A operands of dV += Pn^T dA and
         // dK += dS^T Q, read by the tensor core straight from tensor memory
         tmem_st_32x4(tmem + lane_off + kColST + cg * 32 + g8 * 4, po);
         tmem_st_32x4(tmem + lane_off + kColDPT + cg * 32 + g8 * 4, dso);
-#else
-        const int chunk = cg * 4 + g8;
-        *reinterpret_cast<uint4*>(patom + ((chunk ^ (row & 7)) << 4)) = make_uint4(po[0], po[1], po[2], po[3]);
-        *reinterpret_cast<uint4*>(datom + ((chunk ^ (row & 7)) << 4)) = make_uint4(dso[0], dso[1], dso[2], dso[3]);
-#endif
       }
       };
       if (__all_sync(0xffffffffu, wd == 0xffffffffu)) body(std::integral_constant<int, 0>{});
       else if (p.causal || qpartial) body(std::integral_constant<int, 1>{});
       else body(std::integral_constant<int, 2>{});
       if (threadIdx.x == 64) TRACE(6, 6 * s + 5);
-#if MMSUM_DKV_TS
       tmem_st_wait();
       tc_fence_before();
-#else
-      fence_proxy_async_smem();
-#endif
       mbar_arrive(&sm.pds_full);
     }
     mbar_wait(&sm.pds_free, (g0 + n_steps - 1) & 1);
@@ -2013,9 +1214,7 @@ static int build_maps(const MmsumAttnArgs* a, AttnMaps* mp, bool bwd) {
 
 using namespace mmsum;
 
-// A/B and debugging switches ------------------------------------------------------------------
-static std::atomic<int> g_fwd_variant{0};   // 0 = environment / default, 1..3 = forward kernel version
-extern "C" int mmsum_attn_set_fwd_variant(int v) { g_fwd_variant.store(v); return 0; }
+// Debugging aids ------------------------------------------------------------------------------
 
 // Fills every SM's shared memory and tensor memory with NaN bit patterns: a kernel that consumes stale on-chip state shows up as
 // non-finite / run-to-run different output when launched after this one (tools/gpu_attn_determinism.py).
@@ -2053,31 +1252,15 @@ extern "C" int mmsum_attn_fwd(const MmsumAttnArgs* a, void* stream_v) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_v);
   AttnMaps mp;
   if (int rc = build_maps(a, &mp, false)) return rc;
-  const int smem = (int)sizeof(FwdSmem) + 1024;
+  const int smem = (int)sizeof(Fwd3Smem) + 1024;
   static std::atomic<unsigned long long> attr{0};
-  if (int rc = ensure_dyn_smem(attn_fwd_tc_kernel, smem, attr)) return rc;
-  // self-attention shape (one modality, one entity per sequence, no leave-one-out): heads become the CTA's items
+  if (int rc = ensure_dyn_smem(attn_fwd_tc3_kernel, smem, attr)) return rc;
+  // self-attention shape (one modality, one entity per sequence, no leave-one-out): heads become the CTA's items, so the
+  // per-CTA set-up and the load / MMA / softmax latencies are amortised over the heads instead of paid once per head.  Two
+  // CTAs per sequence (half of the heads each) so that both CTA slots of every SM are used.
   const int head_mode = (a->n_mod == 1 && a->mods[0].E == 1 && !a->mods[0].loo && a->H <= kMaxEnt && a->n_qseq >= 64) ? 1 : 0;
-  static const bool env_v1 = (getenv("MMSUM_ATTN_FWD_V1") != nullptr);   // A/B switch: the first forward kernel
-  static const bool env_v2 = (getenv("MMSUM_ATTN_FWD_V2") != nullptr);   // A/B switch: two coupled groups in one CTA
-  const int variant = g_fwd_variant.load();
-  const bool short_frames = a->q_rows != 0 && a->q_rows != SQ;     // only the default kernel drops rows beyond q_rows
-  const bool use_v1 = !short_frames && (variant ? variant == 1 : env_v1), use_v2 = !short_frames && (variant ? variant == 2 : env_v2);
-  if (!use_v1 && !use_v2) {
-    const int smem3 = (int)sizeof(Fwd3Smem) + 1024;
-    static std::atomic<unsigned long long> attr3{0};
-    if (int rc = ensure_dyn_smem(attn_fwd_tc3_kernel, smem3, attr3)) return rc;
-    // self-attention: two CTAs per sequence (half of the heads each) so that both CTA slots of every SM are used
-    const int hpc = head_mode ? ((a->H % 2 == 0 && a->n_qseq <= 2 * kNumSMs) ? a->H / 2 : a->H) : 0;
-    MMSUM_LAUNCH_PDL(attn_fwd_tc3_kernel, head_mode ? a->n_qseq * (a->H / hpc) : a->n_qseq * a->H, kF3Threads, smem3, stream, mp, *a, hpc);
-  } else if (use_v1) {
-    MMSUM_LAUNCH_PDL(attn_fwd_tc_kernel, head_mode ? a->n_qseq : a->n_qseq * a->H, kAttnThreads, smem, stream, mp, *a, head_mode);
-  } else {
-    const int smem2 = (int)sizeof(Fwd2Smem) + 1024;
-    static std::atomic<unsigned long long> attr2{0};
-    if (int rc = ensure_dyn_smem(attn_fwd_tc2_kernel, smem2, attr2)) return rc;
-    MMSUM_LAUNCH_PDL(attn_fwd_tc2_kernel, head_mode ? a->n_qseq : a->n_qseq * a->H, kF2Threads, smem2, stream, mp, *a, head_mode);
-  }
+  const int hpc = head_mode ? ((a->H % 2 == 0 && a->n_qseq <= 2 * kNumSMs) ? a->H / 2 : a->H) : 0;
+  MMSUM_LAUNCH_PDL(attn_fwd_tc3_kernel, head_mode ? a->n_qseq * (a->H / hpc) : a->n_qseq * a->H, kF3Threads, smem, stream, mp, *a, hpc);
   MMSUM_CHECK_LAUNCH();
   return 0;
 }

@@ -92,7 +92,9 @@ __device__ __forceinline__ float bf16_round(float x) { return __bfloat162float(_
 
 // erf via Abramowitz-Stegun 7.1.26 (|abs err| <= 1.5e-7, far below the bf16 rounding of every consumer): one MUFU.RCP,
 // one MUFU.EX2 and a degree-5 Horner chain instead of libdevice erff (~3x the instructions; the GELU epilogues of the
-// fc1 GEMMs were ALU-bound on it).  E = exp(-x^2/2) = exp(-z^2) is shared with the Gaussian pdf term of GELU'.
+// fc1 GEMMs were ALU-bound on it).  E = exp(-x^2/2) = exp(-z^2) is shared with the Gaussian pdf term of GELU'.  An FMA-only
+// polynomial erf measured slower (DESIGN.md §3): the epilogue is issue-bound on the FMA pipe, and the two MUFU operations of
+// this form run beside it for free.
 __device__ __forceinline__ float fast_ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -104,18 +106,6 @@ __device__ __forceinline__ float fast_rcp(float x) {
   return y;
 }
 // Blackwell packed fp32 pairs (FFMA2 / FMUL2): one issue slot for two lanes of the same elementwise chain.
-#ifndef MMSUM_SCALAR_PAIRS
-#define MMSUM_SCALAR_PAIRS 0   // experiment: the same helpers on two scalar FFMA / FMUL / FADD (A/B of the packed instructions)
-#endif
-#if MMSUM_SCALAR_PAIRS
-struct f32x2 { float a, b; };
-__device__ __forceinline__ f32x2 pack2(float a, float b) { f32x2 o; o.a = a; o.b = b; return o; }
-__device__ __forceinline__ f32x2 splat2(float a) { return pack2(a, a); }
-__device__ __forceinline__ void unpack2(f32x2 v, float& a, float& b) { a = v.a; b = v.b; }
-__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { return pack2(fmaf(a.a, b.a, c.a), fmaf(a.b, b.b, c.b)); }
-__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { return pack2(a.a * b.a, a.b * b.b); }
-__device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { return pack2(a.a + b.a, a.b + b.b); }
-#else
 struct f32x2 { uint64_t r; };
 __device__ __forceinline__ f32x2 pack2(float a, float b) { f32x2 o; asm("mov.b64 %0, {%1, %2};" : "=l"(o.r) : "f"(a), "f"(b)); return o; }
 __device__ __forceinline__ f32x2 splat2(float a) { return pack2(a, a); }
@@ -123,7 +113,6 @@ __device__ __forceinline__ void unpack2(f32x2 v, float& a, float& b) { asm("mov.
 __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 o; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(o.r) : "l"(a.r), "l"(b.r), "l"(c.r)); return o; }
 __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 o; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(o.r) : "l"(a.r), "l"(b.r)); return o; }
 __device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { f32x2 o; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(o.r) : "l"(a.r), "l"(b.r)); return o; }
-#endif
 
 // erf(x / sqrt(2)) for a pair; E = exp(-x*x/2)
 __device__ __forceinline__ f32x2 erf_as2(float x0, float x1, f32x2 x, f32x2& E) {
@@ -143,41 +132,10 @@ __device__ __forceinline__ f32x2 erf_as2(float x0, float x1, f32x2 x, f32x2& E) 
   float e0, e1; unpack2(e, e0, e1);
   return pack2(copysignf(e0, x0), copysignf(e1, x1));
 }
-// erf(x / sqrt(2)) for a pair on the FMA pipe alone: z = x / sqrt(2) clamped to +-3.7 (1 - erf(3.7) = 1.7e-7),
-// erf(z) = z * P(t), t = 2 z^2 / 3.7^2 - 1 in [-1, 1] (well-conditioned Horner), 13 coefficients from a weighted minimax fit:
-// |err| <= 8.6e-7 in fp32 arithmetic (tools/fit_erf_poly.py).  An experiment kept behind a switch: measured SLOWER than the A&S
-// form above (fc1 fwd 144 -> 149 us, fc2 dgrad 164 -> 181 us) — the epilogue is issue-bound on the FMA pipe and the two MUFU
-// operations of the A&S form run beside it for free.
-#ifndef MMSUM_GELU_POLY
-#define MMSUM_GELU_POLY 0
-#endif
-__device__ __forceinline__ f32x2 erf_poly2(float x0, float x1) {
-  const float z0 = fminf(fmaxf(x0 * 0.70710678118654752f, -3.7f), 3.7f);
-  const float z1 = fminf(fmaxf(x1 * 0.70710678118654752f, -3.7f), 3.7f);
-  const f32x2 z = pack2(z0, z1);
-  const f32x2 t = fma2(mul2(z, z), splat2(2.0f / (3.7f * 3.7f)), splat2(-1.f));
-  f32x2 q = fma2(splat2(3.335623013e-03f), t, splat2(-8.240699660e-03f));
-  q = fma2(q, t, splat2(6.850095427e-03f));
-  q = fma2(q, t, splat2(-8.780994488e-03f));
-  q = fma2(q, t, splat2(2.348297531e-02f));
-  q = fma2(q, t, splat2(-3.920011775e-02f));
-  q = fma2(q, t, splat2(5.225112182e-02f));
-  q = fma2(q, t, splat2(-6.962657820e-02f));
-  q = fma2(q, t, splat2(9.046336749e-02f));
-  q = fma2(q, t, splat2(-1.127387113e-01f));
-  q = fma2(q, t, splat2(1.408016399e-01f));
-  q = fma2(q, t, splat2(-1.904646949e-01f));
-  q = fma2(q, t, splat2(3.821373826e-01f));
-  return mul2(q, z);
-}
 __device__ __forceinline__ void gelu_erf2(float& x0, float& x1) {
   const f32x2 x = pack2(x0, x1);
-#if MMSUM_GELU_POLY
-  const f32x2 e = erf_poly2(x0, x1);
-#else
   f32x2 E;
   const f32x2 e = erf_as2(x0, x1, x, E);
-#endif
   const f32x2 hx = mul2(x, splat2(0.5f));
   unpack2(fma2(hx, e, hx), x0, x1);
 }
@@ -195,14 +153,7 @@ __device__ __forceinline__ void gelu_erf_and_grad2(float& x0, float& x1, float& 
 __device__ __forceinline__ void gelu_erf_grad_mul2(float& g0, float& g1, float x0, float x1) {
   const f32x2 x = pack2(x0, x1);
   f32x2 E;
-#if MMSUM_GELU_POLY
-  const f32x2 e = erf_poly2(x0, x1);
-  const f32x2 a = mul2(x, mul2(x, splat2(-0.72134752044448170f)));      // -x^2 / 2 * log2(e)
-  float a0, a1; unpack2(a, a0, a1);
-  E = pack2(fast_ex2(a0), fast_ex2(a1));
-#else
   const f32x2 e = erf_as2(x0, x1, x, E);
-#endif
   const f32x2 cdf = fma2(e, splat2(0.5f), splat2(0.5f));
   const f32x2 d = fma2(x, mul2(E, splat2(0.3989422804014327f)), cdf);
   unpack2(mul2(pack2(g0, g1), d), g0, g1);

@@ -125,12 +125,10 @@ attn_decode_cross_kernel(const __grid_constant__ DecMaps maps, const MmsumAttnAr
   float oc[8][4];
 #pragma unroll
   for (int nd = 0; nd < 8; ++nd) { oc[nd][0] = 0.f; oc[nd][1] = 0.f; oc[nd][2] = 0.f; oc[nd][3] = 0.f; }
-#ifndef MMSUM_DECODE_ORDERED
-#define MMSUM_DECODE_ORDERED 1     // entity outputs are added to the CTA accumulator in ENTITY ORDER (bit-reproducible results)
-#endif
-  // ordered variant: the warp that finished entity i waits until entity i-1 has been added, then adds its own output with plain
-  // read-modify-writes (it holds the turn) and passes the turn on.  Entities are pulled in increasing order, so they also finish
-  // roughly in order and the wait is short; the sum order no longer depends on which warp got which entity or on timing.
+  // Entity outputs are added to the CTA accumulator in ENTITY ORDER (bit-reproducible results): the warp that finished entity i
+  // waits until entity i-1 has been added, then adds its own output with plain read-modify-writes (it holds the turn) and passes
+  // the turn on.  Entities are pulled in increasing order, so they also finish roughly in order and the wait is short; the sum
+  // order does not depend on which warp got which entity or on timing.
   auto add_in_order = [&](int i, int m) {
     if (lane == 0) { while (*reinterpret_cast<volatile int*>(&sm.turn) != i) { } }
     __syncwarp();
@@ -148,20 +146,6 @@ attn_decode_cross_kernel(const __grid_constant__ DecMaps maps, const MmsumAttnAr
     __syncwarp();
     if (lane == 0) *reinterpret_cast<volatile int*>(&sm.turn) = i + 1;
   };
-#if !MMSUM_DECODE_ORDERED
-  int cur_mod = -1;
-  auto flush = [&](int m) {          // fold this warp's partial output of modality m into the CTA accumulator
-    if (m >= 0 && g < R) {
-#pragma unroll
-      for (int nd = 0; nd < 8; ++nd) {
-        atomicAdd(&sm.oacc[m][g][nd * 8 + 2 * t], oc[nd][0]);
-        atomicAdd(&sm.oacc[m][g][nd * 8 + 2 * t + 1], oc[nd][1]);
-      }
-    }
-#pragma unroll
-    for (int nd = 0; nd < 8; ++nd) { oc[nd][0] = 0.f; oc[nd][1] = 0.f; oc[nd][2] = 0.f; oc[nd][3] = 0.f; }
-  };
-#endif
 
   uint32_t phase = 0;
   for (;;) {
@@ -171,9 +155,6 @@ attn_decode_cross_kernel(const __grid_constant__ DecMaps maps, const MmsumAttnAr
     if (i >= n_items) break;
     const DecItem it = sm.items[i];
     if (lane == 0) load_tile(it, p.k_col);
-#if !MMSUM_DECODE_ORDERED
-    if (it.mod != cur_mod) { flush(cur_mod); cur_mod = it.mod; }
-#endif
     const int nkeys = it.nkeys;
     const int nblk = (nkeys + 15) >> 4;
     // validity words of the entity's keys (bit j of word c: key 32c + j may be attended)
@@ -276,13 +257,8 @@ attn_decode_cross_kernel(const __grid_constant__ DecMaps maps, const MmsumAttnAr
       }
     }
     __syncwarp();          // the stage may be overwritten by the next entity's keys
-#if MMSUM_DECODE_ORDERED
     add_in_order(i, it.mod);
-#endif
   }
-#if !MMSUM_DECODE_ORDERED
-  flush(cur_mod);
-#endif
   __syncthreads();
   // ---- modality outputs: [n_mod][hypothesis][head slice] (a modality without a valid entity yields zeros)
   bf16* Og = reinterpret_cast<bf16*>(p.O);

@@ -484,8 +484,7 @@ extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
     // weights and halve each CTA's K loop when 256-wide tiles would leave most of the SMs idle
     // (not for the split-K weight gradients: their K loop supplies the work units, and 256-wide CTA-pair tiles are 12 % faster
     //  there — tools/gpu_gemm_sweep.py)
-    static const bool wgrad128 = [] { const char* e = getenv("MMSUM_WGRAD_BN128"); return e && e[0] == '1'; }();   // A/B switch
-    const bool splitk_ok = a->out_f32 && a->accumulate && a->A2 == nullptr && a->splits <= 0 && !wgrad128;
+    const bool splitk_ok = a->out_f32 && a->accumulate && a->A2 == nullptr && a->splits <= 0;
     if (bn == 256 && a->aux_mode == 0 && !splitk_ok &&
         (long long)((a->M + BM - 1) / BM) * ((a->N + 255) / 256) * 2 <= num_sms()) bn = 128;
   }

@@ -120,9 +120,7 @@ class StepEngine:
         self.bound = False
         self.ws = None
         self.ws_full = None
-        # A/B switches (defaults = the faster variants, DESIGN.md section 4)
-        self.dkv_concat = os.environ.get("MMSUM_DKV_CONCAT", "1") != "0"
-        self.gelu_dact = os.environ.get("MMSUM_GELU_DACT", "1") != "0"
+        # A/B switch (default = the faster variant, DESIGN.md section 2)
         self.trim_frames = os.environ.get("MMSUM_TRIM_FRAMES", "1") != "0"
         self._len_cache = None
         self.ws_key = None
@@ -267,7 +265,7 @@ class StepEngine:
         for k in ("enc_x0", "enc_m0", "enc_r0"):
             w[k] = full[k][:Te]
         w["dec"] = [dict(a, kv=a["kv"][:Tm]) for a in full["dec"]]
-        for k in ("MEM", "dkv_all", "dMEM16", "dMEM32", "mem_valid"):
+        for k in ("MEM", "dkv_all", "dMEM16", "mem_valid"):
             if k in full:
                 w[k] = full[k][:Tm]
         w["pool_e"] = _PoolRows(full["pool"], Te)
@@ -345,12 +343,8 @@ class StepEngine:
         # cross-attention K|V gradients of ALL decoder layers side by side: the memory gradient is then ONE GEMM over the
         # concatenated K (sum_l dkv_l W_l = [dkv_0 | dkv_1 | ...] [W_0; W_1; ...]) instead of L fp32 read-modify-write passes
         # over a [Tm, D] accumulator (TMA reduce-add: 2.5 ms per step at config 2, against 1.75 ms for the single product)
-        if self.dkv_concat:
-            w["dkv_all"] = bf(Tm, L_d * 2 * D)
-            w["Wkv_cat"] = bf(L_d * 2 * D, D)
-        else:
-            w["dkv_all"] = bf(Tm, 2 * D)
-            w["dMEM32"] = f32(Tm, D)
+        w["dkv_all"] = bf(Tm, L_d * 2 * D)
+        w["Wkv_cat"] = bf(L_d * 2 * D, D)
         w["delta"] = f32(N, H, Et, S)
         w["dMEM16"] = bf(Tm, D)
         w["dz32"] = f32(T, D)
@@ -659,7 +653,7 @@ class StepEngine:
     def _ffn_block_fwd(self, a, lp, xin, out, mk, rk, l, kind):
         g = ops.gemm
         g(xin, self.w16(lp + "fc1.weight"), a["a"], bias=self.w32(lp + "fc1.bias"), act=ops.ACT_GELU, aux=a["h"],
-          aux_mode=ops.AUX_STORE_DACT if self.gelu_dact else ops.AUX_STORE_PREACT)   # a["h"]: GELU'(pre-activation) (backward is one multiply)
+          aux_mode=ops.AUX_STORE_DACT)   # a["h"]: GELU'(pre-activation) (backward is one multiply)
         g(a["a"], self.w16(lp + "fc2.weight"), a["f"], bias=self.w32(lp + "fc2.bias"))
         ops.add_ln_fwd(xin, a["f"], self.w32(lp + "final_layer_norm.weight"), self.w32(lp + "final_layer_norm.bias"),
                        out, a[mk], a[rk], self.pd, self.seed, self._sid(kind, l), step_dev=self.step_dev)
@@ -711,7 +705,7 @@ class StepEngine:
         self._bias_grad(df, self.g32(lp + "fc2.bias"))
         self._wgrad(df, a["a"], lp + "fc2.weight")
         dH = w["dH"][:xin.shape[0]]
-        ops.gemm(df, self.w16(lp + "fc2.weight"), dH, b_t=True, act=ops.ACT_GELU, aux=a["h"], aux_mode=ops.AUX_MUL if self.gelu_dact else ops.AUX_MUL_DACT)
+        ops.gemm(df, self.w16(lp + "fc2.weight"), dH, b_t=True, act=ops.ACT_GELU, aux=a["h"], aux_mode=ops.AUX_MUL)
         if df is not dres:
             pool.put(df)
         self._bias_grad(dH, self.g32(lp + "fc1.bias"))
@@ -760,9 +754,6 @@ class StepEngine:
         first = next(iter(self.params.values()))
         if force_zero or first.grad is None:
             self.G32.zero_()
-
-        if not self.dkv_concat:
-            w["dMEM32"].zero_()
         # ---- loss + LM head
         logits = w["logits"]
         ops.ce_fwd_bwd(logits, V, w["labels"], self.label_smoothing, 1.0 / T, grad_out, w["loss_rows"], None, 0.0, True,
@@ -812,7 +803,7 @@ class StepEngine:
             if dyc is not dres:
                 pool.put(dyc)
             dqc = pool.get()
-            dkv = w["dkv_all"][:, l * 2 * D:(l + 1) * 2 * D] if self.dkv_concat else w["dkv_all"]
+            dkv = w["dkv_all"][:, l * 2 * D:(l + 1) * 2 * D]
             ops.attn_bwd(self._cross_attn_args(w, a["qc"], a["kv"], dA3, a["lse_c"], bwd=(dqc, dkv)))
             self._bias_grad(dqc, self.g32(c + "q_proj.bias"))
             self._wgrad(dqc, a["x1"], c + "q_proj.weight")
@@ -821,10 +812,7 @@ class StepEngine:
             pool.put(dqc)
             self._bias_grad(dkv, self.g32(c + "k_proj.bias", c + "v_proj.bias"))
             self._wgrad(dkv, w["MEM"], c + "k_proj.weight", c + "v_proj.weight")
-            if self.dkv_concat:
-                w["Wkv_cat"][l * 2 * D:(l + 1) * 2 * D].copy_(self.w16(c + "k_proj.weight", c + "v_proj.weight"))
-            else:       # A/B: one fp32 reduce-add pass over the memory gradient per layer
-                g(dkv, self.w16(c + "k_proj.weight", c + "v_proj.weight"), w["dMEM32"], b_t=True, accumulate=True)
+            w["Wkv_cat"][l * 2 * D:(l + 1) * 2 * D].copy_(self.w16(c + "k_proj.weight", c + "v_proj.weight"))
             # self block
             d1, d2 = self._self_block_bwd(w, a, lp, dres, dx1, w["dec_valid"], True, l, 4)
             self._ready(lp + "self_attn_layer_norm.bias")
@@ -839,10 +827,7 @@ class StepEngine:
 
         # ---- memory gradients: table, image, text
         dMEM = w["dMEM16"]
-        if self.dkv_concat:
-            g(w["dkv_all"], w["Wkv_cat"], dMEM, b_t=True)
-        else:
-            ops.cast_bf16(w["dMEM32"], dMEM)
+        g(w["dkv_all"], w["Wkv_cat"], dMEM, b_t=True)
         if F > 0:
             t = "table_encoder."
             dtab = dMEM[Tt:Tt + B * F]

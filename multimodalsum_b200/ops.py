@@ -258,11 +258,6 @@ def attn_bwd(a):
     _timed(kind, 2.5 * attn_flops(a), lambda: check(_lib.lib().mmsum_attn_bwd(C.byref(a), _stream()), "mmsum_attn_bwd", 2))
 
 
-def set_attn_fwd_variant(v):
-    """A/B switch of the attention forward kernel (0 = default, 1..3 = version)."""
-    check(_lib.lib().mmsum_attn_set_fwd_variant(int(v)), "mmsum_attn_set_fwd_variant")
-
-
 def debug_poison():
     """Test aid: fill every SM's shared and tensor memory with NaN patterns (see include/mmsum_b200.h)."""
     check(_lib.lib().mmsum_debug_poison(_stream()), "mmsum_debug_poison")

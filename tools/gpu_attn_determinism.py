@@ -1,7 +1,7 @@
-"""Run-to-run determinism / stale-state check of the attention forward kernels.
-(1) kernel level: the multi-entity cross-attention at a small ragged shape and the config-2 shape, each forward variant launched
-    repeatedly with every SM's shared and tensor memory poisoned with NaN patterns in between; outputs must be finite, bitwise
-    identical from launch to launch and agree across variants.
+"""Run-to-run determinism / stale-state check of the attention forward kernel.
+(1) kernel level: the multi-entity cross-attention at small ragged shapes and the config-2 shape, the forward launched
+    repeatedly with every SM's shared and tensor memory poisoned with NaN patterns in between; outputs must be finite and bitwise
+    identical from launch to launch.
 (2) step level: forward of the small graph-test configuration run twice on the same inputs; every workspace buffer is compared
     bitwise between the two runs (first difference = the non-deterministic kernel)."""
 import ctypes as C
@@ -57,36 +57,24 @@ def kernel_level():
     for shape in [(2, 5, 47, 2, 196, 1), (3, 4, 47, 3, 196, 2), (16, 9, 47, 10, 196, 3)]:
         kw, A3, lse, keep = cross_case(*shape)
         a = ops.attn_args(**kw)
-        ref = {}
-        for v in (2, 3):
-            lib.mmsum_attn_set_fwd_variant(v)
-            outs = []
-            for it in range(6):
-                A3.fill_(float("nan")); lse.fill_(float("nan"))
-                if it % 2:
-                    poison()
-                ops.attn_fwd(a)
-                torch.cuda.synchronize()
-                outs.append((A3.clone(), lse.clone()))
-            fin = all(torch.isfinite(o.float()).all().item() for o, _ in outs)
-            same = all(torch.equal(outs[0][0], o) and torch.equal(outs[0][1].nan_to_num(7.0, 7.0, 7.0), l.nan_to_num(7.0, 7.0, 7.0))
-                       for o, l in outs)
-            ref[v] = outs[0]
-            print("shape", shape, "variant", v, "finite", fin, "bitwise-reproducible", same, flush=True)
-        d = (ref[2][0].float() - ref[3][0].float()).abs().max().item()
-        lv2, lv3 = ref[2][1], ref[3][1]
-        written = torch.isfinite(lv2) & torch.isfinite(lv3)
-        dl = (lv2[written] - lv3[written]).abs().max().item() if written.any() else 0.0
-        print("   v2 vs v3: max |dO| %.3e  max |dLSE| %.3e  LSE written-set equal %s" %
-              (d, dl, torch.equal(torch.isnan(lv2), torch.isnan(lv3))), flush=True)
-    lib.mmsum_attn_set_fwd_variant(0)
+        outs = []
+        for it in range(6):
+            A3.fill_(float("nan")); lse.fill_(float("nan"))
+            if it % 2:
+                poison()
+            ops.attn_fwd(a)
+            torch.cuda.synchronize()
+            outs.append((A3.clone(), lse.clone()))
+        fin = all(torch.isfinite(o.float()).all().item() for o, _ in outs)
+        same = all(torch.equal(outs[0][0], o) and torch.equal(outs[0][1].nan_to_num(7.0, 7.0, 7.0), l.nan_to_num(7.0, 7.0, 7.0))
+                   for o, l in outs)
+        print("shape", shape, "finite", fin, "bitwise-reproducible", same, flush=True)
 
 
-def step_level(variant):
+def step_level():
     from golden_util import load_golden
     from multimodalsum_b200.modules import MultimodalSum, YelpTableEncoder
     from multimodalsum_b200.synth import make_batch
-    lib.mmsum_attn_set_fwd_variant(variant)
     gold = load_golden("small_yelp")
     cfg = gold["cfg"]
     cfg.dropout = 0.0
@@ -119,22 +107,20 @@ def step_level(variant):
         s = snap(model.engine.ws)
         s.update(g)
         runs.append((loss.item(), s))
-    print("variant", variant, "losses", [r[0] for r in runs], flush=True)
+    print("losses", [r[0] for r in runs], flush=True)
     base = runs[0][1]
     for it in range(1, 4):
         diff = [k for k, t in base.items()
                 if not torch.equal(t.view(torch.uint8) if t.dtype != torch.bool else t, runs[it][1][k].view(torch.uint8) if t.dtype != torch.bool else runs[it][1][k])]
         nf = [k for k, t in runs[it][1].items() if t.is_floating_point() and k.startswith("grad.") and not torch.isfinite(t).all()]
         print("  run", it, "buffers differing from run 0:", len(diff), diff[:30], "non-finite grads:", len(nf), flush=True)
-    lib.mmsum_attn_set_fwd_variant(0)
 
 
-def first_nonfinite(variant, with_poison):
+def first_nonfinite(with_poison):
     """Wraps the op layer: after every backward op, checks its outputs; prints the first op that produces a non-finite value."""
     from golden_util import load_golden
     from multimodalsum_b200.modules import MultimodalSum, YelpTableEncoder
     from multimodalsum_b200.synth import make_batch
-    lib.mmsum_attn_set_fwd_variant(variant)
     gold = load_golden("small_yelp")
     cfg = gold["cfg"]
     cfg.dropout = 0.0
@@ -222,19 +208,16 @@ def first_nonfinite(variant, with_poison):
             torch.cuda.synchronize()
             state["on"] = False
             nf = [n for n, p in model.named_parameters() if not torch.isfinite(p.grad).all()]
-            print("variant", variant, "poison", with_poison, "run", it, "loss", loss.item(), "non-finite grads", len(nf), nf[:4], flush=True)
+            print("poison", with_poison, "run", it, "loss", loss.item(), "non-finite grads", len(nf), nf[:4], flush=True)
     finally:
         for k, f in orig.items():
             setattr(ops, k, f)
-        lib.mmsum_attn_set_fwd_variant(0)
 
 
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nan":
-        for v in (2, 3):
-            first_nonfinite(v, False)
-            first_nonfinite(v, True)
+        first_nonfinite(False)
+        first_nonfinite(True)
         sys.exit(0)
     kernel_level()
-    step_level(2)
-    step_level(3)
+    step_level()

@@ -26,7 +26,7 @@ for l, a in enumerate(w["enc"]):
 for l, a in enumerate(w["dec"]):
     for k, t in a.items():
         if isinstance(t, torch.Tensor): nanrep("dec%d.%s" % (l, k), t)
-for k in ("delta", "dMEM32", "dMEM16", "dA3", "dO3", "dqkv", "dkv", "dz32", "dH"):
+for k in ("delta", "dMEM16", "dA3", "dO3", "dqkv", "dkv", "dz32", "dH"):
     if k in w: nanrep("bwd." + k, w[k])
 nbad = [n for n in gold["names"] if not torch.isfinite(grads[n]).all()]
 print("non-finite grads:", len(nbad), "of", len(gold["names"]), nbad[:6])
