@@ -124,6 +124,19 @@ int mmsum_beam_update(const float* cand_val, const int32_t* cand_tok, int64_t* i
                       int64_t* beam_idx, int64_t* next_tok, int32_t* next_tok32, int32_t* hist, int32_t B, int32_t k, int32_t K,
                       int32_t L, int32_t eos, int32_t pad, int32_t early_stopping, float length_penalty, void* stream);
 
+/* One sampled token per row (_generate_no_beam_search with do_sample=True, vendored transformers 3.0.2 generation_utils.py):
+ * repetition penalty over the distinct ids of the row's prefix (enforce_repetition_penalty_), EOS ban below min_length and
+ * n-gram ban (postprocess_next_token_scores / calc_banned_ngram_tokens), / temperature, top_k_top_p_filtering (top_k = 0 or
+ * >= V: off; ties at the k-th value kept; top-p ties ranked by token id), softmax, one draw from Philox4x32-10 keyed by
+ * *seed_dev with counter (cur, row).  Then tok = unfinished[row] ? tok : pad, ids[row, cur] = tok, next_tok32[row] = tok
+ * (optional: the decoder's next input), unfinished[row] = 0 if tok == eos.  logits fp32 [rows, ld], ld % 4 == 0, 16-byte
+ * aligned, V <= 57 088 (the row is staged in shared memory); ids int64 [rows, L] token history, L <= 160; cur_dev: device
+ * scalar, current length, 1 <= *cur_dev < L (otherwise the call writes nothing); unfinished: 1 byte per row.  Invalid ranges
+ * (temperature <= 0, top_k < 0, top_p outside [0, 1], penalty < 1) are rejected on the host. */
+int mmsum_sample_token(const float* logits, int64_t ld, int32_t rows, int32_t V, int64_t* ids, int32_t L, const int64_t* cur_dev,
+                       const uint64_t* seed_dev, int32_t min_length, int32_t ngram, int32_t eos, int32_t pad, float temperature,
+                       int32_t top_k, float top_p, float penalty, uint8_t* unfinished, int32_t* next_tok32, void* stream);
+
 /* ---- HBM-bound row kernels (d_model = 1024) ----------------------------------------------------- */
 /* fp32 -> bf16 (weight arena cast, feature cast) */
 int mmsum_cast_f32_bf16(const float* src, void* dst, int64_t n, void* stream);

@@ -91,6 +91,7 @@ EXPORTS = [
     "mmsum_gate_fwd", "mmsum_gate_bwd_u", "mmsum_gate_bwd_o", "mmsum_ce_fwd_bwd", "mmsum_prep_step",
     "mmsum_table_fwd", "mmsum_table_bits_bwd", "mmsum_grad_sumsq", "mmsum_adamw_step",
     "mmsum_embed_ln_decode", "mmsum_attn_decode_cross", "mmsum_attn_decode_self", "mmsum_beam_topk", "mmsum_beam_update",
+    "mmsum_sample_token",
 ]
 
 

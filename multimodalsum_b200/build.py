@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmmsum_b200.so")
 INFO = LIB + ".buildinfo.json"      # written next to the library by build(); git-ignored like the .so, travels with the snapshot
-SOURCES = ["gemm_sm100.cu", "attention_sm100.cu", "decode_sm100.cu", "beam_sm100.cu", "rowwise.cu", "optim.cu"]
+SOURCES = ["gemm_sm100.cu", "attention_sm100.cu", "decode_sm100.cu", "beam_sm100.cu", "sample_sm100.cu", "rowwise.cu", "optim.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--expt-relaxed-constexpr",

@@ -1,4 +1,4 @@
-"""Beam-search generation (BASELINE config 5, SURVEY §8 row a16) on the CUDA kernels of the training step.
+"""Beam-search generation (BASELINE config 5, SURVEY §8 row a16) and sampling on the CUDA kernels of the training step.
 
 Reference: BartForMultiEncConditionalGeneration.generate / _generate_beam_search / adjust_logits_during_generation
 (src/transformer/modeling_multimodalsum.py:2295-3101), postprocess_next_token_scores / calc_banned_ngram_tokens /
@@ -19,6 +19,9 @@ Design (B200-first, not the reference's):
     single `.item()` / `.tolist()` in the token loop (the reference loops over batch x beam in Python with host syncs
     every token, :2933-2983).  Termination is polled every few tokens through a pinned flag; steps taken after every
     business is done cannot change the result (finished businesses no longer admit hypotheses).
+  * sampling (`do_sample=True`, _generate_no_beam_search of the vendored transformers 3.0.2 generation_utils.py) runs the
+    same token loop with `SampleSearch` in place of `BeamSearch`: one kernel per token (csrc/sample_sm100.cu) processes the
+    scores, draws from a counter-based Philox stream and does the loop bookkeeping; `sample_scores` is its restatement.
 Review frames up to 208 tokens are supported (src/test.py uses 158 / 118).
 """
 import torch
@@ -198,10 +201,15 @@ class BeamSearch:
         self.cur_len += 1
         return self.beam_idx
 
+    def all_done(self):
+        """Device bool: every business is done (the token loop's stop flag)."""
+        return self.done.all()
+
     # -- result -----------------------------------------------------------------------------------------
-    def finalize(self):
-        """Unfinished businesses contribute their open beams (:3012-3026); best hypothesis per business, padded like the
-        reference's output (:3036-3061)."""
+    def finalize(self, num_return_sequences=1):
+        """Unfinished businesses contribute their open beams (:3012-3026); the `num_return_sequences` best hypotheses per
+        business in descending score order (rows i*n .. i*n+n-1 belong to business i), padded like the reference's output
+        (:3036-3061).  Row i*n is the n = 1 result (ties go to the lower pool slot, as argmax)."""
         k, cur = self.k, self.cur_len
         live = ~self.done
         norm = float(cur) ** self.length_penalty
@@ -209,9 +217,20 @@ class BeamSearch:
             row = self.row0[:, 0] + j
             self._admit(live, self.beam_scores[row] / norm, self.ids[row], cur)
         filled = self.slot_ids[None, :] < self.pool_n[:, None]
-        best = torch.where(filled, self.pool_score, torch.full_like(self.pool_score, NEG)).argmax(dim=1)
-        tok = self.pool_tok[self.rows, best]
-        lens = self.pool_len[self.rows, best]
+        masked = torch.where(filled, self.pool_score, torch.full_like(self.pool_score, NEG))
+        n = num_return_sequences
+        if n == 1:
+            best = masked.argmax(dim=1)
+            tok = self.pool_tok[self.rows, best]
+            lens = self.pool_len[self.rows, best]
+        else:
+            if n > k:
+                raise ValueError("num_return_sequences (%d) must not exceed num_beams (%d)" % (n, k))
+            order = torch.sort(masked, dim=1, descending=True, stable=True).indices[:, :n]
+            best = order.reshape(-1)
+            tok = self.pool_tok[self.rows[:, None], order].reshape(self.B * n, -1)
+            lens = self.pool_len[self.rows[:, None], order].reshape(-1)
+            self.out_scores = masked[self.rows.repeat_interleave(n), best]      # score of each returned row
         lo, hi = int(lens.min().item()), int(lens.max().item())
         if lo == hi:
             return tok[:, :hi].contiguous()
@@ -222,7 +241,7 @@ class BeamSearch:
 
 
 def beam_search(logits_fn, B, V, dev, num_beams=4, max_length=20, min_length=0, length_penalty=1.0, no_repeat_ngram_size=3,
-                early_stopping=True, pad=1, bos=0, eos=2, reorder_fn=None, poll_every=8):
+                early_stopping=True, pad=1, bos=0, eos=2, reorder_fn=None, poll_every=8, num_return_sequences=1):
     """_generate_beam_search (modeling_multimodalsum.py:2803-3067), do_sample=False.  `logits_fn(input_ids[N, cur_len])`
     returns the fp32 next-token logits [N, V] of the last position (N = B*num_beams, beams of a business adjacent);
     `reorder_fn(beam_idx)` re-orders an incremental decoder's caches (`_reorder_cache`, :3103-3115)."""
@@ -249,7 +268,219 @@ def beam_search(logits_fn, B, V, dev, num_beams=4, max_length=20, min_length=0, 
                 ev.record()
         if reorder_fn is not None and bs.cur_len < max_length:
             reorder_fn(beam_idx)
-    return bs.finalize()
+    return bs.finalize(num_return_sequences)
+
+
+# ---------------------------------------------------------------------------------------------------- sampling
+# Defaults of the reference's PretrainedConfig (vendored transformers 3.0.2 configuration_utils.py), which `generate` falls
+# back to for every argument left at None.
+SAMPLE_DEFAULTS = dict(do_sample=False, temperature=1.0, top_k=50, top_p=1.0, repetition_penalty=1.0, num_return_sequences=1)
+
+
+def validate_generate_args(num_beams, do_sample, temperature, top_k, top_p, repetition_penalty, num_return_sequences,
+                           bad_words_ids=None):
+    """The argument checks of GenerationMixin.generate (generation_utils.py, its asserts) as ValueError, plus what this
+    implementation does not cover as NotImplementedError.  Runs before any device work."""
+    def is_int(v):
+        return isinstance(v, int) and not isinstance(v, bool)
+    if not is_int(num_beams) or num_beams < 1:
+        raise ValueError("num_beams must be a positive integer, got %r" % (num_beams,))
+    if not temperature > 0:
+        raise ValueError("temperature must be > 0, got %r" % (temperature,))
+    if not is_int(top_k) or top_k < 0:
+        raise ValueError("top_k must be an integer >= 0, got %r" % (top_k,))
+    if not 0 <= top_p <= 1:
+        raise ValueError("top_p must be in [0, 1], got %r" % (top_p,))
+    if not repetition_penalty >= 1.0:
+        raise ValueError("repetition_penalty must be >= 1, got %r" % (repetition_penalty,))
+    if not is_int(num_return_sequences) or num_return_sequences < 1:
+        raise ValueError("num_return_sequences must be a positive integer, got %r" % (num_return_sequences,))
+    if num_beams == 1 and not do_sample and num_return_sequences > 1:
+        raise ValueError("greedy decoding (num_beams=1, do_sample=False) returns one sequence per input; "
+                         "num_return_sequences=%d needs do_sample=True or num_beams >= %d" % (num_return_sequences,
+                                                                                              num_return_sequences))
+    if num_beams > 1 and num_return_sequences > num_beams:
+        raise ValueError("num_return_sequences (%d) must not exceed num_beams (%d)" % (num_return_sequences, num_beams))
+    if bad_words_ids is not None:
+        raise NotImplementedError("bad_words_ids is not implemented")
+    if do_sample and num_beams > 1:
+        raise NotImplementedError("beam sampling (do_sample=True with num_beams > 1) is not implemented")
+    if not do_sample and repetition_penalty != 1.0:
+        raise NotImplementedError("repetition_penalty is implemented for do_sample=True only (greedy and beam search run "
+                                  "the beam-search path)")
+
+
+def resolve_generate_args(kw):
+    """`generate(**kw)` keyword arguments -> the keyword arguments of Generator.generate_from_memory.  None means the
+    default, as in the reference; everything is validated here, before any device work.  With do_sample=False and
+    num_return_sequences=1 the result is exactly the beam-search argument set."""
+    s = {k: (v if kw.get(k) is None else kw[k]) for k, v in SAMPLE_DEFAULTS.items()}
+    args = dict(num_beams=kw.get("num_beams") or 1, max_length=kw.get("max_length") or 20, min_length=kw.get("min_length") or 0,
+                length_penalty=1.0 if kw.get("length_penalty") is None else kw["length_penalty"],
+                no_repeat_ngram_size=kw.get("no_repeat_ngram_size") or 0,
+                early_stopping=bool(kw.get("early_stopping")), use_cache=kw.get("use_cache") is not False)
+    validate_generate_args(args["num_beams"], bool(s["do_sample"]), s["temperature"], s["top_k"], s["top_p"],
+                           s["repetition_penalty"], s["num_return_sequences"], kw.get("bad_words_ids"))
+    if s["do_sample"]:
+        args.update(do_sample=True, temperature=float(s["temperature"]), top_k=s["top_k"], top_p=float(s["top_p"]),
+                    repetition_penalty=float(s["repetition_penalty"]), num_return_sequences=s["num_return_sequences"])
+    elif s["num_return_sequences"] != 1:
+        args.update(num_return_sequences=s["num_return_sequences"])
+    return args
+
+
+def sample_scores(logits, ids, cur_len, min_length, no_repeat_ngram_size, temperature, top_k, top_p, repetition_penalty,
+                  eos):
+    """The score processing of one sampling step, restated on tensors: logits fp32 [N, V] of the last position, ids [N, >=
+    cur_len] the prefixes -> processed scores [N, V] with -inf for every token that cannot be drawn.  In the order of
+    _generate_no_beam_search (generation_utils.py):
+      1. postprocess_next_token_scores -> enforce_repetition_penalty_: each distinct id of the prefix (start token included)
+         once, score / penalty if > 0 (>= 0 in the reference's `< 0 ? * : /`), * penalty if < 0;
+      2. ... EOS score -inf while cur_len < min_length;
+      3. ... calc_banned_ngram_tokens: a token that would complete an n-gram already in the prefix is -inf;
+      4. NO adjust_logits_during_generation: the reference calls it on the beam path only (forced BOS / EOS do not apply);
+      5. scores / temperature;
+      6. top_k_top_p_filtering(min_tokens_to_keep=1): top-k keeps every token >= the k-th largest score (ties at the k-th
+         value survive; k = min(top_k, V), 0 = off); top-p on what is left keeps a token iff the softmax mass ranked strictly
+         before it is <= top_p (the crossing token and the top token are kept).  Equal scores are ranked by ascending
+         token id: that tie rule is ours (torch.sort leaves the order of equal values unspecified).
+    The draw is softmax over the result (7)."""
+    scores = logits.float().clone()
+    N, V = scores.shape
+    prev = ids[:, :cur_len]
+    if repetition_penalty != 1.0:
+        seen = torch.zeros(N, V, dtype=torch.bool, device=scores.device).scatter_(1, prev, True)
+        scores = torch.where(seen, torch.where(scores < 0, scores * repetition_penalty, scores / repetition_penalty), scores)
+    if cur_len < min_length:
+        scores[:, eos] = NEG
+    n = no_repeat_ngram_size
+    if n > 0 and cur_len + 1 >= n:
+        for r in range(N):
+            gen = prev[r].tolist()
+            tail = tuple(gen[cur_len - n + 1:])
+            banned = [gen[i + n - 1] for i in range(cur_len - n + 1) if tuple(gen[i:i + n - 1]) == tail]
+            if banned:
+                scores[r, banned] = NEG
+    if temperature != 1.0:
+        scores = scores / temperature
+    if top_k > 0:
+        kth = torch.topk(scores, min(top_k, V), dim=-1).values[:, -1:]
+        scores = scores.masked_fill(scores < kth, NEG)
+    if top_p < 1.0:
+        sorted_s, sorted_i = torch.sort(scores, dim=-1, descending=True, stable=True)
+        cum = torch.softmax(sorted_s, dim=-1).cumsum(dim=-1)
+        remove = cum > top_p
+        remove[:, 1:] = remove[:, :-1].clone()
+        remove[:, 0] = False
+        scores = scores.masked_fill(remove.scatter(1, sorted_i, remove), NEG)
+    return scores
+
+
+class SampleSearch:
+    """State of one batched sampling loop (_generate_no_beam_search with do_sample=True): `B` businesses x `n` samples,
+    rows i*n .. i*n+n-1 belong to business i and are never re-ranked (the decoder's slot table stays the identity).
+
+      ids [N, max_length]   token histories (decoder start token = eos first), pad after a row's EOS by construction
+      unfinished [N]        uint8, 0 once the row appended EOS
+      seed [1]              int64 Philox key, drawn from torch's default generator of the device at every reset()
+
+    Every piece of per-step state is a fixed device buffer updated in place and the length enters as the device scalar
+    `cur_t`, so one step records into a CUDA graph.  On CUDA the step is csrc/sample_sm100.cu (no other path); on the CPU it
+    is `sample_scores` + torch.multinomial, the tensor restatement the kernel is tested against."""
+
+    def __init__(self, B, V, dev, num_return_sequences, max_length, min_length, no_repeat_ngram_size, temperature, top_k,
+                 top_p, repetition_penalty, pad, eos):
+        n = num_return_sequences
+        self.B, self.n, self.V, self.dev = B, n, V, dev
+        self.max_length, self.min_length, self.ngram = max_length, min_length, no_repeat_ngram_size
+        self.temperature, self.top_k, self.top_p, self.penalty = temperature, top_k, top_p, repetition_penalty
+        self.pad, self.eos = pad, eos
+        N = B * n
+        self.ids = torch.empty((N, max_length), dtype=torch.long, device=dev)
+        self.unfinished = torch.empty(N, dtype=torch.uint8, device=dev)
+        self.cur_t = torch.empty(1, dtype=torch.long, device=dev)
+        self.seed = torch.zeros(1, dtype=torch.long, device=dev)
+        self.kernel_path = torch.device(dev).type == "cuda"
+        self.dec_ids32 = None
+        self._gen = None
+        self._clear()
+
+    def _clear(self):
+        self.ids.fill_(self.pad)
+        self.ids[:, 0] = self.eos
+        self.unfinished.fill_(1)
+        self.cur_len = 1
+        self.cur_t.fill_(1)
+
+    def reset(self):
+        """Back to the start state, in place, and this call's seed: one draw from torch's default generator of the device
+        (no host sync), so torch.manual_seed makes a call reproducible and consecutive calls differ."""
+        self._clear()
+        self.seed.random_()
+        if not self.kernel_path:
+            self._gen = torch.Generator().manual_seed(int(self.seed.item()))
+
+    def attach_decoder(self, ids32, hist):
+        """The decoder's next-token input [N] (int32), written by the sampler.  The slot table needs no work: rows are never
+        re-ranked and the decode self-attention writes hist[n][t] = n itself."""
+        self.dec_ids32 = ids32
+
+    def all_done(self):
+        return self.unfinished.eq(0).all()
+
+    def advance(self, logits):
+        """logits: fp32 [N, V] next-token logits of the current prefixes; appends one token per row."""
+        if self.kernel_path:
+            ops.sample_token(logits, self.V, self.ids, self.cur_t, self.seed, self.min_length, self.ngram, self.eos, self.pad,
+                             self.temperature, self.top_k, self.top_p, self.penalty, self.unfinished, self.dec_ids32)
+        else:
+            cur = self.cur_len
+            scores = sample_scores(logits, self.ids, cur, self.min_length, self.ngram, self.temperature, self.top_k,
+                                   self.top_p, self.penalty, self.eos)
+            tok = torch.multinomial(torch.softmax(scores, dim=-1), 1, generator=self._gen).squeeze(1)
+            tok = torch.where(self.unfinished.bool(), tok, torch.full_like(tok, self.pad))     # tokens_to_add
+            self.ids[:, cur] = tok
+            self.unfinished.mul_((tok != self.eos).to(torch.uint8))
+            if self.dec_ids32 is not None:
+                self.dec_ids32.copy_(tok)
+        self.cur_t.add_(1)
+        self.cur_len += 1
+
+    def finalize(self):
+        """The reference returns input_ids when the loop ends: at max_length, or right after the step in which the last row
+        appended EOS.  Steps the token loop ran after that (it polls the stop flag with a lag) only appended pad."""
+        ids = self.ids[:, :self.cur_len]
+        if not (bool(self.unfinished.any()) or self.cur_len <= 1):
+            first_eos = (ids[:, 1:] == self.eos).long().argmax(dim=1) + 1
+            ids = ids[:, :int(first_eos.max()) + 1]
+        return ids.clone()                    # never a view of the plan's buffer: the next call overwrites it
+
+
+def sample_search(logits_fn, B, V, dev, num_return_sequences=1, max_length=20, min_length=0, no_repeat_ngram_size=0,
+                  temperature=1.0, top_k=50, top_p=1.0, repetition_penalty=1.0, pad=1, eos=2, poll_every=8):
+    """_generate_no_beam_search with do_sample=True.  `logits_fn(input_ids[N, cur_len])` returns the fp32 next-token logits
+    [N, V] of the last position (N = B * num_return_sequences, the rows of a business adjacent)."""
+    ss = SampleSearch(B, V, dev, num_return_sequences, max_length, min_length, no_repeat_ngram_size, temperature, top_k,
+                      top_p, repetition_penalty, pad, eos)
+    ss.reset()
+    cuda = torch.device(dev).type == "cuda"
+    flag = torch.zeros(1, dtype=torch.bool, pin_memory=True) if cuda else None
+    ev = None
+    while ss.cur_len < max_length:
+        ss.advance(logits_fn(ss.ids[:, :ss.cur_len]))
+        if not cuda:
+            if bool(ss.all_done()):
+                break
+        else:
+            if ev is not None and ev.query():
+                if bool(flag[0]):
+                    break
+                ev = None
+            if ev is None and ss.cur_len % poll_every == 0:
+                flag.copy_(ss.all_done().reshape(1), non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record()
+    return ss.finalize()
 
 
 class DecodeState:
@@ -444,14 +675,20 @@ class Generator:
         w["hist"].copy_(w["hist_alt"])
 
     # ------------------------------------------------------------------ fused token loop (one CUDA graph per token)
-    def _plan(self, mem, k, kw):
-        """Static buffers + the recorded token step for one (memory layout, beam-search setting): the K|V projections of a
+    def _plan(self, mem, k, kw, sample=None):
+        """Static buffers + the recorded token step for one (memory layout, search setting): the K|V projections of a
         new memory are written into the plan's buffers and the same CUDA graph is replayed — capture and instantiation
-        (~0.15 s for ~220 nodes) are paid once per shape, not once per generate() call."""
+        (~0.15 s for ~220 nodes) are paid once per shape, not once per generate() call.  `k` rows per business: beams, or
+        samples when `sample` holds the sampling parameters (a SampleSearch then replaces the BeamSearch)."""
         cfg = self.eng.cfg
         dev = mem.MEM.device
-        key = (mem.B, k, tuple(mem.mods), mem.MEM.shape[0], mem.Et, mem.pres is None, kw["max_length"], kw["min_length"],
-               float(kw["length_penalty"]), kw["no_repeat_ngram_size"], bool(kw["early_stopping"]), str(dev))
+        if sample is None:
+            key = (mem.B, k, tuple(mem.mods), mem.MEM.shape[0], mem.Et, mem.pres is None, kw["max_length"], kw["min_length"],
+                   float(kw["length_penalty"]), kw["no_repeat_ngram_size"], bool(kw["early_stopping"]), str(dev))
+        else:
+            key = ("sample", mem.B, k, tuple(mem.mods), mem.MEM.shape[0], mem.Et, mem.pres is None, kw["max_length"],
+                   kw["min_length"], kw["no_repeat_ngram_size"], sample["temperature"], sample["top_k"], sample["top_p"],
+                   sample["repetition_penalty"], str(dev))
         plan = self._plans.get(key)
         if plan is not None:
             return plan
@@ -464,8 +701,13 @@ class Generator:
         N = mem.B * k
         st.cws = self._decode_ws(st, N, dev)
         st.cws["fused"] = True
-        bs = BeamSearch(mem.B, cfg.vocab_size, dev, k, kw["max_length"], kw["min_length"], kw["length_penalty"],
-                        kw["no_repeat_ngram_size"], kw["early_stopping"], cfg.pad_token_id, cfg.bos_token_id, cfg.eos_token_id)
+        if sample is None:
+            bs = BeamSearch(mem.B, cfg.vocab_size, dev, k, kw["max_length"], kw["min_length"], kw["length_penalty"],
+                            kw["no_repeat_ngram_size"], kw["early_stopping"], cfg.pad_token_id, cfg.bos_token_id, cfg.eos_token_id)
+        else:
+            bs = SampleSearch(mem.B, cfg.vocab_size, dev, k, kw["max_length"], kw["min_length"], kw["no_repeat_ngram_size"],
+                              sample["temperature"], sample["top_k"], sample["top_p"], sample["repetition_penalty"],
+                              cfg.pad_token_id, cfg.eos_token_id)
         bs.attach_decoder(st.cws["ids"], st.cws["hist"])
         plan = dict(st=st, bs=bs, graph=None, captured=False)
         if len(self._plans) >= 4:                     # a handful of shapes at most; drop the oldest
@@ -474,16 +716,17 @@ class Generator:
         return plan
 
     @torch.no_grad()
-    def _fused_beam_search(self, mem, rd, poll_every=8, **kw):
+    def _fused_beam_search(self, mem, rd, poll_every=8, sample=None, num_return_sequences=1, **kw):
         """Decoder step + beam update + cache re-ranking of one token recorded ONCE and replayed: the host issues a single
         graph launch per token (the reference runs ~47 k eager ops and several host syncs per token, :2857-3010).  The very
         first token of a new shape runs kernel by kernel (one-time function attributes, allocator warm-up), the capture
-        follows it; later calls with the same shape replay the graph from the first token on."""
+        follows it; later calls with the same shape replay the graph from the first token on.  With `sample` (the sampling
+        parameters) the same loop runs the sampler over num_beams = samples per business instead of the beam update."""
         import os
         eng = self.eng
         cfg = eng.cfg
         k = kw.pop("num_beams")
-        plan = self._plan(mem, k, kw)
+        plan = self._plan(mem, k, kw, sample)
         st, bs = plan["st"], plan["bs"]
         w, smem = st.cws, st.mem
         # ---- this call's memory: validity bookkeeping copied, K|V projected straight into the plan's buffers
@@ -516,7 +759,7 @@ class Generator:
 
         max_length = kw["max_length"]
         if max_length <= 1:
-            return bs.finalize()
+            return bs.finalize() if sample is not None else bs.finalize(num_return_sequences)
         if not plan["captured"]:
             plan["captured"] = True
             token_step()
@@ -547,34 +790,48 @@ class Generator:
                     break
                 ev = None
             if ev is None and bs.cur_len % poll_every == 0:
-                flag.copy_(bs.done.all().reshape(1), non_blocking=True)
+                flag.copy_(bs.all_done().reshape(1), non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record()
         self.last_decode_steps = bs.cur_len - 1
-        return bs.finalize()
+        return bs.finalize() if sample is not None else bs.finalize(num_return_sequences)
 
     # ------------------------------------------------------------------ public entry points
     @torch.no_grad()
     def generate_from_memory(self, mem, rating_diff=None, num_beams=4, max_length=20, min_length=0, length_penalty=1.0,
-                             no_repeat_ngram_size=3, early_stopping=True, use_cache=True):
-        """`bart_model.generate(text_hiddens, ..., rating_diff=..., num_beams=...)` as src/test.py:156-158 calls it."""
+                             no_repeat_ngram_size=3, early_stopping=True, use_cache=True, do_sample=False, temperature=1.0,
+                             top_k=50, top_p=1.0, repetition_penalty=1.0, num_return_sequences=1):
+        """`bart_model.generate(text_hiddens, ..., rating_diff=..., num_beams=...)` as src/test.py:156-158 calls it ->
+        token ids [B * num_return_sequences, <= max_length], the rows of a business adjacent.  do_sample=True (num_beams
+        must be 1): _generate_no_beam_search with num_return_sequences samples per business on the device sampler
+        (`SampleSearch`); otherwise beam search, returning the num_return_sequences best hypotheses per business."""
+        validate_generate_args(num_beams, do_sample, temperature, top_k, top_p, repetition_penalty, num_return_sequences)
         cfg = self.model.cfg
         B, dev = mem.B, mem.MEM.device
+        rows = num_return_sequences if do_sample else num_beams
         rd = torch.zeros(B, device=dev) if rating_diff is None else rating_diff.reshape(B).float()
-        rd = rd.repeat_interleave(num_beams).contiguous()
-        if num_beams > 8:
-            use_cache = False                     # the decode attention kernel holds up to 8 beams per business
+        rd = rd.repeat_interleave(rows).contiguous()
+        if rows > 8:
+            use_cache = False                     # the decode attention kernel holds up to 8 rows (beams, samples) per business
+        sample = dict(temperature=float(temperature), top_k=int(top_k), top_p=float(top_p),
+                      repetition_penalty=float(repetition_penalty)) if do_sample else None
         if use_cache:
             eng = self._engine(dev)
             eng.refresh_bf16_weights()
-            return self._fused_beam_search(mem, rd, num_beams=num_beams, max_length=max_length, min_length=min_length,
+            return self._fused_beam_search(mem, rd, num_beams=rows, max_length=max_length, min_length=min_length,
                                            length_penalty=length_penalty, no_repeat_ngram_size=no_repeat_ngram_size,
-                                           early_stopping=early_stopping)
-        st = self.prepare(mem, num_beams)
+                                           early_stopping=early_stopping, sample=sample,
+                                           num_return_sequences=num_return_sequences)
+        st = self.prepare(mem, rows)
         logits_fn, reorder_fn = (lambda ids: self.last_logits(st, ids, rd)), None
+        if sample is not None:
+            return sample_search(logits_fn, B, cfg.vocab_size, dev, num_return_sequences=rows, max_length=max_length,
+                                 min_length=min_length, no_repeat_ngram_size=no_repeat_ngram_size, pad=cfg.pad_token_id,
+                                 eos=cfg.eos_token_id, **sample)
         return beam_search(logits_fn, B, cfg.vocab_size, dev, num_beams=num_beams, max_length=max_length, min_length=min_length,
                            length_penalty=length_penalty, no_repeat_ngram_size=no_repeat_ngram_size, early_stopping=early_stopping,
-                           pad=cfg.pad_token_id, bos=cfg.bos_token_id, eos=cfg.eos_token_id, reorder_fn=reorder_fn)
+                           pad=cfg.pad_token_id, bos=cfg.bos_token_id, eos=cfg.eos_token_id, reorder_fn=reorder_fn,
+                           num_return_sequences=num_return_sequences)
 
     @torch.no_grad()
     def generate(self, reviews, reviews_mask, field, field_value, img, img_mask, rating_diff=None, **kw):

@@ -213,18 +213,11 @@ class _BartLMBase(nn.Module, _EngineRoot):
 
     @torch.no_grad()
     def _lm_generate(self, hiddens, masks, rating_diff, kw):
-        from .generation import Generator
+        from .generation import Generator, resolve_generate_args
+        args = resolve_generate_args(kw)     # defaults and validation (beam sampling, bad_words_ids: NotImplementedError)
         eng = _engine_of(self, hiddens[0].device)
         root = self._root_ref() if getattr(self, "_root_ref", None) is not None else self
         mem = INF.build_memory(eng, hiddens, masks)
-        unsupported = {k: v for k, v in kw.items() if k in ("do_sample", "top_k", "top_p", "temperature", "repetition_penalty",
-                                                            "bad_words_ids", "num_return_sequences") and v not in (None, False, 1, 1.0)}
-        if unsupported:
-            raise NotImplementedError("only beam search / greedy decoding are implemented (src/test.py path): %s" % sorted(unsupported))
-        args = dict(num_beams=kw.get("num_beams") or 1, max_length=kw.get("max_length") or 20, min_length=kw.get("min_length") or 0,
-                    length_penalty=1.0 if kw.get("length_penalty") is None else kw["length_penalty"],
-                    no_repeat_ngram_size=kw.get("no_repeat_ngram_size") or 0,
-                    early_stopping=bool(kw.get("early_stopping")), use_cache=kw.get("use_cache") is not False)
         gen = getattr(root, "_generator", None)
         if gen is None:                       # one Generator per model: it caches the recorded token-step graphs per shape
             gen = Generator(root)
@@ -248,7 +241,8 @@ class BartForMultiEncConditionalGeneration(_BartLMBase):
 
     def generate(self, text_hiddens, text_attention_mask, table_hiddens, table_attention_mask, img_hiddens, img_attention_mask,
                  input_ids=None, rating_diff=None, **kw):
-        """Beam search over the given memories (:2295-2693) -> token ids [B, <= max_length]."""
+        """Beam search, greedy decoding or sampling (do_sample=True, temperature, top_k, top_p, repetition_penalty) over the
+        given memories (:2295-2693) -> token ids [B * num_return_sequences, <= max_length]."""
         return self._lm_generate([text_hiddens, table_hiddens, img_hiddens],
                                  [text_attention_mask, table_attention_mask, img_attention_mask], rating_diff, kw)
 

@@ -296,6 +296,15 @@ def beam_update(cand_val, cand_tok, ids, beam_scores, done, pool_score, pool_tok
                                        int(bool(early_stopping)), C.c_float(length_penalty), _stream()), "mmsum_beam_update")
 
 
+def sample_token(logits, V, ids, cur_dev, seed_dev, min_length, ngram, eos, pad, temperature, top_k, top_p, penalty, unfinished,
+                 next_tok32=None):
+    """One sampled token per row, loop bookkeeping included (see include/mmsum_b200.h); every argument is device state."""
+    check(_lib.lib().mmsum_sample_token(_ptr(logits), C.c_int64(logits.stride(0)), logits.shape[0], V, _ptr(ids), ids.shape[1],
+                                        _ptr(cur_dev), _ptr(seed_dev), min_length, ngram, eos, pad, C.c_float(temperature),
+                                        top_k, C.c_float(top_p), C.c_float(penalty), _ptr(unfinished), _ptr(next_tok32),
+                                        _stream()), "mmsum_sample_token")
+
+
 def prep_step(reviews, reviews_mask, rating, table_valid, img_mask, **kw):
     a = _lib.PrepArgs()
     for k, v in kw.items():
