@@ -19,6 +19,7 @@ import weakref
 
 import torch
 
+from . import layers as L
 from . import ops
 from .synth import ModelConfig
 
@@ -318,13 +319,14 @@ class StepEngine:
             w["enc_x0"] = bf(Te, D)
             w["enc_m0"], w["enc_r0"] = f32(Te), f32(Te)
         dec = []
+        U = bf(2, T, D) if cfg.multimodal else None      # gate pre-activations: forward scratch shared by the layers
         for l in range(L_d):
             d = dict(x=bf(T, D), qkv=bf(T, 3 * D), ctx=bf(T, D), o=bf(T, D), x1=bf(T, D), qc=bf(T, D), kv=bf(Tm, 2 * D),
                      A3=bf(nm, T, D), O3=bf(nm, T, D), x2=bf(T, D), h=bf(T, FF), a=bf(T, FF), f=bf(T, D),
                      lse=f32(N, H, 1, S), lse_c=f32(N, H, Et, S),
                      m1=f32(T), r1=f32(T), m2=f32(T), r2=f32(T), m3=f32(T), r3=f32(T))
             if cfg.multimodal:
-                d.update(AB=bf(2, T, D), yc=bf(T, D))
+                d.update(U=U, AB=bf(2, T, D), yc=bf(T, D))
             dec.append(d)
         w["dec"] = dec
         w["dec_m0"], w["dec_r0"] = f32(T), f32(T)
@@ -351,7 +353,7 @@ class StepEngine:
         w["dA3"] = bf(nm, T, D)
         w["dO3"] = bf(nm, T, D)
         if cfg.multimodal:
-            w.update(U=bf(2, T, D), dU=bf(2, T, D), dca=bf(T, 2 * D), dcb=bf(T, 2 * D))
+            w.update(dU=bf(2, T, D), dca=bf(T, 2 * D), dcb=bf(T, 2 * D))
         if F > 0:
             w.update(dtab_h=bf(B * F, D), dtabX=bf(B * F, 2 * D))
         self.ws_full, self.ws_key = w, key
@@ -362,37 +364,23 @@ class StepEngine:
         # the step number is added inside the kernels from the device-resident counter `step_dev` (graph-replayable)
         return kind * 64 + layer
 
-    def _self_attn_args(self, w, qkv, out, lse, key_valid, causal, bwd=None, frame=None):
-        """frame: rows per sequence (the encoder's trimmed frame; None = 128)."""
-        D, H, S = self.cfg.d_model, self.cfg.heads, w["S"]
+    def _self_attn_args(self, w, qkv, out, lse, key_valid, causal, dqkv=None, frame=None):
+        """frame: rows per sequence (the encoder's trimmed frame; None = 128).  dqkv: the backward's gradient buffer."""
+        D, S = self.cfg.d_model, w["S"]
         fr = S if frame is None else frame
-        kw = dict(Q=qkv, ldq=3 * D, q_col=0, KV=qkv, ldkv=3 * D, k_col=D, v_col=2 * D, O=out, ldo=D, LSE=lse,
-                  key_valid=key_valid, ent_valid=None, inv_n=None, n_qseq=w["N"], H=H, R=1, causal=int(causal), E_total=1,
-                  scale=self.cfg.head_dim ** -0.5, q_rows=(0 if fr == S else fr), mods=[(0, 0, 1, fr, 0, 0)])
-        if bwd is not None:
-            dqkv = bwd
-            kw.update(DELTA=w["delta"], dQ=dqkv, lddq=3 * D, dq_col=0, dKV=dqkv, lddkv=3 * D, dk_col=D, dv_col=2 * D)
-        return ops.attn_args(**kw)
+        bwd = {} if dqkv is None else dict(DELTA=w["delta"], dQ=dqkv, lddq=3 * D, dq_col=0, dKV=dqkv, lddkv=3 * D, dk_col=D,
+                                           dv_col=2 * D)
+        return L.self_attn_args(self, qkv, out, lse, key_valid, w["N"], causal, fr, q_rows=(0 if fr == S else fr), **bwd)
 
-    def _cross_attn_args(self, w, qc, kv, out3, lse, bwd=None):
-        D, H, S, T = self.cfg.d_model, self.cfg.heads, w["S"], w["T"]
-        B, R, F, n_img, ik, Tt = w["B"], w["R"], w["F"], w["n_img"], w["img_keys"], w["Tt"]
-        mods, eb = [], 0
-        if Tt > 0:
-            mods.append((0, 0, R, w["S_enc"], 1, 0))  # text: leave-one-out over the R reviews of the business (encoder frames)
-            eb = R
-        if F > 0:
-            mods.append((Tt, len(mods) * T * D, 1, F, 0, eb))
-            eb += 1
-        if n_img > 0:
-            mods.append((Tt + B * F, len(mods) * T * D, n_img, ik, 0, eb))
-        kw = dict(Q=qc, ldq=D, q_col=0, KV=kv, ldkv=2 * D, k_col=0, v_col=D, O=out3, ldo=D, LSE=lse,
-                  key_valid=w["mem_valid"], ent_valid=w["ent_valid"], inv_n=w["inv_n"], n_qseq=w["N"], H=H, R=R, causal=0,
-                  E_total=w["Et"], scale=self.cfg.head_dim ** -0.5, mods=mods)
-        if bwd is not None:
-            dqc, dkv = bwd
-            kw.update(DELTA=w["delta"], dQ=dqc, lddq=D, dq_col=0, dKV=dkv, lddkv=dkv.stride(0), dk_col=0, dv_col=D)
-        return ops.attn_args(**kw)
+    def _cross_attn_args(self, w, qc, kv, out3, lse, dqc=None, dkv=None):
+        """Memory rows = [text B*R*S_enc (leave-one-out over the R reviews of a business) | table B*F | image]."""
+        D, B, R, F, n_img, Tt = self.cfg.d_model, w["B"], w["R"], w["F"], w["n_img"], w["Tt"]
+        mods = ([(0, R, w["S_enc"])] if Tt > 0 else []) + ([(Tt, 1, F)] if F > 0 else []) + \
+               ([(Tt + B * F, n_img, w["img_keys"])] if n_img > 0 else [])
+        bwd = {} if dqc is None else dict(DELTA=w["delta"], dQ=dqc, lddq=D, dq_col=0, dKV=dkv, lddkv=dkv.stride(0), dk_col=0,
+                                          dv_col=D)
+        return L.cross_attn_args(self, qc, kv, out3, lse, mods, w["mem_valid"], w["ent_valid"], w["inv_n"], w["N"], R,
+                                 loo=Tt > 0, **bwd)
 
     # ------------------------------------------------------------------ forward
     def _stage_bookkeeping(self, w, batch, img_mask_u8):
@@ -497,20 +485,20 @@ class StepEngine:
         if not self.bound:
             raise RuntimeError("engine.bind(named_parameters) first")
         cfg = self.cfg
-        D, FF, V = cfg.d_model, cfg.ffn_dim, cfg.vocab_size
+        V = cfg.vocab_size
         has_text, gates = cfg.text_memory, cfg.multimodal
         if has_text:
             B, R, S = batch.reviews.shape
         else:
             (B, S), R = batch.labels.shape, 1
-        F = {None: 0, "yelp": 47, "amazon": 133}[cfg.table]
+        F = L.table_dims(cfg.table)
         n_img, img_keys = (batch.img.shape[1], batch.img.shape[2]) if cfg.image else (0, 0)
         if S != 128:
             raise ValueError("the attention kernels are specialised to 128-token frames")
         S_enc = self._encoder_frame(batch, S) if has_text else S
         w = self._alloc(B, R, S, F, n_img, img_keys, S_enc)
         self.ws = w
-        T, Tt, Tm, Te = w["T"], w["Tt"], w["Tm"], w["Te"]
+        T, Tt, Te = w["T"], w["Tt"], w["Te"]
         w["batch"] = batch                 # backward re-reads the bit-code table fields
         self.step_count += 1
         self.step_dev.add_(1)
@@ -523,19 +511,12 @@ class StepEngine:
         if refresh:
             self.refresh_bf16_weights()
         bm = "bart_model.model."
-        g = ops.gemm
+        drop = lambda kind, l: (pd, seed, self._sid(kind, l), self.step_dev)
 
         # ---- table front end + step bookkeeping (integer work, bit-exact)
         img_mask_u8 = None
         if F > 0:
-            t = "table_encoder."
-            W1name = t + ("hours_embedding.weight" if cfg.table == "yelp" else "price_embedding.weight")
-            if cfg.table == "yelp":
-                W0, W1 = self.w32(t + "rating_embedding.weight"), self.w32(W1name)
-            else:
-                W0, W1 = self.w32(W1name), self.w32(t + "rating_embedding.weight")
-            ops.table_fwd(cfg.table, B, self.w32(bm + "shared.weight"), batch.field, batch.field_value, W0, W1,
-                          w["tabX"], w["tab_valid"])
+            L.table_embed(self, batch.field, batch.field_value, w["tabX"], w["tab_valid"])
         if n_img > 0:
             img_mask_u8 = batch.img_mask.view(torch.uint8) if batch.img_mask.dtype == torch.bool else batch.img_mask
         if has_text:
@@ -550,70 +531,54 @@ class StepEngine:
             self._stage_bookkeeping(w, batch, img_mask_u8)
         MEM = w["MEM"]
         if F > 0:
-            t = "table_encoder."
-            g(w["tabX"], self.w16(t + "fc.weight"), w["tab_h"], bias=self.w32(t + "fc.bias"), act=ops.ACT_RELU)
-            g(w["tab_h"], self.w16(t + "linear.weight"), MEM[Tt:Tt + B * F])
+            L.table_project(self, w["tabX"], w["tab_h"], MEM[Tt:Tt + B * F])
         if n_img > 0:
             img = batch.img.reshape(B * n_img * img_keys, 1024)
             if img.dtype == torch.float32:
                 ops.cast_bf16(img.contiguous(), w["img16"])
                 img = w["img16"]
             w["img_in"] = img
-            g(img, self.w16("img_encoder.linear.weight"), MEM[Tt + B * F:])
+            ops.gemm(img, self.w16("img_encoder.linear.weight"), MEM[Tt + B * F:])
 
         # ---- encoder (BartEncoder.forward :346-404)
         if has_text:
-            pre = bm + "encoder."
             x = w["enc_x0"]
-            ops.embed_ln_fwd(w["enc_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"), None, None,
-                             self.w32(pre + "layernorm_embedding.weight"), self.w32(pre + "layernorm_embedding.bias"),
-                             x, w["enc_m0"], w["enc_r0"], Te, S_enc, pd, seed, self._sid(0, 0), step_dev=self.step_dev)
+            ops.embed_ln_fwd(w["enc_ids"], *L.embed_params(self, "encoder", None), x, w["enc_m0"], w["enc_r0"], Te, S_enc, *drop(0, 0))
             L_e = cfg.encoder_layers
             for l in range(L_e):
                 a = w["enc"][l]
                 a["x"] = x
-                lp = pre + "layers.%d." % l
+                lp = bm + "encoder.layers.%d." % l
                 out = MEM[:Te] if l == L_e - 1 else w["enc"][l + 1]["x"]
-                self._self_block_fwd(w, a, lp, x, w["enc_valid"], False, l, 1, frame=S_enc)
-                self._ffn_block_fwd(a, lp, a["x1"], out, "m2", "r2", l, 2)
+                attend = lambda qkv, ctx, a=a: ops.attn_fwd(self._self_attn_args(w, qkv, ctx, a["lse"], w["enc_valid"], False,
+                                                                                 frame=S_enc))
+                L.self_block(self, lp, x, a, attend, (a["m1"], a["r1"]), drop(1, l))
+                L.ffn_block(self, lp, a["x1"], a, out, (a["m2"], a["r2"]), drop(2, l), dact=a["h"])   # a["h"]: GELU'
                 x = out
 
         # ---- decoder, batched leave-one-out (BartDecoder.forward :530-660 over 9·B sequences)
-        pre = bm + "decoder."
         L_d = cfg.decoder_layers
         x = w["dec"][0]["x"]
-        ops.embed_ln_fwd(w["dec_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"),
-                         w["rating_diff"], self.w32(pre + "rating_embeddings"),
-                         self.w32(pre + "layernorm_embedding.weight"), self.w32(pre + "layernorm_embedding.bias"),
-                         x, w["dec_m0"], w["dec_r0"], T, S, pd, seed, self._sid(3, 0), step_dev=self.step_dev)
+        ops.embed_ln_fwd(w["dec_ids"], *L.embed_params(self, "decoder", w["rating_diff"]), x, w["dec_m0"], w["dec_r0"], T, S,
+                         *drop(3, 0))
         for l in range(L_d):
             a = w["dec"][l]
-            lp = pre + "layers.%d." % l
-            c = lp + "encoder_attn."
+            lp = bm + "decoder.layers.%d." % l
             out = w["x_out"] if l == L_d - 1 else w["dec"][l + 1]["x"]
-            self._self_block_fwd(w, a, lp, a["x"], w["dec_valid"], True, l, 4)
-            # cross-attention block (SelfAttention.forward multimodal branch :722-745)
-            g(a["x1"], self.w16(c + "q_proj.weight"), a["qc"], bias=self.w32(c + "q_proj.bias"))
-            g(MEM, self.w16(c + "k_proj.weight", c + "v_proj.weight"), a["kv"], bias=self.w32(c + "k_proj.bias", c + "v_proj.bias"))
-            ops.attn_fwd(self._cross_attn_args(w, a["qc"], a["kv"], a["A3"], a["lse_c"]))
-            nm = a["A3"].shape[0]
-            g(a["A3"].view(nm * T, D), self.w16(c + "out_proj.weight"), a["O3"].view(nm * T, D), bias=self.w32(c + "out_proj.bias"))
-            if gates:
-                U = w["U"]
-                ops.gemm_cat(a["O3"][0], a["O3"][1], self.w16(c + "alpha_proj.weight"), U[0], bias=self.w32(c + "alpha_proj.bias"))
-                ops.gemm_cat(a["O3"][0], a["O3"][2], self.w16(c + "beta_proj.weight"), U[1], bias=self.w32(c + "beta_proj.bias"))
-                ops.gate_fwd(a["O3"], U, w["pres"], a["yc"], a["AB"], T, R * S, D)
-                yc = a["yc"]
-            else:
-                yc = a["O3"][0]
-            ops.add_ln_fwd(a["x1"], yc, self.w32(lp + "encoder_attn_layer_norm.weight"), self.w32(lp + "encoder_attn_layer_norm.bias"),
-                           a["x2"], a["m2"], a["r2"], pd, seed, self._sid(5, l), step_dev=self.step_dev)
-            self._ffn_block_fwd(a, lp, a["x2"], out, "m3", "r3", l, 6)
+            attend = lambda qkv, ctx, a=a: ops.attn_fwd(self._self_attn_args(w, qkv, ctx, a["lse"], w["dec_valid"], True))
+
+            def attend_mem(qc, A3, a=a, l=l):
+                L.project_kv(self, MEM, l, a["kv"])     # this layer's K|V of the memory, kept for the backward
+                ops.attn_fwd(self._cross_attn_args(w, qc, a["kv"], A3, a["lse_c"]))
+
+            L.self_block(self, lp, a["x"], a, attend, (a["m1"], a["r1"]), drop(4, l))
+            L.cross_block(self, lp, a["x1"], a, attend_mem, (a["m2"], a["r2"]), drop(5, l), w["pres"], R * S)
+            L.ffn_block(self, lp, a["x2"], a, out, (a["m3"], a["r3"]), drop(6, l), dact=a["h"])
             x = out
 
         # ---- LM head + loss (:2281, src/utils.py:32-38); mean over all 9·B·128 rows == mean of the 9 pass means
         logits = w["logits"]
-        g(x, self.w16(bm + "shared.weight"), logits[:, :V], bias=self.w32_flb(), raster_m_fast=True)
+        ops.gemm(x, self.w16(bm + "shared.weight"), logits[:, :V], bias=self.w32_flb(), raster_m_fast=True)
         ops.ce_fwd_bwd(logits, V, w["labels"], label_smoothing, 0.0, None, w["loss_rows"], w["loss"], 1.0 / T, False,
                        lse_rows=w["lse_rows"])
         return w["loss"]
@@ -640,23 +605,6 @@ class StepEngine:
 
     def w32_flb(self):
         return self.final_logits_bias.view(-1) if getattr(self, "final_logits_bias", None) is not None else None
-
-    def _self_block_fwd(self, w, a, lp, x, key_valid, causal, l, kind, frame=None):
-        g = ops.gemm
-        s = lp + "self_attn."
-        g(x, self.w16(s + "q_proj.weight", s + "v_proj.weight"), a["qkv"], bias=self.w32(s + "q_proj.bias", s + "v_proj.bias"))
-        ops.attn_fwd(self._self_attn_args(w, a["qkv"], a["ctx"], a["lse"], key_valid, causal, frame=frame))
-        g(a["ctx"], self.w16(s + "out_proj.weight"), a["o"], bias=self.w32(s + "out_proj.bias"))
-        ops.add_ln_fwd(x, a["o"], self.w32(lp + "self_attn_layer_norm.weight"), self.w32(lp + "self_attn_layer_norm.bias"),
-                       a["x1"], a["m1"], a["r1"], self.pd, self.seed, self._sid(kind, l), step_dev=self.step_dev)
-
-    def _ffn_block_fwd(self, a, lp, xin, out, mk, rk, l, kind):
-        g = ops.gemm
-        g(xin, self.w16(lp + "fc1.weight"), a["a"], bias=self.w32(lp + "fc1.bias"), act=ops.ACT_GELU, aux=a["h"],
-          aux_mode=ops.AUX_STORE_DACT)   # a["h"]: GELU'(pre-activation) (backward is one multiply)
-        g(a["a"], self.w16(lp + "fc2.weight"), a["f"], bias=self.w32(lp + "fc2.bias"))
-        ops.add_ln_fwd(xin, a["f"], self.w32(lp + "final_layer_norm.weight"), self.w32(lp + "final_layer_norm.bias"),
-                       out, a[mk], a[rk], self.pd, self.seed, self._sid(kind, l), step_dev=self.step_dev)
 
     # ------------------------------------------------------------------ backward
     def _wgrad(self, dy, x, gname, gname2=None, col_slice=None):
@@ -731,7 +679,7 @@ class StepEngine:
         if do is not dres:
             pool.put(do)
         dqkv = w["dqkv"][:a["qkv"].shape[0]]
-        ops.attn_bwd(self._self_attn_args(w, a["qkv"], dctx, a["lse"], key_valid, causal, bwd=dqkv, frame=w["S_enc"] if enc else None))
+        ops.attn_bwd(self._self_attn_args(w, a["qkv"], dctx, a["lse"], key_valid, causal, dqkv=dqkv, frame=w["S_enc"] if enc else None))
         pool.put(dctx)
         self._bias_grad(dqkv, self.g32(s + "q_proj.bias", s + "v_proj.bias"))
         self._wgrad(dqkv, a["x"], s + "q_proj.weight", s + "v_proj.weight")
@@ -804,7 +752,7 @@ class StepEngine:
                 pool.put(dyc)
             dqc = pool.get()
             dkv = w["dkv_all"][:, l * 2 * D:(l + 1) * 2 * D]
-            ops.attn_bwd(self._cross_attn_args(w, a["qc"], a["kv"], dA3, a["lse_c"], bwd=(dqc, dkv)))
+            ops.attn_bwd(self._cross_attn_args(w, a["qc"], a["kv"], dA3, a["lse_c"], dqc, dkv))
             self._bias_grad(dqc, self.g32(c + "q_proj.bias"))
             self._wgrad(dqc, a["x1"], c + "q_proj.weight")
             dx1 = pool.get()

@@ -13,7 +13,7 @@ Design (B200-first, not the reference's):
     per business and head for all beams; self-attention caches that never move, addressed through a slot table that the
     beam re-ranking permutes), and the ~200 launches of a step are replayed from one CUDA graph.  `last_logits`
     recomputes the whole prefix in a 128-position causal frame with the training kernels and is kept as the cross-check
-    of the cached path;
+    of the cached path; both run the layer forwards of `layers.py`, on different attention and embedding kernels;
   * the beam bookkeeping is VECTORISED OVER BUSINESSES AND RUNS ON THE DEVICE (`BeamSearch`): n-gram blocking, the
     top-2k candidate merge, the per-business hypothesis pools and the early-stopping flags are tensor ops without a
     single `.item()` / `.tolist()` in the token loop (the reference loops over batch x beam in Python with host syncs
@@ -27,6 +27,7 @@ Review frames up to 208 tokens are supported (src/test.py uses 158 / 118).
 import torch
 
 from . import inference as INF
+from . import layers as L
 from . import ops
 
 NEG = float("-inf")
@@ -564,54 +565,23 @@ class Generator:
     def _decode_launches(self, st):
         """Every kernel of one decode step; all per-step state (token ids, position, slot table) is read from device memory."""
         eng, cfg, mem, w = self.eng, self.eng.cfg, st.mem, st.cws
-        D, H = cfg.d_model, cfg.heads
         N = w["x"].shape[0]
-        nm = len(mem.mods)
-        g = ops.gemm
-        bm = "bart_model.model."
-        pre = bm + "decoder."
-        scale = cfg.head_dim ** -0.5
+        stats, scale = (w["mean"], w["rstd"]), cfg.head_dim ** -0.5
         x, nxt = w["x"], w["nxt"]
-        ops.embed_ln_decode(w["ids"], eng.w32(bm + "shared.weight"), eng.w32(pre + "embed_positions.weight"), w["rd"],
-                            eng.w32(pre + "rating_embeddings"), eng.w32(pre + "layernorm_embedding.weight"),
-                            eng.w32(pre + "layernorm_embedding.bias"), x, w["mean"], w["rstd"], N, w["pos_dev"])
-        cross = ops.attn_args(Q=w["qc"], ldq=D, q_col=0, KV=mem.kv[0], ldkv=2 * D, k_col=0, v_col=D, O=w["A3"], ldo=D, LSE=None,
-                              key_valid=mem.mem_valid, ent_valid=mem.ent_valid, inv_n=w["inv_n"], n_qseq=N, H=H, R=st.beams,
-                              causal=0, E_total=mem.Et, scale=scale, mods=INF.cross_mods(mem, N, D))
+        ops.embed_ln_decode(w["ids"], *L.embed_params(eng, "decoder", w["rd"]), x, *stats, N, w["pos_dev"])
+        cross = L.cross_attn_args(eng, w["qc"], mem.kv[0], w["A3"], None, mem.mods, mem.mem_valid, mem.ent_valid, w["inv_n"],
+                                  N, st.beams)
+        fork = (w["side"], w["ev_fork"], w["ev_join"])     # the two gate GEMMs are 16-CTA GEMMs: run them side by side
         for l in range(cfg.decoder_layers):
-            lp = pre + "layers.%d." % l
-            s_, c = lp + "self_attn.", lp + "encoder_attn."
-            g(x, eng.w16(s_ + "q_proj.weight", s_ + "v_proj.weight"), w["qkv"], bias=eng.w32(s_ + "q_proj.bias", s_ + "v_proj.bias"))
-            ops.attn_decode_self(w["qkv"], w["kvs"][l], w["hist"], w["pos_dev"], w["ctx"], H, scale)
-            g(w["ctx"], eng.w16(s_ + "out_proj.weight"), w["o"], bias=eng.w32(s_ + "out_proj.bias"))
-            ops.add_ln_fwd(x, w["o"], eng.w32(lp + "self_attn_layer_norm.weight"), eng.w32(lp + "self_attn_layer_norm.bias"), w["x1"],
-                           w["mean"], w["rstd"], 0.0, 0, 0)
-            g(w["x1"], eng.w16(c + "q_proj.weight"), w["qc"], bias=eng.w32(c + "q_proj.bias"))
+            lp = L.BM + "decoder.layers.%d." % l
             cross.KV = mem.kv[l].data_ptr()
-            ops.attn_decode_cross(cross)
-            g(w["A3"].view(nm * N, D), eng.w16(c + "out_proj.weight"), w["O3"].view(nm * N, D), bias=eng.w32(c + "out_proj.bias"))
-            if nm == 3:
-                # the two gate projections are independent 16-CTA GEMMs: they run side by side (a fork / join in the graph)
-                main = torch.cuda.current_stream()
-                w["ev_fork"].record(main)
-                w["side"].wait_event(w["ev_fork"])
-                with torch.cuda.stream(w["side"]):
-                    ops.gemm_cat(w["O3"][0], w["O3"][2], eng.w16(c + "beta_proj.weight"), w["U"][1], bias=eng.w32(c + "beta_proj.bias"))
-                    w["ev_join"].record(w["side"])
-                ops.gemm_cat(w["O3"][0], w["O3"][1], eng.w16(c + "alpha_proj.weight"), w["U"][0], bias=eng.w32(c + "alpha_proj.bias"))
-                main.wait_event(w["ev_join"])
-                ops.gate_fwd(w["O3"], w["U"], mem.pres, w["yc"], w["AB"], N, st.beams, D)
-                yc = w["yc"]
-            else:
-                yc = w["O3"][0]
-            ops.add_ln_fwd(w["x1"], yc, eng.w32(lp + "encoder_attn_layer_norm.weight"), eng.w32(lp + "encoder_attn_layer_norm.bias"),
-                           w["x2"], w["mean"], w["rstd"], 0.0, 0, 0)
-            g(w["x2"], eng.w16(lp + "fc1.weight"), w["a"], bias=eng.w32(lp + "fc1.bias"), act=ops.ACT_GELU)
-            g(w["a"], eng.w16(lp + "fc2.weight"), w["f"], bias=eng.w32(lp + "fc2.bias"))
-            ops.add_ln_fwd(w["x2"], w["f"], eng.w32(lp + "final_layer_norm.weight"), eng.w32(lp + "final_layer_norm.bias"), nxt,
-                           w["mean"], w["rstd"], 0.0, 0, 0)
+            attend = lambda qkv, ctx, l=l: ops.attn_decode_self(qkv, w["kvs"][l], w["hist"], w["pos_dev"], ctx, cfg.heads, scale)
+            L.self_block(eng, lp, x, w, attend, stats, L.NO_DROP)
+            L.cross_block(eng, lp, w["x1"], w, lambda qc, A3: ops.attn_decode_cross(cross), stats, L.NO_DROP, mem.pres,
+                          st.beams, fork)
+            L.ffn_block(eng, lp, w["x2"], w, nxt, stats, L.NO_DROP)
             x, nxt = nxt, x
-        g(x, eng.w16(bm + "shared.weight"), w["logits"], bias=eng.w32_flb())
+        ops.gemm(x, eng.w16(L.BM + "shared.weight"), w["logits"], bias=eng.w32_flb())
 
     @torch.no_grad()
     def step_logits(self, st, input_ids, rating_diff):
@@ -735,12 +705,10 @@ class Generator:
             smem.pres.copy_(mem.pres)
         w["inv_n"].copy_(mem.inv_n.repeat_interleave(k, dim=0))
         for l in range(cfg.decoder_layers):
-            c = "bart_model.model.decoder.layers.%d.encoder_attn." % l
             if mem.kv:
                 smem.kv[l].copy_(mem.kv[l])
             else:
-                ops.gemm(mem.MEM, eng.w16(c + "k_proj.weight", c + "v_proj.weight"), smem.kv[l],
-                         bias=eng.w32(c + "k_proj.bias", c + "v_proj.bias"))
+                L.project_kv(eng, mem.MEM, l, smem.kv[l])
         # ---- reset the per-call state in place
         bs.reset()
         w["rd"].copy_(rd.reshape(-1))

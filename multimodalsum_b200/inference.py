@@ -7,15 +7,16 @@ These are the bodies behind the drop-in surface of SURVEY §8(b):
   build_memory             what BartDecoder.forward does with its memory lists (mask inversion :572-575, null entities
                            :856-866, modality presence :732-736) — integer bookkeeping, torch on the device
   decoder_hidden, lm_head  BartDecoder.forward :530-660 + LM head :2281 over full 128-position frames
-Training does NOT go through here: `MultimodalSum.forward` runs the fused step (engine.StepEngine).  Everything is
-computed by the same C-ABI kernels (bf16 activations, fp32 statistics); torch only allocates and does the integer
-mask bookkeeping.  All functions expect CUDA tensors and raise otherwise (no CPU path).
+Training does NOT go through here: `MultimodalSum.forward` runs the fused step (engine.StepEngine); both run the layer
+forwards of `layers.py`, on the same C-ABI kernels (bf16 activations, fp32 statistics).  Torch only allocates and does
+the integer mask bookkeeping.  All functions expect CUDA tensors and raise otherwise (no CPU path).
 """
 import math
 from dataclasses import dataclass, field as dc_field
 
 import torch
 
+from . import layers as L
 from . import ops
 
 FRAME = 128          # query tile of the attention kernels
@@ -35,10 +36,6 @@ def _need_cuda(t, what):
         raise RuntimeError("%s must be a CUDA tensor: mmsum_b200 has no CPU path" % what)
 
 
-def table_dims(dataset):
-    return 47 if dataset == "yelp" else 133
-
-
 # ---------------------------------------------------------------------------------------------- modality encoders
 @torch.no_grad()
 def table_forward(eng, field, field_value, out=None):
@@ -49,22 +46,14 @@ def table_forward(eng, field, field_value, out=None):
     _need_cuda(field, "field")
     dev = field.device
     D = cfg.d_model
-    F = table_dims(cfg.table)
+    F = L.table_dims(cfg.table)
     vals = [v.to(torch.int64).contiguous() for v in field_value]
     B = vals[0].shape[0]
-    t = "table_encoder."
-    W1n = t + ("hours_embedding.weight" if cfg.table == "yelp" else "price_embedding.weight")
-    if cfg.table == "yelp":
-        W0, W1 = eng.w32(t + "rating_embedding.weight"), eng.w32(W1n)
-    else:
-        W0, W1 = eng.w32(W1n), eng.w32(t + "rating_embedding.weight")
     tabX, valid, tab_h = _bf(dev, B * F, 2 * D), torch.zeros(B, F, device=dev, dtype=torch.uint8), _bf(dev, B * F, D)
-    ops.table_fwd(cfg.table, B, eng.w32("bart_model.model.shared.weight"), field.to(torch.int64).contiguous(), vals, W0, W1,
-                  tabX, valid)
-    ops.gemm(tabX, eng.w16(t + "fc.weight"), tab_h, bias=eng.w32(t + "fc.bias"), act=ops.ACT_RELU)
+    L.table_embed(eng, field.to(torch.int64).contiguous(), vals, tabX, valid)
     if out is None:
         out = _bf(dev, B * F, D)
-    ops.gemm(tab_h, eng.w16(t + "linear.weight"), out)
+    L.table_project(eng, tabX, tab_h, out)
     return out.view(B, F, D), valid
 
 
@@ -106,30 +95,19 @@ def encoder_forward(eng, input_ids, attention_mask=None):
     valid = torch.zeros(N, Sp, device=dev, dtype=torch.uint8)
     valid[:, :S] = (attention_mask != 0).to(torch.uint8)
     kvalid = valid.reshape(-1)
-    g = ops.gemm
-    bm = "bart_model.model."
-    pre = bm + "encoder."
-    x, x1, nxt = _bf(dev, T, D), _bf(dev, T, D), _bf(dev, T, D)
-    qkv, ctx, o, a_buf, f_buf = _bf(dev, T, 3 * D), _bf(dev, T, D), _bf(dev, T, D), _bf(dev, T, cfg.ffn_dim), _bf(dev, T, D)
-    mean, rstd = _f32(dev, T), _f32(dev, T)
+    x, nxt = _bf(dev, T, D), _bf(dev, T, D)
+    buf = dict(qkv=_bf(dev, T, 3 * D), ctx=_bf(dev, T, D), o=_bf(dev, T, D), x1=_bf(dev, T, D), a=_bf(dev, T, cfg.ffn_dim),
+               f=_bf(dev, T, D))
+    stats = (_f32(dev, T), _f32(dev, T))
     lse = _f32(dev, N * tiles, H, 1, FRAME)
-    ops.embed_ln_fwd(ids.reshape(-1), eng.w32(bm + "shared.weight"), eng.w32(pre + "embed_positions.weight"), None, None,
-                     eng.w32(pre + "layernorm_embedding.weight"), eng.w32(pre + "layernorm_embedding.bias"), x, mean, rstd,
-                     T, Sp, 0.0, 0, 0)
-    Sk = min(Sp, MAX_KEYS)
+    ops.embed_ln_fwd(ids.reshape(-1), *L.embed_params(eng, "encoder", None), x, *stats, T, Sp, *L.NO_DROP)
+    # a frame of Sp rows = Sp/128 query tiles attending to one key entity of <= 208 rows
+    attend = lambda qkv, ctx: ops.attn_fwd(L.self_attn_args(eng, qkv, ctx, lse, kvalid, N * tiles, False, min(Sp, MAX_KEYS),
+                                                            R=tiles, ent_stride=Sp))
     for l in range(cfg.encoder_layers):
-        lp = pre + "layers.%d." % l
-        s_ = lp + "self_attn."
-        g(x, eng.w16(s_ + "q_proj.weight", s_ + "v_proj.weight"), qkv, bias=eng.w32(s_ + "q_proj.bias", s_ + "v_proj.bias"))
-        # a frame of Sp rows = Sp/128 query tiles attending to one key entity of <= 208 rows
-        ops.attn_fwd(ops.attn_args(Q=qkv, ldq=3 * D, q_col=0, KV=qkv, ldkv=3 * D, k_col=D, v_col=2 * D, O=ctx, ldo=D, LSE=lse,
-                                   key_valid=kvalid, ent_valid=None, inv_n=None, n_qseq=N * tiles, H=H, R=tiles, causal=0,
-                                   E_total=1, scale=cfg.head_dim ** -0.5, mods=[(0, 0, 1, Sk, 0, 0, Sp)]))
-        g(ctx, eng.w16(s_ + "out_proj.weight"), o, bias=eng.w32(s_ + "out_proj.bias"))
-        ops.add_ln_fwd(x, o, eng.w32(lp + "self_attn_layer_norm.weight"), eng.w32(lp + "self_attn_layer_norm.bias"), x1, mean, rstd, 0.0, 0, 0)
-        g(x1, eng.w16(lp + "fc1.weight"), a_buf, bias=eng.w32(lp + "fc1.bias"), act=ops.ACT_GELU)
-        g(a_buf, eng.w16(lp + "fc2.weight"), f_buf, bias=eng.w32(lp + "fc2.bias"))
-        ops.add_ln_fwd(x1, f_buf, eng.w32(lp + "final_layer_norm.weight"), eng.w32(lp + "final_layer_norm.bias"), nxt, mean, rstd, 0.0, 0, 0)
+        lp = L.BM + "encoder.layers.%d." % l
+        L.self_block(eng, lp, x, buf, attend, stats, L.NO_DROP)
+        L.ffn_block(eng, lp, buf["x1"], buf, nxt, stats, L.NO_DROP)
         x, nxt = nxt, x
     return x.view(N, Sp, D)[:, :S]
 
@@ -198,25 +176,12 @@ def build_memory(eng, hiddens, masks):
 
 @torch.no_grad()
 def project_memory(eng, mem):
-    """Cross-attention K|V of the whole memory, one GEMM per decoder layer (k_proj | v_proj are adjacent in the arena)."""
+    """Cross-attention K|V of the whole memory, one GEMM per decoder layer."""
     if mem.kv:
         return mem
-    dev = mem.MEM.device
-    D = eng.cfg.d_model
     for l in range(eng.cfg.decoder_layers):
-        c = "bart_model.model.decoder.layers.%d.encoder_attn." % l
-        mem.kv.append(ops.gemm(mem.MEM, eng.w16(c + "k_proj.weight", c + "v_proj.weight"), _bf(dev, mem.MEM.shape[0], 2 * D),
-                               bias=eng.w32(c + "k_proj.bias", c + "v_proj.bias")))
+        mem.kv.append(L.project_kv(eng, mem.MEM, l, _bf(mem.MEM.device, mem.MEM.shape[0], 2 * eng.cfg.d_model)))
     return mem
-
-
-def cross_mods(mem, q_rows, D):
-    """MmsumAttnMod tuples of a memory for a query buffer of `q_rows` rows per modality output."""
-    out, eb = [], 0
-    for i, (base, E, S) in enumerate(mem.mods):
-        out.append((base, i * q_rows * D, E, S, 0, eb, 0))
-        eb += E
-    return out
 
 
 # ---------------------------------------------------------------------------------------------- decoder (full frames)
@@ -248,47 +213,23 @@ def decoder_hidden(eng, mem, dec_ids, rating_diff=None, per_biz=1, dec_valid=Non
         kv_[:, :cur] = (dec_valid != 0).to(torch.uint8)
         kvalid = kv_.reshape(-1)
     rd = torch.zeros(N, device=dev) if rating_diff is None else rating_diff.reshape(N).float().contiguous()
-    g = ops.gemm
-    bm = "bart_model.model."
-    pre = bm + "decoder."
-    x, x1, x2, nxt = _bf(dev, T, D), _bf(dev, T, D), _bf(dev, T, D), _bf(dev, T, D)
-    qkv, ctx, o, qc = _bf(dev, T, 3 * D), _bf(dev, T, D), _bf(dev, T, D), _bf(dev, T, D)
-    A3, O3 = _bf(dev, nm, T, D), _bf(dev, nm, T, D)
-    a_buf, f_buf = _bf(dev, T, FF), _bf(dev, T, D)
-    mean, rstd = _f32(dev, T), _f32(dev, T)
-    lse, lse_c = _f32(dev, N, H, 1, S), _f32(dev, N, H, mem.Et, S)
+    x, nxt = _bf(dev, T, D), _bf(dev, T, D)
+    buf = dict(qkv=_bf(dev, T, 3 * D), ctx=_bf(dev, T, D), o=_bf(dev, T, D), x1=_bf(dev, T, D), qc=_bf(dev, T, D),
+               A3=_bf(dev, nm, T, D), O3=_bf(dev, nm, T, D), x2=_bf(dev, T, D), a=_bf(dev, T, FF), f=_bf(dev, T, D))
     if nm == 3:
-        U, AB, yc = _bf(dev, 2, T, D), _bf(dev, 2, T, D), _bf(dev, T, D)
+        buf.update(U=_bf(dev, 2, T, D), AB=_bf(dev, 2, T, D), yc=_bf(dev, T, D))
+    stats = (_f32(dev, T), _f32(dev, T))
+    lse, lse_c = _f32(dev, N, H, 1, S), _f32(dev, N, H, mem.Et, S)
     inv_n = mem.inv_n.repeat_interleave(per_biz, dim=0).contiguous() if per_biz > 1 else mem.inv_n
-    mods = cross_mods(mem, T, D)
-    ops.embed_ln_fwd(ids.reshape(-1), eng.w32(bm + "shared.weight"), eng.w32(pre + "embed_positions.weight"), rd,
-                     eng.w32(pre + "rating_embeddings"), eng.w32(pre + "layernorm_embedding.weight"),
-                     eng.w32(pre + "layernorm_embedding.bias"), x, mean, rstd, T, S, 0.0, 0, 0)
+    ops.embed_ln_fwd(ids.reshape(-1), *L.embed_params(eng, "decoder", rd), x, *stats, T, S, *L.NO_DROP)
+    attend_self = lambda qkv, ctx: ops.attn_fwd(L.self_attn_args(eng, qkv, ctx, lse, kvalid, N, True, S))
     for l in range(cfg.decoder_layers):
-        lp = pre + "layers.%d." % l
-        s_, c = lp + "self_attn.", lp + "encoder_attn."
-        g(x, eng.w16(s_ + "q_proj.weight", s_ + "v_proj.weight"), qkv, bias=eng.w32(s_ + "q_proj.bias", s_ + "v_proj.bias"))
-        ops.attn_fwd(ops.attn_args(Q=qkv, ldq=3 * D, q_col=0, KV=qkv, ldkv=3 * D, k_col=D, v_col=2 * D, O=ctx, ldo=D, LSE=lse,
-                                   key_valid=kvalid, ent_valid=None, inv_n=None, n_qseq=N, H=H, R=1, causal=1, E_total=1,
-                                   scale=cfg.head_dim ** -0.5, mods=[(0, 0, 1, S, 0, 0)]))
-        g(ctx, eng.w16(s_ + "out_proj.weight"), o, bias=eng.w32(s_ + "out_proj.bias"))
-        ops.add_ln_fwd(x, o, eng.w32(lp + "self_attn_layer_norm.weight"), eng.w32(lp + "self_attn_layer_norm.bias"), x1, mean, rstd, 0.0, 0, 0)
-        g(x1, eng.w16(c + "q_proj.weight"), qc, bias=eng.w32(c + "q_proj.bias"))
-        ops.attn_fwd(ops.attn_args(Q=qc, ldq=D, q_col=0, KV=mem.kv[l], ldkv=2 * D, k_col=0, v_col=D, O=A3, ldo=D, LSE=lse_c,
-                                   key_valid=mem.mem_valid, ent_valid=mem.ent_valid, inv_n=inv_n, n_qseq=N, H=H, R=per_biz, causal=0,
-                                   E_total=mem.Et, scale=cfg.head_dim ** -0.5, mods=mods))
-        g(A3.view(nm * T, D), eng.w16(c + "out_proj.weight"), O3.view(nm * T, D), bias=eng.w32(c + "out_proj.bias"))
-        if nm == 3:
-            ops.gemm_cat(O3[0], O3[1], eng.w16(c + "alpha_proj.weight"), U[0], bias=eng.w32(c + "alpha_proj.bias"))
-            ops.gemm_cat(O3[0], O3[2], eng.w16(c + "beta_proj.weight"), U[1], bias=eng.w32(c + "beta_proj.bias"))
-            ops.gate_fwd(O3, U, mem.pres, yc, AB, T, per_biz * S, D)
-            y = yc
-        else:
-            y = O3[0]
-        ops.add_ln_fwd(x1, y, eng.w32(lp + "encoder_attn_layer_norm.weight"), eng.w32(lp + "encoder_attn_layer_norm.bias"), x2, mean, rstd, 0.0, 0, 0)
-        g(x2, eng.w16(lp + "fc1.weight"), a_buf, bias=eng.w32(lp + "fc1.bias"), act=ops.ACT_GELU)
-        g(a_buf, eng.w16(lp + "fc2.weight"), f_buf, bias=eng.w32(lp + "fc2.bias"))
-        ops.add_ln_fwd(x2, f_buf, eng.w32(lp + "final_layer_norm.weight"), eng.w32(lp + "final_layer_norm.bias"), nxt, mean, rstd, 0.0, 0, 0)
+        lp = L.BM + "decoder.layers.%d." % l
+        attend_mem = lambda qc, A3: ops.attn_fwd(L.cross_attn_args(eng, qc, mem.kv[l], A3, lse_c, mem.mods, mem.mem_valid,
+                                                                   mem.ent_valid, inv_n, N, per_biz))
+        L.self_block(eng, lp, x, buf, attend_self, stats, L.NO_DROP)
+        L.cross_block(eng, lp, buf["x1"], buf, attend_mem, stats, L.NO_DROP, mem.pres, per_biz * S)
+        L.ffn_block(eng, lp, buf["x2"], buf, nxt, stats, L.NO_DROP)
         x, nxt = nxt, x
     return x.view(N, S, D)
 
