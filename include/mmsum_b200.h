@@ -228,6 +228,38 @@ int mmsum_table_fwd(const MmsumTableArgs* args, void* stream);
 int mmsum_table_bits_bwd(const void* dX, const int64_t* bits, float* dW, int32_t B, int32_t F, int32_t f0, int32_t nrows,
                          int32_t nb, void* stream);
 
+/* ---- ordered (bitwise-reproducible) variants of the backward's fp32 reductions -----------------------------------------
+ * Same arguments and results as the calls above up to fp32 rounding, but every sum lands in an order fixed by the shape (and,
+ * for the GEMM, the SM count), so equal inputs give equal bits on every run, whatever the scheduling.  The calls above finish
+ * these sums with fp32 atomics or TMA reduce-adds from several CTAs; here each CTA writes its partial sums to the caller's
+ * `workspace` (fp32, never allocated by the library) and a second pass adds them in index order with one read-modify-write per
+ * output element.  A workspace smaller than stated is rejected on the host before any launch.
+ *
+ * mmsum_gemm_bf16_ordered: the same tiling and split-K choice as mmsum_gemm_bf16; with more than one split every split stores its
+ *   partial tile to its own region of `workspace` and the splits are then added to D in split order.  One split (and every
+ *   non-accumulating call) is mmsum_gemm_bf16 itself: one writer per element.  mmsum_gemm_ordered_workspace writes the fp32
+ *   element count the call needs for `args` (0: none) to *elems; it reads no pointer of `args` and launches nothing. */
+int mmsum_gemm_bf16_ordered(const MmsumGemmArgs* args, float* workspace, int64_t workspace_elems, void* stream);
+int mmsum_gemm_ordered_workspace(const MmsumGemmArgs* args, int64_t* elems);
+/* mmsum_add_ln_bwd: workspace >= 444 * 2048 floats (per-CTA dgamma | dbeta rows). */
+int mmsum_add_ln_bwd_ordered(const void* d1, const void* d2, const void* res, const void* y, const float* gamma, const float* mean,
+                             const float* rstd, void* dres, void* dy, float* dgamma, float* dbeta, int32_t rows, int32_t d_model,
+                             float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, float* workspace,
+                             int64_t workspace_elems, void* stream);
+/* mmsum_colsum: workspace >= max(151552, N) floats (per-row-chunk column sums). */
+int mmsum_colsum_ordered(const void* x, int64_t ld, int32_t rows, int32_t N, float* out, float* workspace, int64_t workspace_elems,
+                         void* stream);
+/* mmsum_embed_ln_bwd: V = rows of E (< 2^22).  The dE scatter becomes a stable counting sort of the rows by token id followed by
+ * a fixed-order sum per id (its rows in row order within tiles of 64 sorted rows, then the tile sums in tile order) added once
+ * (pad id skipped as before); dremb, dgamma and dbeta are summed in a fixed order; dP already has one writer per element.
+ * workspace >= 592 * 2048 + S * 1024 + 2048 * ceil(rows / 64) + V + 1 + 2 * rows elements (4 bytes each). */
+int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
+                               const float* rating_diff, const float* remb, const float* gamma, const float* mean, const float* rstd,
+                               float* dE, float* dP, float* dremb, float* dgamma, float* dbeta, float* dz_scratch, int32_t rows,
+                               int32_t S, int32_t d_model, int32_t pad_id, float p_drop, uint64_t seed, uint32_t stream_id,
+                               const uint32_t* step_dev, int32_t V, float* workspace, int64_t workspace_elems, void* stream);
+/* mmsum_table_bits_bwd needs no variant: each dW element is summed by one thread in a fixed order and added once. */
+
 /* ---- optimizer over the flat arenas ---------------------------------------------------------------
  * mmsum_grad_sumsq: out[0] = sum g^2 (two deterministic stages; partial needs >= 1184 floats) — the global norm of
  * torch.nn.utils.clip_grad_norm_ (src/multimodal_train.py:361-362).

@@ -92,6 +92,8 @@ EXPORTS = [
     "mmsum_table_fwd", "mmsum_table_bits_bwd", "mmsum_grad_sumsq", "mmsum_adamw_step",
     "mmsum_embed_ln_decode", "mmsum_attn_decode_cross", "mmsum_attn_decode_self", "mmsum_beam_topk", "mmsum_beam_update",
     "mmsum_sample_token",
+    "mmsum_gemm_bf16_ordered", "mmsum_gemm_ordered_workspace", "mmsum_add_ln_bwd_ordered", "mmsum_colsum_ordered",
+    "mmsum_embed_ln_bwd_ordered",
 ]
 
 

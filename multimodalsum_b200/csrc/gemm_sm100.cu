@@ -66,6 +66,7 @@ struct GemmKernelArgs {
   int out_f32;
   int accumulate;
   int k_split;    // > 0: A columns [k_split, K) come from the second A tensor map (concat along K)
+  int ws_rows;    // EPI 3: rows of one split's region of the partial workspace (split sp stores at row sp * ws_rows + m)
 };
 
 // work unit t -> (m unit, n tile, k split); an m unit is one m-tile (CL = 1) or a pair of adjacent m-tiles (CL = 2)
@@ -77,7 +78,8 @@ __device__ __forceinline__ void decode_tile(const GemmKernelArgs& g, int m_units
   else                 { nt = r % g.n_tiles; mu = r / g.n_tiles; }
 }
 
-// EPI: 0 plain epilogue (alpha, bias, ReLU), 1 = GELU/ReLU with the pre-activation saved to aux, 2 = multiply by act'(aux)
+// EPI: 0 plain epilogue (alpha, bias, ReLU), 1 = GELU/ReLU with the pre-activation saved to aux, 2 = multiply by act'(aux),
+//      3 = fp32 split-K partials stored (not reduce-added) to each split's own region of a workspace (ordered split-K)
 template <int BN, bool A_MN, bool B_MN, int EPI, int CL>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmA2,
@@ -315,8 +317,9 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             __syncwarp();
             if (lane == 0) {
               if (ncol0 < g.N && m0 + q * 32 < g.M) {
-                if (g.accumulate) tma_reduce_add_2d(&tmD, stg, ncol0, m0 + q * 32);
-                else              tma_store_2d(&tmD, stg, ncol0, m0 + q * 32);
+                if (EPI == 3)          tma_store_2d(&tmD, stg, ncol0, sp * g.ws_rows + m0 + q * 32);
+                else if (g.accumulate) tma_reduce_add_2d(&tmD, stg, ncol0, m0 + q * 32);
+                else                   tma_store_2d(&tmD, stg, ncol0, m0 + q * 32);
               }
               tma_store_commit();
             }
@@ -383,6 +386,20 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     __syncwarp();
     tc_fence_after();
     if (CL == 2) tmem_dealloc2(tmem_base, 512); else tmem_dealloc(tmem_base, 512);
+  }
+}
+
+// Ordered split-K: D[m, n] = (((D[m, n] + P_0[m, n]) + P_1[m, n]) + ...) over the splits in index order, one read-modify-write
+// per element.  P_s = ws + s * split_stride, row pitch ldw.
+__global__ void __launch_bounds__(256) splitk_ordered_reduce_kernel(const float* __restrict__ ws, int splits, long long split_stride,
+                                                                    int ldw, float* __restrict__ D, long long ldd, int M, int N) {
+  const long long n_el = (long long)M * N;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n_el; i += (long long)gridDim.x * 256) {
+    const int m = (int)(i / N), n = (int)(i - (long long)m * N);
+    const float* p = ws + (long long)m * ldw + n;
+    float acc = D[(long long)m * ldd + n];
+    for (int s = 0; s < splits; ++s) acc += p[s * split_stride];
+    D[(long long)m * ldd + n] = acc;
   }
 }
 
@@ -471,9 +488,15 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& ta2, const CUte
 
 using namespace mmsum;
 
-extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_v);
-  if (!a || !a->A || !a->B || !a->D) return MMSUM_ERR_INVALID;
+static int launch_gemm_case(int bn, int am, int bm, int epi, int cl, const CUtensorMap& ta, const CUtensorMap& ta2,
+                            const CUtensorMap& tb, const CUtensorMap& td, const CUtensorMap& taux, const GemmKernelArgs& ka,
+                            int grid, cudaStream_t stream);
+
+// ordered = false: mmsum_gemm_bf16.  ordered = true: mmsum_gemm_bf16_ordered (ws / ws_elems) or, with need != NULL, only the
+// workspace size query (nothing is launched and no pointer is read).
+static int gemm_impl(const MmsumGemmArgs* a, cudaStream_t stream, bool ordered, float* ws, int64_t ws_elems, int64_t* need) {
+  if (need != nullptr) *need = 0;
+  if (!a || (need == nullptr && (!a->A || !a->B || !a->D))) return MMSUM_ERR_INVALID;
   if (a->M <= 0 || a->N <= 0 || a->K <= 0) return MMSUM_ERR_INVALID;
   if (!a->out_f32 && a->accumulate) return MMSUM_ERR_INVALID;
   if (a->aux_mode != 0 && (!a->aux || (a->N % 8) != 0 || (a->ld_aux % 8) != 0)) return MMSUM_ERR_INVALID;
@@ -533,6 +556,19 @@ extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
   ka.ld_aux = a->ld_aux;
   ka.out_f32 = a->out_f32;
   ka.accumulate = a->accumulate;
+  ka.ws_rows = 0;
+  // ordered split-K: every split stores its partial tile to its own [m_tiles * 128, ldw] region of `ws`, then one pass adds the
+  // regions to D in split order (splits == 1 keeps the single TMA reduce-add per element, which is already one writer)
+  const bool ws_mode = ordered && ka.splits > 1;
+  const int ldw = (a->N + 3) / 4 * 4;                         // 16-byte row pitch for the tensor map
+  const long long split_stride = (long long)ka.m_tiles * BM * ldw;
+  if (ws_mode) {
+    if (ka.act != 0 || ka.aux_mode != 0) return MMSUM_ERR_INVALID;
+    if (need != nullptr) { *need = split_stride * ka.splits; return 0; }
+    if (!ws || (reinterpret_cast<uintptr_t>(ws) & 15) || ws_elems < split_stride * ka.splits) return MMSUM_ERR_INVALID;
+    ka.ws_rows = ka.m_tiles * BM;
+  }
+  if (need != nullptr) return 0;
 
   CUtensorMap ta, ta2, tb, td;
   int rc;
@@ -560,7 +596,8 @@ extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
   if (a->b_mn_major) rc = make_tmap(&tb, a->B, 0, (uint64_t)a->N, (uint64_t)a->K, (uint64_t)a->ldb * 2, 64, 64);
   else               rc = make_tmap(&tb, a->B, 0, (uint64_t)a->K, (uint64_t)a->N, (uint64_t)a->ldb * 2, 64, (uint32_t)(bn / cl));
   if (rc) return rc;
-  if (a->out_f32) rc = make_tmap(&td, a->D, 1, (uint64_t)a->N, (uint64_t)a->M, (uint64_t)a->ldd * 4, 32, 32);
+  if (ws_mode)    rc = make_tmap(&td, ws, 1, (uint64_t)a->N, (uint64_t)(ka.ws_rows * ka.splits), (uint64_t)ldw * 4, 32, 32);
+  else if (a->out_f32) rc = make_tmap(&td, a->D, 1, (uint64_t)a->N, (uint64_t)a->M, (uint64_t)a->ldd * 4, 32, 32);
   else            rc = make_tmap(&td, a->D, 0, (uint64_t)a->N, (uint64_t)a->M, (uint64_t)a->ldd * 2, 64, 32);
   if (rc) return rc;
   CUtensorMap taux = td;   // pre-activation copy (aux_mode 1) leaves through its own map, same tiling as D
@@ -575,7 +612,24 @@ extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
   int grid = total < nsm ? total : nsm;
   if (cl == 2) grid = (int)(pairs * 2 < nsm ? pairs * 2 : nsm);
   const int am = a->a_mn_major ? 1 : 0, bm = a->b_mn_major ? 1 : 0;
-  const int epi = (a->aux_mode == 3) ? 1 : (a->aux_mode == 4 ? 2 : a->aux_mode);   // 3 / 4 share the kernels of 1 / 2
+  // aux modes 3 / 4 share the kernels of 1 / 2; EPI 3 = ordered split-K partials
+  const int epi = ws_mode ? 3 : ((a->aux_mode == 3) ? 1 : (a->aux_mode == 4 ? 2 : a->aux_mode));
+  if (ws_mode) {
+    if (int rc2 = launch_gemm_case(bn, am, bm, epi, cl, ta, ta2, tb, td, taux, ka, grid, stream)) return rc2;
+    const long long n_el = (long long)a->M * a->N;
+    const long long rblocks = (n_el + 255) / 256;
+    const int rgrid = (int)(rblocks < (long long)nsm * 8 ? rblocks : (long long)nsm * 8);
+    splitk_ordered_reduce_kernel<<<rgrid, 256, 0, stream>>>(ws, ka.splits, split_stride, ldw, reinterpret_cast<float*>(a->D),
+                                                             a->ldd, a->M, a->N);
+    MMSUM_CHECK_LAUNCH();
+    return 0;
+  }
+  return launch_gemm_case(bn, am, bm, epi, cl, ta, ta2, tb, td, taux, ka, grid, stream);
+}
+
+static int launch_gemm_case(int bn, int am, int bm, int epi, int cl, const CUtensorMap& ta, const CUtensorMap& ta2,
+                            const CUtensorMap& tb, const CUtensorMap& td, const CUtensorMap& taux, const GemmKernelArgs& ka,
+                            int grid, cudaStream_t stream) {
 #define MMSUM_GEMM_CASE(BN_, AM_, BM_, EPI_, CL_) \
   if (bn == BN_ && am == AM_ && bm == BM_ && epi == EPI_ && cl == CL_) \
     return launch_gemm<BN_, (AM_ != 0), (BM_ != 0), EPI_, CL_>(ta, ta2, tb, td, taux, ka, grid, stream);
@@ -600,6 +654,32 @@ extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream_v) {
   MMSUM_GEMM_CASE(256, 0, 1, 1, 1)
   MMSUM_GEMM_CASE(256, 0, 0, 2, 1)
   MMSUM_GEMM_CASE(256, 0, 1, 2, 1)
+  // ordered split-K partials (fp32 output, plain epilogue)
+  MMSUM_GEMM_CASE(256, 0, 0, 3, 2)
+  MMSUM_GEMM_CASE(256, 0, 1, 3, 2)
+  MMSUM_GEMM_CASE(256, 1, 1, 3, 2)
+  MMSUM_GEMM_CASE(256, 1, 0, 3, 2)
+  MMSUM_GEMM_CASE(256, 0, 0, 3, 1)
+  MMSUM_GEMM_CASE(256, 0, 1, 3, 1)
+  MMSUM_GEMM_CASE(256, 1, 1, 3, 1)
+  MMSUM_GEMM_CASE(256, 1, 0, 3, 1)
+  MMSUM_GEMM_CASE(128, 0, 0, 3, 1)
+  MMSUM_GEMM_CASE(128, 0, 1, 3, 1)
+  MMSUM_GEMM_CASE(128, 1, 1, 3, 1)
+  MMSUM_GEMM_CASE(128, 1, 0, 3, 1)
 #undef MMSUM_GEMM_CASE
   return MMSUM_ERR_INVALID;
+}
+
+extern "C" int mmsum_gemm_bf16(const MmsumGemmArgs* a, void* stream) {
+  return gemm_impl(a, reinterpret_cast<cudaStream_t>(stream), false, nullptr, 0, nullptr);
+}
+
+extern "C" int mmsum_gemm_bf16_ordered(const MmsumGemmArgs* a, float* workspace, int64_t workspace_elems, void* stream) {
+  return gemm_impl(a, reinterpret_cast<cudaStream_t>(stream), true, workspace, workspace_elems, nullptr);
+}
+
+extern "C" int mmsum_gemm_ordered_workspace(const MmsumGemmArgs* a, int64_t* elems) {
+  if (!elems) return MMSUM_ERR_INVALID;
+  return gemm_impl(a, nullptr, true, nullptr, 0, elems);
 }

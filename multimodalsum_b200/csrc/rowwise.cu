@@ -131,6 +131,9 @@ __global__ void __launch_bounds__(256) embed_ln_fwd_kernel(const int* __restrict
 
 // backward of the above: dz (fp32, [rows, D]) for the position / rating reductions, scatter-add into dE (pad id
 // skipped: nn.Embedding(padding_idx=1)), dgamma/dbeta.
+// kOrdered: no dE scatter (embed_group_kernel + embed_scatter_tile/span_kernel add the dz rows per token id instead) and the
+// block's dgamma / dbeta sums go to its own row of `partial` [gridDim.x][2 * D] (ordered_colsum_kernel adds them up).
+template <bool kOrdered>
 __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restrict__ dout, const bf16* __restrict__ dout2,
                                                            const int* __restrict__ ids,
                                                            const float* __restrict__ E, const float* __restrict__ P,
@@ -138,7 +141,8 @@ __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restric
                                                            const float* __restrict__ gamma, const float* __restrict__ mean_i,
                                                            const float* __restrict__ rstd_i, float* __restrict__ dE,
                                                            float* __restrict__ dz_out, float* __restrict__ dgamma,
-                                                           float* __restrict__ dbeta, int rows, int S, int pad_id, DropCfg dc_in) {
+                                                           float* __restrict__ dbeta, int rows, int S, int pad_id, DropCfg dc_in,
+                                                           float* __restrict__ partial) {
   const DropCfg dc = resolve_drop(dc_in);
   __shared__ float sg[8][D / 4];  // staged reduction of dgamma / dbeta across the block's warps (two passes of D/4... see below)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
@@ -189,7 +193,7 @@ __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restric
       const int c = col_of(lane, i);
       const float dz = rstd * (dy[i] - s1 - z[i] * s2);
       dzr[c] = dz;
-      if (id != pad_id) atomicAdd(der + c, dz);
+      if (!kOrdered && id != pad_id) atomicAdd(der + c, dz);
     }
   }
   // block reduce dgamma/dbeta then one atomic per column per block
@@ -204,15 +208,20 @@ __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restric
       for (int c = threadIdx.x; c < 256; c += blockDim.x) {
         float s = 0.f;
         for (int w = 0; w < nw; ++w) s += sg[w][c];
-        atomicAdd(dst + quarter * 256 + c, s);
+        if (kOrdered) partial[(long long)blockIdx.x * 2 * D + pass * D + quarter * 256 + c] = s;
+        else          atomicAdd(dst + quarter * 256 + c, s);
       }
     }
   }
 }
 
 // dP[t+2] += sum_seq dz[seq*S+t],  dremb += sum_rows rating_diff[seq] * dz[row]
+// (every dP element has exactly one writer, so its single atomic is already order-free; the S blocks of a column all add into
+//  dremb, so kOrdered stores the position's dremb sum to partial[t][c] instead, summed over t by ordered_colsum_kernel)
+template <bool kOrdered>
 __global__ void __launch_bounds__(256) embed_pos_bwd_kernel(const float* __restrict__ dz, const float* __restrict__ rating_diff,
-                                                            float* __restrict__ dP, float* __restrict__ dremb, int n_seq, int S) {
+                                                            float* __restrict__ dP, float* __restrict__ dremb, int n_seq, int S,
+                                                            float* __restrict__ partial) {
   // grid: (D/256, S); thread = one column, loops over sequences
   const int c = blockIdx.x * 256 + threadIdx.x;
   const int t = blockIdx.y;
@@ -223,7 +232,161 @@ __global__ void __launch_bounds__(256) embed_pos_bwd_kernel(const float* __restr
     if (rating_diff != nullptr) r += rating_diff[q] * v;
   }
   atomicAdd(dP + (long long)(t + 2) * D + c, s);
-  if (rating_diff != nullptr) atomicAdd(dremb + c, r);
+  if (rating_diff != nullptr) {
+    if (kOrdered) partial[(long long)t * D + c] = r;
+    else          atomicAdd(dremb + c, r);
+  }
+}
+
+// ---- ordered (bitwise-reproducible) reductions
+// out0[c] += sum_p part[p * width + c] for c < split, out1[c - split] += ... otherwise; the parts are summed in a fixed tree:
+// row group g of the block sums parts g, g + 8, g + 16, ... in order, then the 8 group sums are added in order g = 0..7.
+__global__ void __launch_bounds__(256) ordered_colsum_kernel(const float* __restrict__ part, int nparts, int width, int split,
+                                                             float* __restrict__ out0, float* __restrict__ out1) {
+  __shared__ float sm[8][32];
+  const int cl = threadIdx.x & 31, grp = threadIdx.x >> 5;
+  const int c = blockIdx.x * 32 + cl;
+  float s = 0.f;
+  if (c < width)
+    for (int p = grp; p < nparts; p += 8) s += part[(long long)p * width + c];
+  sm[grp][cl] = s;
+  __syncthreads();
+  if (grp == 0 && c < width) {
+    float t = 0.f;
+#pragma unroll
+    for (int g = 0; g < 8; ++g) t += sm[g][cl];
+    if (c < split) out0[c] += t;
+    else           out1[c - split] += t;
+  }
+}
+
+// inclusive block scan over 1024 threads (op: sum or max), scratch `ws` >= 32 ints
+template <bool kMax>
+__device__ __forceinline__ int block_scan_1024(int v, int* ws) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int u = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v = kMax ? max(v, u) : v + u;
+  }
+  if (lane == 31) ws[warp] = v;
+  __syncthreads();
+  if (warp == 0) {
+    int w = ws[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int u = __shfl_up_sync(0xffffffffu, w, o);
+      if (lane >= o) w = kMax ? max(w, u) : w + u;
+    }
+    ws[lane] = w;
+  }
+  __syncthreads();
+  if (warp > 0) { const int u = ws[warp - 1]; v = kMax ? max(v, u) : v + u; }
+  __syncthreads();
+  return v;
+}
+
+// Stable grouping of the rows by token id (one block of 1024 threads): a counting sort.  cursor [V + 1] ints: histogram, then
+// exclusive offsets, and on return the END of each id's group; cursor[V] = number of non-pad rows.  order [rows]: the non-pad
+// row indices sorted by (id, row); sid [rows]: the id at each sorted position.  The rows are placed 1024 at a time in row order;
+// inside a tile, a bitonic sort of (id << 10 | lane) ranks rows of the same id by row.
+__global__ void __launch_bounds__(1024) embed_group_kernel(const int* __restrict__ ids, int rows, int V, int pad_id,
+                                                           int* __restrict__ cursor, int* __restrict__ order, int* __restrict__ sid) {
+  __shared__ unsigned keys[1024];
+  __shared__ int ws[32];
+  const int tid = threadIdx.x;
+  for (int i = tid; i < V; i += 1024) cursor[i] = 0;
+  __syncthreads();
+  for (int r = tid; r < rows; r += 1024) {
+    const int id = ids[r];
+    if (id != pad_id && id >= 0 && id < V) atomicAdd(&cursor[id], 1);    // integer counts: order-free
+  }
+  __syncthreads();
+  const int per = (V + 1023) / 1024;
+  const int b0 = min(V, tid * per), b1 = min(V, b0 + per);
+  int cnt = 0;
+  for (int i = b0; i < b1; ++i) cnt += cursor[i];
+  const int incl = block_scan_1024<false>(cnt, ws);
+  int run = incl - cnt;
+  for (int i = b0; i < b1; ++i) { const int c = cursor[i]; cursor[i] = run; run += c; }
+  if (tid == 1023) cursor[V] = incl;
+  __syncthreads();
+  for (int base = 0; base < rows; base += 1024) {
+    const int r = base + tid;
+    const int id = r < rows ? ids[r] : -1;
+    const bool valid = r < rows && id != pad_id && id >= 0 && id < V;
+    keys[tid] = valid ? (((unsigned)id << 10) | (unsigned)tid) : 0xFFFFFFFFu;
+    __syncthreads();
+    for (int k = 2; k <= 1024; k <<= 1)
+      for (int j = k >> 1; j > 0; j >>= 1) {
+        const int p = tid ^ j;
+        if (p > tid) {
+          const unsigned a = keys[tid], b = keys[p];
+          if ((a > b) == ((tid & k) == 0)) { keys[tid] = b; keys[p] = a; }
+        }
+        __syncthreads();
+      }
+    const unsigned key = keys[tid];
+    const unsigned kid = key >> 10;
+    const bool first = tid == 0 || (keys[tid - 1] >> 10) != kid;
+    const bool last = tid == 1023 || (keys[tid + 1] >> 10) != kid;
+    const int start = block_scan_1024<true>(first ? tid : 0, ws);
+    const int rank = tid - start;
+    const bool v = key != 0xFFFFFFFFu;
+    if (v) { order[cursor[kid] + rank] = base + (int)(key & 1023u); sid[cursor[kid] + rank] = (int)kid; }
+    __syncthreads();
+    if (v && last) cursor[kid] += rank + 1;
+    __syncthreads();
+  }
+}
+
+// dE[id] += sum of the dz rows of that id, in a fixed order, with one read-modify-write per element.  The sorted positions are
+// cut into tiles of kScatterTile; embed_scatter_tile_kernel sums each (id, tile) segment in row order.  A group inside one tile
+// is added to dE there; a group that spans tiles leaves its first segment in tail[tile] and every later one in head[tile], and
+// embed_scatter_span_kernel adds tail + head + head + ... in tile order.  So no group is summed by one long serial chain.
+static constexpr int kScatterTile = 64;
+__global__ void __launch_bounds__(256) embed_scatter_tile_kernel(const float* __restrict__ dz, const int* __restrict__ sid,
+                                                                 const int* __restrict__ order, const int* __restrict__ cursor,
+                                                                 int V, float* __restrict__ dE, float* __restrict__ head,
+                                                                 float* __restrict__ tail) {
+  __shared__ int s_row[kScatterTile], s_id[kScatterTile + 2];     // s_id[0]: id before the tile, s_id[n + 1]: id after it
+  const int total = cursor[V];
+  const int t = blockIdx.x, p0 = t * kScatterTile;
+  if (p0 >= total) return;
+  const int n = min(kScatterTile, total - p0);
+  if (threadIdx.x < n) { s_row[threadIdx.x] = order[p0 + threadIdx.x]; s_id[threadIdx.x + 1] = sid[p0 + threadIdx.x]; }
+  if (threadIdx.x == 0) { s_id[0] = p0 > 0 ? sid[p0 - 1] : -1; s_id[n + 1] = p0 + n < total ? sid[p0 + n] : -1; }
+  __syncthreads();
+  const int c = blockIdx.y * 256 + threadIdx.x;
+  float acc = 0.f;
+  int seg = 0;
+  for (int i = 0; i < n; ++i) {
+    acc += dz[(long long)s_row[i] * D + c];
+    if (i == n - 1 || s_id[i + 2] != s_id[i + 1]) {              // the segment ends at i
+      const int id = s_id[i + 1];
+      if (seg == 0 && s_id[0] == id)                  head[(long long)t * D + c] = acc;   // continues a group
+      else if (i == n - 1 && s_id[n + 1] == id)       tail[(long long)t * D + c] = acc;   // starts a group that continues
+      else                                            dE[(long long)id * D + c] += acc;   // the whole group
+      acc = 0.f;
+      seg = i + 1;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256) embed_scatter_span_kernel(const int* __restrict__ sid, const int* __restrict__ cursor, int V,
+                                                                 const float* __restrict__ head, const float* __restrict__ tail,
+                                                                 float* __restrict__ dE) {
+  const int total = cursor[V];
+  const int c = blockIdx.y * 256 + threadIdx.x;
+  for (int p = blockIdx.x; p < total; p += gridDim.x) {
+    const int id = sid[p];
+    if (p > 0 && sid[p - 1] == id) continue;
+    const int ts = p / kScatterTile, te = (cursor[id] - 1) / kScatterTile;      // cursor[id]: end of the group
+    if (ts == te) continue;
+    float acc = tail[(long long)ts * D + c];
+    for (int t = ts + 1; t <= te; ++t) acc += head[(long long)t * D + c];
+    dE[(long long)id * D + c] += acc;
+  }
 }
 
 // ------------------------------------------------------------------ residual + dropout + LayerNorm
@@ -295,13 +458,16 @@ __global__ void __launch_bounds__(256, 2) add_ln_fwd_kernel(const bf16* __restri
 //  produced y — to save the separate colsum launch: a third 16 KB smem accumulator per warp and the extra spills at the
 //  168-register cap made this kernel 27 % slower, 55 -> 70 us, more than the side-stream colsum ever cost.)
 // dgamma / dbeta partial sums live in shared memory ([warp][value i][lane]: conflict-free), not in 64 registers, so
-// three 128-thread blocks fit per SM; one atomic per column per block at the end.
+// three 128-thread blocks fit per SM; one atomic per column per block at the end (kOrdered: the block's column sums go to its row of
+// `partial` [gridDim.x][2 * D] instead, summed by ordered_colsum_kernel).
+template <bool kOrdered>
 __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restrict__ d1, const bf16* __restrict__ d2,
                                                             const bf16* __restrict__ res, const bf16* __restrict__ y,
                                                             const float* __restrict__ gamma, const float* __restrict__ mean_i,
                                                             const float* __restrict__ rstd_i, bf16* __restrict__ dres,
                                                             bf16* __restrict__ dy_out, float* __restrict__ dgamma,
-                                                            float* __restrict__ dbeta, int rows, DropCfg dc_in) {
+                                                            float* __restrict__ dbeta, int rows, DropCfg dc_in,
+                                                            float* __restrict__ partial) {
   pdl_launch_dependents();
   pdl_wait();
   const DropCfg dc = resolve_drop(dc_in);
@@ -374,15 +540,21 @@ __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restri
     const int idx = (j * 8 + k) * 32 + l;
     float a = 0.f, bsum = 0.f;
     for (int w = 0; w < nw; ++w) { a += sacc[w * (2 * VPL * 32) + idx]; bsum += sacc[w * (2 * VPL * 32) + VPL * 32 + idx]; }
-    atomicAdd(dgamma + c, a);
-    atomicAdd(dbeta + c, bsum);
+    if (kOrdered) {
+      partial[(long long)blockIdx.x * 2 * D + c] = a;
+      partial[(long long)blockIdx.x * 2 * D + D + c] = bsum;
+    } else {
+      atomicAdd(dgamma + c, a);
+      atomicAdd(dbeta + c, bsum);
+    }
   }
 }
 
 // ------------------------------------------------------------------ column sums (bias gradients)
-// out[n] += sum_r x[r, n]   x bf16 [rows, ld]; N multiple of 8
+// out[n] += sum_r x[r, n]   x bf16 [rows, ld]; N multiple of 8 (kOrdered: row chunk y stores its sums to partial[y][n])
+template <bool kOrdered>
 __global__ void __launch_bounds__(256) colsum_kernel(const bf16* __restrict__ x, long long ld, int rows, int N,
-                                                     float* __restrict__ out, int rows_per_block) {
+                                                     float* __restrict__ out, int rows_per_block, float* __restrict__ partial) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float sm[8][256];
@@ -421,7 +593,8 @@ __global__ void __launch_bounds__(256) colsum_kernel(const bf16* __restrict__ x,
     float s = 0.f;
 #pragma unroll
     for (int w = 0; w < 8; ++w) s += sm[w][threadIdx.x];
-    atomicAdd(out + c, s);
+    if (kOrdered) partial[(long long)blockIdx.y * N + c] = s;
+    else          atomicAdd(out + c, s);
   }
 }
 
@@ -905,13 +1078,58 @@ extern "C" int mmsum_embed_ln_bwd(const void* dout, const void* dout2, const int
                                   float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
                                   float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, void* stream) {
   if (d_model != D || rows <= 0 || S <= 0 || rows % S || !dz_scratch) return MMSUM_ERR_INVALID;
-  embed_ln_bwd_kernel<<<nblocks(rows, 8 * 4, 148 * 4), 256, 0, STREAM(stream)>>>(
+  embed_ln_bwd_kernel<false><<<nblocks(rows, 8 * 4, 148 * 4), 256, 0, STREAM(stream)>>>(
       reinterpret_cast<const bf16*>(dout), reinterpret_cast<const bf16*>(dout2), ids, E, P, rating_diff, remb, gamma, mean,
       rstd, dE, dz_scratch, dgamma, dbeta,
-      rows, S, pad_id, make_drop(p_drop, seed, stream_id, step_dev));
+      rows, S, pad_id, make_drop(p_drop, seed, stream_id, step_dev), nullptr);
   MMSUM_CHECK_LAUNCH();
-  embed_pos_bwd_kernel<<<dim3(D / 256, S), 256, 0, STREAM(stream)>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S);
+  embed_pos_bwd_kernel<false><<<dim3(D / 256, S), 256, 0, STREAM(stream)>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, nullptr);
   MMSUM_CHECK_LAUNCH();
+  return 0;
+}
+
+static int ordered_colsum(const float* part, int nparts, int width, int split, float* out0, float* out1, cudaStream_t stream) {
+  ordered_colsum_kernel<<<(width + 31) / 32, 256, 0, stream>>>(part, nparts, width, split, out0, out1);
+  MMSUM_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
+                                          const float* rating_diff, const float* remb, const float* gamma, const float* mean,
+                                          const float* rstd, float* dE, float* dP, float* dremb, float* dgamma, float* dbeta,
+                                          float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
+                                          float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, int32_t V,
+                                          float* workspace, int64_t workspace_elems, void* stream) {
+  if (d_model != D || rows <= 0 || S <= 0 || rows % S || !dz_scratch) return MMSUM_ERR_INVALID;
+  if (!dout || !ids || !E || !P || !gamma || !mean || !rstd || !dE || !dP || !dgamma || !dbeta) return MMSUM_ERR_INVALID;
+  if (rating_diff != nullptr && (!remb || !dremb)) return MMSUM_ERR_INVALID;
+  if (V <= 0 || V >= (1 << 22) || !workspace) return MMSUM_ERR_INVALID;
+  const int nblk = nblocks(rows, 8 * 4, 148 * 4);
+  const int ntiles = (rows + kScatterTile - 1) / kScatterTile;
+  if (workspace_elems < (int64_t)nblk * 2 * D + (int64_t)S * D + 2LL * ntiles * D + V + 1 + 2LL * rows) return MMSUM_ERR_INVALID;
+  cudaStream_t st = STREAM(stream);
+  float* part_ln = workspace;
+  float* part_remb = part_ln + (long long)nblk * 2 * D;
+  float* head = part_remb + (long long)S * D;
+  float* tail = head + (long long)ntiles * D;
+  int* cursor = reinterpret_cast<int*>(tail + (long long)ntiles * D);
+  int* order = cursor + V + 1;
+  int* sid = order + rows;
+  embed_ln_bwd_kernel<true><<<nblk, 256, 0, st>>>(
+      reinterpret_cast<const bf16*>(dout), reinterpret_cast<const bf16*>(dout2), ids, E, P, rating_diff, remb, gamma, mean,
+      rstd, dE, dz_scratch, dgamma, dbeta, rows, S, pad_id, make_drop(p_drop, seed, stream_id, step_dev), part_ln);
+  MMSUM_CHECK_LAUNCH();
+  if (int rc = ordered_colsum(part_ln, nblk, 2 * D, D, dgamma, dbeta, st)) return rc;
+  embed_group_kernel<<<1, 1024, 0, st>>>(ids, rows, V, pad_id, cursor, order, sid);
+  MMSUM_CHECK_LAUNCH();
+  embed_scatter_tile_kernel<<<dim3(ntiles, D / 256), 256, 0, st>>>(dz_scratch, sid, order, cursor, V, dE, head, tail);
+  MMSUM_CHECK_LAUNCH();
+  embed_scatter_span_kernel<<<dim3(nblocks(rows, 16, 148 * 4), D / 256), 256, 0, st>>>(sid, cursor, V, head, tail, dE);
+  MMSUM_CHECK_LAUNCH();
+  embed_pos_bwd_kernel<true><<<dim3(D / 256, S), 256, 0, st>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, part_remb);
+  MMSUM_CHECK_LAUNCH();
+  if (rating_diff != nullptr)
+    if (int rc = ordered_colsum(part_remb, S, D, D, dremb, nullptr, st)) return rc;
   return 0;
 }
 
@@ -934,13 +1152,31 @@ extern "C" int mmsum_add_ln_bwd(const void* d1, const void* d2, const void* res,
   if (d_model != D || rows <= 0 || !d1 || !res || !y || !dres || !dy) return MMSUM_ERR_INVALID;
   if (p_drop > 0.f && dres == dy) return MMSUM_ERR_INVALID;
   static std::atomic<unsigned long long> attr{0};
-  if (int rc = ensure_dyn_smem(add_ln_bwd_kernel, 4 * 2 * VPL * 32 * 4, attr)) return rc;
-  MMSUM_LAUNCH_PDL(add_ln_bwd_kernel, nblocks(rows, 4 * 4, 148 * 3), 128, 4 * 2 * VPL * 32 * 4, STREAM(stream), 
+  if (int rc = ensure_dyn_smem(add_ln_bwd_kernel<false>, 4 * 2 * VPL * 32 * 4, attr)) return rc;
+  MMSUM_LAUNCH_PDL(add_ln_bwd_kernel<false>, nblocks(rows, 4 * 4, 148 * 3), 128, 4 * 2 * VPL * 32 * 4, STREAM(stream), 
       reinterpret_cast<const bf16*>(d1), reinterpret_cast<const bf16*>(d2), reinterpret_cast<const bf16*>(res),
       reinterpret_cast<const bf16*>(y), gamma, mean, rstd, reinterpret_cast<bf16*>(dres), reinterpret_cast<bf16*>(dy),
-      dgamma, dbeta, rows, make_drop(p_drop, seed, stream_id, step_dev));
+      dgamma, dbeta, rows, make_drop(p_drop, seed, stream_id, step_dev), nullptr);
   MMSUM_CHECK_LAUNCH();
   return 0;
+}
+
+extern "C" int mmsum_add_ln_bwd_ordered(const void* d1, const void* d2, const void* res, const void* y, const float* gamma,
+                                        const float* mean, const float* rstd, void* dres, void* dy, float* dgamma, float* dbeta,
+                                        int32_t rows, int32_t d_model, float p_drop, uint64_t seed, uint32_t stream_id,
+                                        const uint32_t* step_dev, float* workspace, int64_t workspace_elems, void* stream) {
+  if (d_model != D || rows <= 0 || !d1 || !res || !y || !dres || !dy || !dgamma || !dbeta) return MMSUM_ERR_INVALID;
+  if (p_drop > 0.f && dres == dy) return MMSUM_ERR_INVALID;
+  const int nblk = nblocks(rows, 4 * 4, 148 * 3);
+  if (!workspace || workspace_elems < (int64_t)nblk * 2 * D) return MMSUM_ERR_INVALID;
+  static std::atomic<unsigned long long> attr{0};
+  if (int rc = ensure_dyn_smem(add_ln_bwd_kernel<true>, 4 * 2 * VPL * 32 * 4, attr)) return rc;
+  MMSUM_LAUNCH_PDL(add_ln_bwd_kernel<true>, nblk, 128, 4 * 2 * VPL * 32 * 4, STREAM(stream),
+      reinterpret_cast<const bf16*>(d1), reinterpret_cast<const bf16*>(d2), reinterpret_cast<const bf16*>(res),
+      reinterpret_cast<const bf16*>(y), gamma, mean, rstd, reinterpret_cast<bf16*>(dres), reinterpret_cast<bf16*>(dy),
+      dgamma, dbeta, rows, make_drop(p_drop, seed, stream_id, step_dev), workspace);
+  MMSUM_CHECK_LAUNCH();
+  return ordered_colsum(workspace, nblk, 2 * D, D, dgamma, dbeta, STREAM(stream));
 }
 
 extern "C" int mmsum_colsum(const void* x, int64_t ld, int32_t rows, int32_t N, float* out, void* stream) {
@@ -948,9 +1184,23 @@ extern "C" int mmsum_colsum(const void* x, int64_t ld, int32_t rows, int32_t N, 
   const int gx = (N + 255) / 256;
   int gy = (148 * 4) / gx; if (gy < 1) gy = 1; if (gy > (rows + 63) / 64) gy = (rows + 63) / 64;
   const int rpb = (rows + gy - 1) / gy;
-  MMSUM_LAUNCH_PDL(colsum_kernel, dim3(gx, gy), 256, 0, STREAM(stream), reinterpret_cast<const bf16*>(x), ld, rows, N, out, rpb);
+  MMSUM_LAUNCH_PDL(colsum_kernel<false>, dim3(gx, gy), 256, 0, STREAM(stream), reinterpret_cast<const bf16*>(x), ld, rows, N, out, rpb,
+                   nullptr);
   MMSUM_CHECK_LAUNCH();
   return 0;
+}
+
+extern "C" int mmsum_colsum_ordered(const void* x, int64_t ld, int32_t rows, int32_t N, float* out, float* workspace,
+                                    int64_t workspace_elems, void* stream) {
+  if (!x || !out || rows <= 0 || N <= 0 || (N % 8) || (ld % 8)) return MMSUM_ERR_INVALID;
+  const int gx = (N + 255) / 256;
+  int gy = (148 * 4) / gx; if (gy < 1) gy = 1; if (gy > (rows + 63) / 64) gy = (rows + 63) / 64;
+  const int rpb = (rows + gy - 1) / gy;
+  if (!workspace || workspace_elems < (int64_t)gy * N) return MMSUM_ERR_INVALID;
+  MMSUM_LAUNCH_PDL(colsum_kernel<true>, dim3(gx, gy), 256, 0, STREAM(stream), reinterpret_cast<const bf16*>(x), ld, rows, N, out, rpb,
+                   workspace);
+  MMSUM_CHECK_LAUNCH();
+  return ordered_colsum(workspace, gy, N, N, out, nullptr, STREAM(stream));
 }
 
 extern "C" int mmsum_gate_fwd(const void* o3, const void* u, const uint8_t* pres, void* y, void* ab, int32_t rows,

@@ -133,6 +133,12 @@ class StepEngine:
         self.dropout = cfg.dropout
         self.grad_ready_hook = None      # callable(lo, hi): gradient arena range [lo, hi) is final (data-parallel buckets)
         self.graph_mode = False          # replay forward / backward from recorded CUDA graphs (see forward_step)
+        # torch.are_deterministic_algorithms_enabled() as read by the last forward: its backward then runs the ordered
+        # (bitwise-reproducible) reductions, with their fp32 scratch (main stream / bias-gradient stream) sized per step shape
+        self.det = False
+        self.det_ws = None
+        self.det_ws_side = None
+        self._det_sized = set()
         self._graphs = {}
         self._graph_entry = None
         self._w16_fresh = False          # True only right after a fused optimizer wrote W16 itself
@@ -431,7 +437,8 @@ class StepEngine:
         # one small host sync per step, which costs a graph-launch latency, not the launch-bound step the graphs remove)
         S_in = batch.reviews.shape[-1] if batch.reviews is not None else 0
         frame = self._encoder_frame(batch, S_in) if self.cfg.text_memory else None
-        key = (self._batch_key(batch), bool(training), label_smoothing, frame)
+        self.det = torch.are_deterministic_algorithms_enabled()       # (a replay runs no forward(): the mode is read here too)
+        key = (self._batch_key(batch), bool(training), label_smoothing, frame, self.det)
         ent = self._graphs.get(key)
         if ent is None:
             if len(self._graphs) >= 4:
@@ -498,6 +505,9 @@ class StepEngine:
         S_enc = self._encoder_frame(batch, S) if has_text else S
         w = self._alloc(B, R, S, F, n_img, img_keys, S_enc)
         self.ws = w
+        self.det = torch.are_deterministic_algorithms_enabled()
+        if self.det and training:
+            self._size_ordered_workspaces()       # before any recorded graph of this shape can need it (backward re-checks)
         T, Tt, Te = w["T"], w["Tt"], w["Te"]
         w["batch"] = batch                 # backward re-reads the bit-code table fields
         self.step_count += 1
@@ -603,6 +613,46 @@ class StepEngine:
                 self._len_cache = (weakref.ref(m), m._version, n)
         return min(S, max(16, (int(n) + 15) // 16 * 16))
 
+    def _size_ordered_workspaces(self):
+        """Scratch of the ordered backward, sized once per step shape (like the other workspaces) for every encoder frame the
+        shape can run: the largest split-K partial set of the step's weight-gradient GEMMs, the LayerNorm and embedding partials
+        (main stream), and the bias-gradient partials (side stream).  The split choice is not monotone in the frame, so all
+        frames are visited.  A graph recorded in this mode holds the old scratch's address: when the scratch has to grow, those
+        graphs are dropped.  The library rejects a call whose scratch is too small."""
+        if self.ws_key in self._det_sized:
+            return
+        cfg, w = self.cfg, self.ws_full
+        D, FF, V = cfg.d_model, cfg.ffn_dim, cfg.vocab_size
+        B, R, S, F, T = w["B"], w["R"], w["S"], w["F"], w["T"]
+        side = B * F + B * w["n_img"] * w["img_keys"]
+        frames = range(16, S + 1, 16) if w["Tt"] > 0 and self.trim_frames else [S]
+        shapes = {(V, D, T), (D, FF, T), (FF, D, T), (D, D, T), (3 * D, D, T), (D, D, w["nm"] * T)}
+        need = max(ops.ADD_LN_BWD_WORKSPACE, ops.embed_ln_bwd_workspace(T, S, V))
+        for f in frames:
+            Te = B * R * f
+            shapes.add((2 * D, D, (Te if w["Tt"] > 0 else 0) + side))
+            if w["Tt"] > 0:
+                shapes.update({(D, FF, Te), (FF, D, Te), (D, D, Te), (3 * D, D, Te)})
+                need = max(need, ops.embed_ln_bwd_workspace(Te, f, V))
+        if F > 0:
+            shapes.update({(D, D, B * F), (D, 2 * D, B * F)})
+        if w["n_img"] > 0:
+            shapes.add((D, 1024, B * w["n_img"] * w["img_keys"]))
+        need = max([need] + [ops.gemm_workspace_elems(*sh) for sh in shapes])
+        need_side = ops.colsum_workspace(max(FF, 3 * D))
+        grown = False
+        if self.det_ws is None or self.det_ws.numel() < need:
+            self.det_ws, grown = torch.empty(need, device=self.device, dtype=torch.float32), True
+        if self.det_ws_side is None or self.det_ws_side.numel() < need_side:
+            self.det_ws_side, grown = torch.empty(need_side, device=self.device, dtype=torch.float32), True
+        if grown:
+            self._graphs = {k: e for k, e in self._graphs.items() if not (k[-1] and "bwd" in e)}
+        self._det_sized.add(self.ws_key)
+
+    def _ows(self):
+        """The main-stream scratch of the ordered reductions when this step runs them, else None (the atomic fast path)."""
+        return self.det_ws if self.det else None
+
     def w32_flb(self):
         return self.final_logits_bias.view(-1) if getattr(self, "final_logits_bias", None) is not None else None
 
@@ -612,21 +662,22 @@ class StepEngine:
         out = self.g32(gname, gname2)
         if col_slice is not None:
             out = out[:, col_slice[0]:col_slice[1]]
-        ops.gemm(dy, x, out, a_t=True, b_t=True, accumulate=True)
+        ops.gemm(dy, x, out, a_t=True, b_t=True, accumulate=True, workspace=self._ows())
 
     # Bias gradients (column sums of an upstream-gradient matrix) are short, launch-latency-dominated kernels that sit
     # off the critical dgrad chain: they run on a side stream and overlap the GEMMs that consume the same matrix.  The main
     # stream joins the side stream before any scratch buffer is recycled, before a gradient range is declared final and
     # at the end of backward.
     def _bias_grad(self, x, out):
+        ws = self.det_ws_side if self.det else None
         if self.side_stream is None:
-            ops.colsum(x, out)
+            ops.colsum(x, out, workspace=ws)
             return
         main = torch.cuda.current_stream()
         self._ev_main.record(main)
         self.side_stream.wait_event(self._ev_main)
         with torch.cuda.stream(self.side_stream):
-            ops.colsum(x, out)
+            ops.colsum(x, out, workspace=ws)
             self._ev_side.record(self.side_stream)
         self._side_pending = True
 
@@ -648,7 +699,7 @@ class StepEngine:
         df = pool.get() if pd > 0 else dres
         ops.add_ln_bwd(d1, d2, xin, a["f"], self.w32(lp + "final_layer_norm.weight"), a[mk], a[rk], dres, df,
                        self.g32(lp + "final_layer_norm.weight"), self.g32(lp + "final_layer_norm.bias"), pd, self.seed,
-                       self._sid(kind, l), step_dev=self.step_dev)
+                       self._sid(kind, l), step_dev=self.step_dev, workspace=self._ows())
         pool.put(d1, d2)
         self._bias_grad(df, self.g32(lp + "fc2.bias"))
         self._wgrad(df, a["a"], lp + "fc2.weight")
@@ -670,7 +721,7 @@ class StepEngine:
         do = pool.get() if pd > 0 else dres
         ops.add_ln_bwd(d1, d2, a["x"], a["o"], self.w32(lp + "self_attn_layer_norm.weight"), a["m1"], a["r1"], dres, do,
                        self.g32(lp + "self_attn_layer_norm.weight"), self.g32(lp + "self_attn_layer_norm.bias"), pd, self.seed,
-                       self._sid(kind, l), step_dev=self.step_dev)
+                       self._sid(kind, l), step_dev=self.step_dev, workspace=self._ows())
         pool.put(d1, d2)
         self._bias_grad(do, self.g32(s + "out_proj.bias"))
         self._wgrad(do, a["ctx"], s + "out_proj.weight")
@@ -699,6 +750,8 @@ class StepEngine:
         pool, pd, seed = w["pool"], self.pd, self.seed
         bm = "bart_model.model."
         g = ops.gemm
+        if self.det:
+            self._size_ordered_workspaces()
         first = next(iter(self.params.values()))
         if force_zero or first.grad is None:
             self.G32.zero_()
@@ -710,7 +763,7 @@ class StepEngine:
         d1 = pool.get()
         g(dl, self.w16(bm + "shared.weight"), d1, b_t=True)
         xfin = w["x_out"]
-        ops.gemm(dl, xfin, self.g32(bm + "shared.weight"), a_t=True, b_t=True, accumulate=True)
+        ops.gemm(dl, xfin, self.g32(bm + "shared.weight"), a_t=True, b_t=True, accumulate=True, workspace=self._ows())
         d2 = None
 
         # ---- decoder layers, last to first
@@ -726,7 +779,7 @@ class StepEngine:
             dyc = pool.get() if pd > 0 else dres
             ops.add_ln_bwd(d1, d2, a["x1"], yc, self.w32(lp + "encoder_attn_layer_norm.weight"), a["m2"], a["r2"], dres, dyc,
                            self.g32(lp + "encoder_attn_layer_norm.weight"), self.g32(lp + "encoder_attn_layer_norm.bias"),
-                           pd, seed, self._sid(5, l), step_dev=self.step_dev)
+                           pd, seed, self._sid(5, l), step_dev=self.step_dev, workspace=self._ows())
             pool.put(d1, d2)
             nm = a["A3"].shape[0]
             if gates:
@@ -769,7 +822,8 @@ class StepEngine:
                          w["rating_diff"], self.w32(pre + "rating_embeddings"), self.w32(pre + "layernorm_embedding.weight"),
                          w["dec_m0"], w["dec_r0"], self.g32(bm + "shared.weight"), self.g32(pre + "embed_positions.weight"),
                          self.g32(pre + "rating_embeddings"), self.g32(pre + "layernorm_embedding.weight"),
-                         self.g32(pre + "layernorm_embedding.bias"), w["dz32"], T, S, cfg.pad_token_id, pd, seed, self._sid(3, 0), step_dev=self.step_dev)
+                         self.g32(pre + "layernorm_embedding.bias"), w["dz32"], T, S, cfg.pad_token_id, pd, seed, self._sid(3, 0), step_dev=self.step_dev,
+                         workspace=self._ows())
         pool.put(d1, d2)
         self._ready(pre + "embed_positions.weight")
 
@@ -813,7 +867,8 @@ class StepEngine:
             ops.embed_ln_bwd(d1, d2, w["enc_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"), None, None,
                              self.w32(pre + "layernorm_embedding.weight"), w["enc_m0"], w["enc_r0"], self.g32(bm + "shared.weight"),
                              self.g32(pre + "embed_positions.weight"), None, self.g32(pre + "layernorm_embedding.weight"),
-                             self.g32(pre + "layernorm_embedding.bias"), w["dz32"], Te, S_enc, cfg.pad_token_id, pd, seed, self._sid(0, 0), step_dev=self.step_dev)
+                             self.g32(pre + "layernorm_embedding.bias"), w["dz32"], Te, S_enc, cfg.pad_token_id, pd, seed, self._sid(0, 0), step_dev=self.step_dev,
+                             workspace=self._ows())
             pool.put(d1, d2)
         self._ready(bm + "shared.weight")
         for n, p in self.params.items():

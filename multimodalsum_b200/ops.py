@@ -1,4 +1,5 @@
 """Thin torch-tensor -> C-ABI wrappers.  torch is used for device memory and streams only."""
+import collections
 import ctypes as C
 
 import torch
@@ -11,6 +12,20 @@ LAUNCHES = 0      # kernels launched through the C-ABI since import (bench.py: g
 # Optional instrumentation hook (bench.py roofline): callable(kind, work) -> context manager that brackets ONE C-ABI call with
 # CUDA events on the launching stream.  kind / work: "gemm" FLOPs; "attn_fwd" / "attn_bwd" FLOPs; row kernels algorithmic bytes.
 KERNEL_TIMER = None
+
+# calls of the ordered (bitwise-reproducible) entry points, by entry point
+ORDERED_CALLS = collections.Counter()
+# fp32 workspace elements the ordered row calls need (include/mmsum_b200.h)
+ADD_LN_BWD_WORKSPACE = 444 * 2048
+
+
+def colsum_workspace(N):
+    return max(151552, N)
+
+
+def embed_ln_bwd_workspace(rows, S, V):
+    return 592 * 2048 + S * 1024 + 2048 * ((rows + 63) // 64) + V + 1 + 2 * rows
+
 
 ACT_NONE, ACT_GELU, ACT_RELU = 0, 1, 2
 AUX_NONE, AUX_STORE_PREACT, AUX_MUL_DACT, AUX_STORE_DACT, AUX_MUL = 0, 1, 2, 3, 4
@@ -40,10 +55,11 @@ def _check2d(t, name, dtype=None):
 
 
 def gemm(A, B, out=None, *, a_t=False, b_t=False, out_dtype=torch.bfloat16, bias=None, act=ACT_NONE,
-         aux=None, aux_mode=AUX_NONE, alpha=1.0, accumulate=False, splits=0, block_n=0, raster_m_fast=False):
+         aux=None, aux_mode=AUX_NONE, alpha=1.0, accumulate=False, splits=0, block_n=0, raster_m_fast=False, workspace=None):
     """out[M,N] (+)= epi(alpha * A·Bᵀ).
 
     A: [M,K] (a_t=False) or [K,M] (a_t=True, read MN-major, no copy); B: [N,K] or [K,N] (b_t=True).
+    workspace (fp32, contiguous): ordered split-K (mmsum_gemm_bf16_ordered, bitwise reproducible); see gemm_workspace_elems.
     """
     _check2d(A, "A", torch.bfloat16)
     _check2d(B, "B", torch.bfloat16)
@@ -83,12 +99,39 @@ def gemm(A, B, out=None, *, a_t=False, b_t=False, out_dtype=torch.bfloat16, bias
     a.act, a.aux_mode = act, aux_mode
     a.aux = aux.data_ptr() if aux is not None else None
     a.ld_aux = aux.stride(0) if aux is not None else 0
-    if KERNEL_TIMER is not None:
+    if workspace is not None:
+        _gemm_ordered(a, workspace, M, N, K)
+    elif KERNEL_TIMER is not None:
         with KERNEL_TIMER("gemm", 2.0 * M * N * K):
             check(_lib.lib().mmsum_gemm_bf16(C.byref(a), _stream()), "mmsum_gemm_bf16")
     else:
         check(_lib.lib().mmsum_gemm_bf16(C.byref(a), _stream()), "mmsum_gemm_bf16")
     return out
+
+
+def _gemm_workspace(a):
+    n = C.c_int64(0)
+    _check_rc(_lib.lib().mmsum_gemm_ordered_workspace(C.byref(a), C.byref(n)), "mmsum_gemm_ordered_workspace")
+    return n.value
+
+
+def gemm_workspace_elems(M, N, K, *, a_t=True, b_t=True):
+    """fp32 workspace elements of an ordered fp32 accumulating GEMM of this shape (0: one split, nothing to order)."""
+    a = GemmArgs()
+    a.M, a.N, a.K = M, N, K
+    a.a_mn_major, a.b_mn_major = int(a_t), int(b_t)
+    a.out_f32, a.accumulate = 1, 1
+    return _gemm_workspace(a)
+
+
+def _gemm_ordered(a, workspace, M, N, K):
+    if workspace.dtype != torch.float32 or not workspace.is_contiguous() or not workspace.is_cuda:
+        raise ValueError("workspace must be a contiguous fp32 CUDA tensor")
+    n_kernels = 2 if _gemm_workspace(a) > 0 else 1
+    ORDERED_CALLS["gemm"] += 1
+    _timed("gemm_ordered" if n_kernels == 2 else "gemm", 2.0 * M * N * K,
+           lambda: check(_lib.lib().mmsum_gemm_bf16_ordered(C.byref(a), _ptr(workspace), C.c_int64(workspace.numel()), _stream()),
+                         "mmsum_gemm_bf16_ordered", n_kernels))
 
 
 def gemm_cat(A, A2, B, out=None, *, bias=None, out_dtype=torch.bfloat16):
@@ -143,7 +186,16 @@ def _embed_ln_fwd(ids, E, P, rating_diff, remb, gamma, beta, out, mean, rstd, ro
 
 
 def embed_ln_bwd(dout, dout2, ids, E, P, rating_diff, remb, gamma, mean, rstd, dE, dP, dremb, dgamma, dbeta, dz, rows, S,
-                 pad_id, p_drop, seed, sid, step_dev=None):
+                 pad_id, p_drop, seed, sid, step_dev=None, workspace=None):
+    """workspace (fp32, >= embed_ln_bwd_workspace(rows, S, E.shape[0]) elements): the ordered variant (bitwise reproducible)."""
+    if workspace is not None:
+        ORDERED_CALLS["embed_ln_bwd"] += 1
+        _timed("embed_ln_bwd_ordered", rows * E.shape[1] * 12.0, lambda: check(_lib.lib().mmsum_embed_ln_bwd_ordered(
+            _ptr(dout), _ptr(dout2), _ptr(ids), _ptr(E), _ptr(P), _ptr(rating_diff), _ptr(remb), _ptr(gamma), _ptr(mean),
+            _ptr(rstd), _ptr(dE), _ptr(dP), _ptr(dremb), _ptr(dgamma), _ptr(dbeta), _ptr(dz), rows, S, E.shape[1], pad_id,
+            C.c_float(p_drop), C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), E.shape[0], _ptr(workspace),
+            C.c_int64(workspace.numel()), _stream()), "mmsum_embed_ln_bwd_ordered", 6 if rating_diff is not None else 5))
+        return
     check(_lib.lib().mmsum_embed_ln_bwd(_ptr(dout), _ptr(dout2), _ptr(ids), _ptr(E), _ptr(P), _ptr(rating_diff), _ptr(remb),
                                         _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dE), _ptr(dP), _ptr(dremb), _ptr(dgamma),
                                         _ptr(dbeta), _ptr(dz), rows, S, E.shape[1], pad_id, C.c_float(p_drop),
@@ -161,9 +213,17 @@ def _add_ln_fwd(res, y, gamma, beta, out, mean, rstd, p_drop, seed, sid, step_de
                                       C.c_float(p_drop), C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), _stream()), "mmsum_add_ln_fwd")
 
 
-def add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_drop, seed, sid, step_dev=None):
+def add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_drop, seed, sid, step_dev=None, workspace=None):
+    """workspace (fp32, >= ADD_LN_BWD_WORKSPACE elements): the ordered variant (bitwise reproducible)."""
     rows, d = res.shape
     n_mats = 3 + (1 if d2 is not None else 0) + 1 + (1 if dy.data_ptr() != dres.data_ptr() else 0)   # d1 (+d2), res, y in; dres (+dy) out
+    if workspace is not None:
+        ORDERED_CALLS["add_ln_bwd"] += 1
+        _timed("add_ln_bwd_ordered", float(n_mats) * rows * d * 2, lambda: check(_lib.lib().mmsum_add_ln_bwd_ordered(
+            _ptr(d1), _ptr(d2), _ptr(res), _ptr(y), _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dres), _ptr(dy), _ptr(dgamma),
+            _ptr(dbeta), rows, d, C.c_float(p_drop), C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), _ptr(workspace),
+            C.c_int64(workspace.numel()), _stream()), "mmsum_add_ln_bwd_ordered", 2))
+        return
     _timed("add_ln_bwd", float(n_mats) * rows * d * 2, lambda: _add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_drop, seed, sid, step_dev))
 
 
@@ -174,9 +234,16 @@ def _add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_dr
                                       C.c_uint32(sid), _ptr(step_dev), _stream()), "mmsum_add_ln_bwd")
 
 
-def colsum(x, out):
-    """out[n] += Σ_r x[r, n]  (x bf16 2-D, possibly a column-slice view)."""
+def colsum(x, out, workspace=None):
+    """out[n] += Σ_r x[r, n]  (x bf16 2-D, possibly a column-slice view).  workspace (fp32, >= colsum_workspace(N) elements):
+    the ordered variant (bitwise reproducible)."""
     _check2d(x, "x", torch.bfloat16)
+    if workspace is not None:
+        ORDERED_CALLS["colsum"] += 1
+        _timed("colsum_ordered", 2.0 * x.shape[0] * x.shape[1], lambda: check(_lib.lib().mmsum_colsum_ordered(
+            _ptr(x), C.c_int64(x.stride(0)), x.shape[0], x.shape[1], _ptr(out), _ptr(workspace), C.c_int64(workspace.numel()),
+            _stream()), "mmsum_colsum_ordered", 2))
+        return
     _timed("colsum", 2.0 * x.shape[0] * x.shape[1], lambda: _colsum(x, out))
 
 
