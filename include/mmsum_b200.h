@@ -64,7 +64,9 @@ typedef struct MmsumAttnMod {
   int32_t loo;         /* 1: entity e is skipped for target e */
   int32_t ent_base;    /* index of entity 0 of this modality in the [.., E_total] arrays */
   int32_t ent_stride;  /* KV rows between consecutive entities (0 = Sk); > Sk when entity frames are padded */
-  int32_t reserved;
+  int32_t no_dkv;      /* bwd: 1 = this modality's dK/dV is not wanted (frozen k/v projections and memory producer): its key tiles
+                          are not enumerated and its dKV rows are not written; with every modality flagged only the dQ/DELTA pass
+                          runs.  0 or 1; ignored by the forward and the decode step */
 } MmsumAttnMod;
 
 typedef struct MmsumAttnArgs {
@@ -154,7 +156,11 @@ int mmsum_embed_ln_fwd(const int32_t* ids, const float* E, const float* P, const
 int mmsum_embed_ln_decode(const int32_t* ids, const float* E, const float* P, const float* rating_diff, const float* remb,
                           const float* gamma, const float* beta, void* out, float* mean, float* rstd, int32_t rows,
                           int32_t d_model, const int32_t* pos_dev, void* stream);
-/* backward: scatter-add into dE (pad id skipped, nn.Embedding(padding_idx=1) :1001), dP, dremb, dgamma, dbeta (all +=) */
+/* backward: scatter-add into dE (pad id skipped, nn.Embedding(padding_idx=1) :1001), dP, dremb, dgamma, dbeta (all +=).
+ * Each of dE, dP, dremb and the pair dgamma / dbeta may be NULL (a frozen parameter): that output is not computed, and the kernel
+ * that only serves it is not launched; the other outputs are bitwise those of the full call.  One of dgamma / dbeta alone is
+ * rejected; with every output NULL nothing is launched.  rating_diff needs remb (the forward's input is recomputed) even when
+ * dremb is NULL. */
 int mmsum_embed_ln_bwd(const void* dout, const void* dout2 /* optional addend */, const int32_t* ids, const float* E, const float* P, const float* rating_diff,
                        const float* remb, const float* gamma, const float* mean, const float* rstd, float* dE, float* dP,
                        float* dremb, float* dgamma, float* dbeta, float* dz_scratch, int32_t rows, int32_t S,
@@ -166,7 +172,9 @@ int mmsum_embed_ln_bwd(const void* dout, const void* dout2 /* optional addend */
 int mmsum_add_ln_fwd(const void* res, const void* y, const float* gamma, const float* beta, void* out, float* mean,
                      float* rstd, int32_t rows, int32_t d_model, float p_drop, uint64_t seed, uint32_t stream_id,
                      const uint32_t* step_dev, void* stream);
-/* backward: upstream = d1 (+ d2 if not NULL); dres = dz, dy = dz * mask (may alias dres when p_drop == 0); dgamma/dbeta += */
+/* backward: upstream = d1 (+ d2 if not NULL); dres = dz, dy = dz * mask (may alias dres when p_drop == 0); dgamma/dbeta +=.
+ * dgamma = dbeta = NULL (a frozen LayerNorm) runs a variant without the gamma / beta reduction, with the same dres / dy bits;
+ * one of the two alone is rejected.  The same holds for mmsum_add_ln_bwd_ordered, which then needs no workspace. */
 int mmsum_add_ln_bwd(const void* d1, const void* d2, const void* res, const void* y, const float* gamma, const float* mean,
                      const float* rstd, void* dres, void* dy, float* dgamma, float* dbeta, int32_t rows, int32_t d_model,
                      float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, void* stream);
@@ -258,6 +266,15 @@ int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_
                                float* dE, float* dP, float* dremb, float* dgamma, float* dbeta, float* dz_scratch, int32_t rows,
                                int32_t S, int32_t d_model, int32_t pad_id, float p_drop, uint64_t seed, uint32_t stream_id,
                                const uint32_t* step_dev, int32_t V, float* workspace, int64_t workspace_elems, void* stream);
+/* mmsum_embed_ln_bwd_ordered requires every output (dremb when rating_diff is given); mmsum_embed_ln_bwd_ordered_subset is the same
+ * call where, as for mmsum_embed_ln_bwd, each of dE, dP, dremb and the pair dgamma / dbeta may be NULL and is then not computed
+ * (dE == NULL launches none of the sort / scatter kernels), but not all of them. */
+int mmsum_embed_ln_bwd_ordered_subset(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
+                                      const float* rating_diff, const float* remb, const float* gamma, const float* mean,
+                                      const float* rstd, float* dE, float* dP, float* dremb, float* dgamma, float* dbeta,
+                                      float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id, float p_drop,
+                                      uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, int32_t V, float* workspace,
+                                      int64_t workspace_elems, void* stream);
 /* mmsum_table_bits_bwd needs no variant: each dW element is summed by one thread in a fixed order and added once. */
 
 /* ---- optimizer over the flat arenas ---------------------------------------------------------------

@@ -32,7 +32,7 @@ class GemmArgs(C.Structure):
 
 class AttnMod(C.Structure):
     _fields_ = [("kv_row_base", C.c_int64), ("o_off", C.c_int64), ("E", C.c_int32), ("Sk", C.c_int32),
-                ("loo", C.c_int32), ("ent_base", C.c_int32), ("ent_stride", C.c_int32), ("reserved", C.c_int32)]
+                ("loo", C.c_int32), ("ent_base", C.c_int32), ("ent_stride", C.c_int32), ("no_dkv", C.c_int32)]
 
 
 class AttnArgs(C.Structure):
@@ -93,7 +93,7 @@ EXPORTS = [
     "mmsum_embed_ln_decode", "mmsum_attn_decode_cross", "mmsum_attn_decode_self", "mmsum_beam_topk", "mmsum_beam_update",
     "mmsum_sample_token",
     "mmsum_gemm_bf16_ordered", "mmsum_gemm_ordered_workspace", "mmsum_add_ln_bwd_ordered", "mmsum_colsum_ordered",
-    "mmsum_embed_ln_bwd_ordered",
+    "mmsum_embed_ln_bwd_ordered", "mmsum_embed_ln_bwd_ordered_subset",
 ]
 
 

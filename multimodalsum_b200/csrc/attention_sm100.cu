@@ -845,6 +845,8 @@ __host__ __device__ inline bool mod_packed(const MmsumAttnMod& md) {
 __host__ __device__ inline int mod_tiles(const MmsumAttnMod& md) {
   return mod_packed(md) ? (md.E * md.Sk + SQ - 1) / SQ : md.E * ((md.Sk + SQ - 1) / SQ);
 }
+// key tiles of the dK/dV pass: none for a modality whose dK/dV is not wanted (its dKV rows are left as they are)
+__host__ __device__ inline int dkv_tiles(const MmsumAttnMod& md) { return md.no_dkv ? 0 : mod_tiles(md); }
 
 static constexpr int kKvStages = 4;                 // Q / dA ring depth (P^T / dS^T stay in TMEM, so smem has room for four)
 struct BwdKVSmem {
@@ -882,7 +884,7 @@ attn_bwd_dkv_tc_kernel(const __grid_constant__ CUtensorMap q64, const __grid_con
   const int h_begin = (bh % hgroups) * head_mode, h_end = h_begin + head_mode;
   int m = 0;
   for (m = 0; m < p.n_mod; ++m) {
-    const int cnt = mod_tiles(p.mods[m]);
+    const int cnt = dkv_tiles(p.mods[m]);
     if (rem < cnt) break;
     rem -= cnt;
   }
@@ -1181,6 +1183,8 @@ static int validate_tc(const MmsumAttnArgs* a, bool bwd) {
   if (bwd) {
     if (!a->DELTA || !a->dQ || !a->dKV) return MMSUM_ERR_INVALID;
     if ((a->lddq % 8) || (a->lddkv % 8) || (a->dq_col % 8) || (a->dk_col % 8) || (a->dv_col % 8)) return MMSUM_ERR_INVALID;
+    for (int m = 0; m < a->n_mod; ++m)
+      if (a->mods[m].no_dkv != 0 && a->mods[m].no_dkv != 1) return MMSUM_ERR_INVALID;
   }
   return 0;
 }
@@ -1276,7 +1280,7 @@ extern "C" int mmsum_attn_bwd(const MmsumAttnArgs* a, void* stream_v) {
   for (int m = 0; m < a->n_mod; ++m) {
     const uint64_t r = (uint64_t)a->mods[m].kv_row_base + (uint64_t)n_biz * a->mods[m].E * (a->mods[m].ent_stride > 0 ? a->mods[m].ent_stride : a->mods[m].Sk);
     if (r > kvrows) kvrows = r;
-    tiles += mod_tiles(a->mods[m]);
+    tiles += dkv_tiles(a->mods[m]);
   }
   CUtensorMap kv128, q64, do64;
   if (int rc = make_tmap(&kv128, a->KV, 0, (uint64_t)a->ldkv, kvrows, (uint64_t)a->ldkv * 2, 64, SQ)) return rc;
@@ -1303,7 +1307,7 @@ extern "C" int mmsum_attn_bwd(const MmsumAttnArgs* a, void* stream_v) {
     MMSUM_LAUNCH_PDL(attn_bwd_dq_tc_kernel, head_mode ? a->n_qseq : a->n_qseq * a->H, kAttnThreads, smem_q, stream, mp, *a, head_mode);
     MMSUM_CHECK_LAUNCH();
   }
-  if (part != 1) {
+  if (part != 1 && tiles > 0) {
     // self-attention shape: 4 heads per CTA (amortises the set-up, still ~2 waves of 2 CTAs/SM at 144 sequences)
     const int heads_per_cta = (a->n_mod == 1 && a->mods[0].E == 1 && !a->mods[0].loo && n_biz >= 64 && a->H % 4 == 0) ? 4 : 1;
     MMSUM_LAUNCH_PDL(attn_bwd_dkv_tc_kernel, n_biz * (a->H / heads_per_cta) * tiles, kKvThreads, smem_kv, stream, q64, do64, kv128, *a,

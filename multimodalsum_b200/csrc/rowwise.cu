@@ -133,6 +133,7 @@ __global__ void __launch_bounds__(256) embed_ln_fwd_kernel(const int* __restrict
 // skipped: nn.Embedding(padding_idx=1)), dgamma/dbeta.
 // kOrdered: no dE scatter (embed_group_kernel + embed_scatter_tile/span_kernel add the dz rows per token id instead) and the
 // block's dgamma / dbeta sums go to its own row of `partial` [gridDim.x][2 * D] (ordered_colsum_kernel adds them up).
+// dE == NULL: no scatter; dgamma == NULL (then dbeta == NULL too): no gamma / beta flush.  dz is always written.
 template <bool kOrdered>
 __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restrict__ dout, const bf16* __restrict__ dout2,
                                                            const int* __restrict__ ids,
@@ -193,9 +194,10 @@ __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restric
       const int c = col_of(lane, i);
       const float dz = rstd * (dy[i] - s1 - z[i] * s2);
       dzr[c] = dz;
-      if (!kOrdered && id != pad_id) atomicAdd(der + c, dz);
+      if (!kOrdered && dE != nullptr && id != pad_id) atomicAdd(der + c, dz);
     }
   }
+  if (dgamma == nullptr) return;   // uniform over the block
   // block reduce dgamma/dbeta then one atomic per column per block
   for (int pass = 0; pass < 2; ++pass) {
     float* acc = pass == 0 ? ag : ab;
@@ -215,7 +217,7 @@ __global__ void __launch_bounds__(256) embed_ln_bwd_kernel(const bf16* __restric
   }
 }
 
-// dP[t+2] += sum_seq dz[seq*S+t],  dremb += sum_rows rating_diff[seq] * dz[row]
+// dP[t+2] += sum_seq dz[seq*S+t],  dremb += sum_rows rating_diff[seq] * dz[row]   (dP or dremb may be NULL: not written)
 // (every dP element has exactly one writer, so its single atomic is already order-free; the S blocks of a column all add into
 //  dremb, so kOrdered stores the position's dremb sum to partial[t][c] instead, summed over t by ordered_colsum_kernel)
 template <bool kOrdered>
@@ -225,14 +227,15 @@ __global__ void __launch_bounds__(256) embed_pos_bwd_kernel(const float* __restr
   // grid: (D/256, S); thread = one column, loops over sequences
   const int c = blockIdx.x * 256 + threadIdx.x;
   const int t = blockIdx.y;
+  const bool remb_on = rating_diff != nullptr && dremb != nullptr;
   float s = 0.f, r = 0.f;
   for (int q = 0; q < n_seq; ++q) {
     const float v = dz[((long long)q * S + t) * D + c];
     s += v;
-    if (rating_diff != nullptr) r += rating_diff[q] * v;
+    if (remb_on) r += rating_diff[q] * v;
   }
-  atomicAdd(dP + (long long)(t + 2) * D + c, s);
-  if (rating_diff != nullptr) {
+  if (dP != nullptr) atomicAdd(dP + (long long)(t + 2) * D + c, s);
+  if (remb_on) {
     if (kOrdered) partial[(long long)t * D + c] = r;
     else          atomicAdd(dremb + c, r);
   }
@@ -460,7 +463,8 @@ __global__ void __launch_bounds__(256, 2) add_ln_fwd_kernel(const bf16* __restri
 // dgamma / dbeta partial sums live in shared memory ([warp][value i][lane]: conflict-free), not in 64 registers, so
 // three 128-thread blocks fit per SM; one atomic per column per block at the end (kOrdered: the block's column sums go to its row of
 // `partial` [gridDim.x][2 * D] instead, summed by ordered_colsum_kernel).
-template <bool kOrdered>
+// !kGrads (frozen LayerNorm: dgamma = dbeta = NULL): no accumulators and no flush, the same dres / dy bits.
+template <bool kOrdered, bool kGrads = true>
 __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restrict__ d1, const bf16* __restrict__ d2,
                                                             const bf16* __restrict__ res, const bf16* __restrict__ y,
                                                             const float* __restrict__ gamma, const float* __restrict__ mean_i,
@@ -475,8 +479,10 @@ __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restri
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   float* sg = sacc + warp * (2 * VPL * 32);
   float* sb = sg + VPL * 32;
+  if (kGrads) {
 #pragma unroll
-  for (int i = 0; i < VPL; ++i) { sg[i * 32 + lane] = 0.f; sb[i * 32 + lane] = 0.f; }
+    for (int i = 0; i < VPL; ++i) { sg[i * 32 + lane] = 0.f; sb[i * 32 + lane] = 0.f; }
+  }
   for (int row = blockIdx.x * nw + warp; row < rows; row += gridDim.x * nw) {
     // all 12-16 global loads of the row are issued before the first use (the kernel is latency-bound otherwise)
     uint4 ry[4], rr[4], r1[4], r2[4];
@@ -517,8 +523,10 @@ __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restri
 #pragma unroll
       for (int k = 0; k < 8; ++k) {
         const int i = j * 8 + k;
-        sg[i * 32 + lane] += t[i] * z[i];
-        sb[i * 32 + lane] += t[i];
+        if (kGrads) {
+          sg[i * 32 + lane] += t[i] * z[i];
+          sb[i * 32 + lane] += t[i];
+        }
         t[i] *= gg[k];                                                          // t := d xhat
         s1 += t[i]; s2 += t[i] * z[i];
       }
@@ -533,6 +541,7 @@ __global__ void __launch_bounds__(128, 3) add_ln_bwd_kernel(const bf16* __restri
       store_row_bf16(dy_out + (long long)row * D, lane, t);
     }
   }
+  if (!kGrads) return;
   __syncthreads();
   // column c = (i>>3)*256 + lane*8 + (i&7)  <->  (i, lane)
   for (int c = threadIdx.x; c < D; c += blockDim.x) {
@@ -1078,13 +1087,18 @@ extern "C" int mmsum_embed_ln_bwd(const void* dout, const void* dout2, const int
                                   float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
                                   float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, void* stream) {
   if (d_model != D || rows <= 0 || S <= 0 || rows % S || !dz_scratch) return MMSUM_ERR_INVALID;
+  if ((dgamma == nullptr) != (dbeta == nullptr) || (rating_diff != nullptr && !remb)) return MMSUM_ERR_INVALID;
+  const bool want_remb = rating_diff != nullptr && dremb != nullptr;
+  if (!dE && !dgamma && !dP && !want_remb) return 0;
   embed_ln_bwd_kernel<false><<<nblocks(rows, 8 * 4, 148 * 4), 256, 0, STREAM(stream)>>>(
       reinterpret_cast<const bf16*>(dout), reinterpret_cast<const bf16*>(dout2), ids, E, P, rating_diff, remb, gamma, mean,
       rstd, dE, dz_scratch, dgamma, dbeta,
       rows, S, pad_id, make_drop(p_drop, seed, stream_id, step_dev), nullptr);
   MMSUM_CHECK_LAUNCH();
-  embed_pos_bwd_kernel<false><<<dim3(D / 256, S), 256, 0, STREAM(stream)>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, nullptr);
-  MMSUM_CHECK_LAUNCH();
+  if (dP || want_remb) {
+    embed_pos_bwd_kernel<false><<<dim3(D / 256, S), 256, 0, STREAM(stream)>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, nullptr);
+    MMSUM_CHECK_LAUNCH();
+  }
   return 0;
 }
 
@@ -1094,15 +1108,19 @@ static int ordered_colsum(const float* part, int nparts, int width, int split, f
   return 0;
 }
 
-extern "C" int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
-                                          const float* rating_diff, const float* remb, const float* gamma, const float* mean,
-                                          const float* rstd, float* dE, float* dP, float* dremb, float* dgamma, float* dbeta,
-                                          float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
-                                          float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, int32_t V,
-                                          float* workspace, int64_t workspace_elems, void* stream) {
+// the ordered embedding backward; each of dE, dP, dremb and the pair dgamma / dbeta may be NULL (not computed), not all of them
+static int embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
+                                const float* rating_diff, const float* remb, const float* gamma, const float* mean,
+                                const float* rstd, float* dE, float* dP, float* dremb, float* dgamma, float* dbeta,
+                                float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
+                                float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, int32_t V,
+                                float* workspace, int64_t workspace_elems, void* stream) {
   if (d_model != D || rows <= 0 || S <= 0 || rows % S || !dz_scratch) return MMSUM_ERR_INVALID;
-  if (!dout || !ids || !E || !P || !gamma || !mean || !rstd || !dE || !dP || !dgamma || !dbeta) return MMSUM_ERR_INVALID;
-  if (rating_diff != nullptr && (!remb || !dremb)) return MMSUM_ERR_INVALID;
+  if (!dout || !ids || !E || !P || !gamma || !mean || !rstd) return MMSUM_ERR_INVALID;
+  if ((dgamma == nullptr) != (dbeta == nullptr)) return MMSUM_ERR_INVALID;
+  if (rating_diff != nullptr && !remb) return MMSUM_ERR_INVALID;
+  const bool want_remb = rating_diff != nullptr && dremb != nullptr;
+  if (!dE && !dgamma && !dP && !want_remb) return MMSUM_ERR_INVALID;
   if (V <= 0 || V >= (1 << 22) || !workspace) return MMSUM_ERR_INVALID;
   const int nblk = nblocks(rows, 8 * 4, 148 * 4);
   const int ntiles = (rows + kScatterTile - 1) / kScatterTile;
@@ -1119,18 +1137,45 @@ extern "C" int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, c
       reinterpret_cast<const bf16*>(dout), reinterpret_cast<const bf16*>(dout2), ids, E, P, rating_diff, remb, gamma, mean,
       rstd, dE, dz_scratch, dgamma, dbeta, rows, S, pad_id, make_drop(p_drop, seed, stream_id, step_dev), part_ln);
   MMSUM_CHECK_LAUNCH();
-  if (int rc = ordered_colsum(part_ln, nblk, 2 * D, D, dgamma, dbeta, st)) return rc;
-  embed_group_kernel<<<1, 1024, 0, st>>>(ids, rows, V, pad_id, cursor, order, sid);
-  MMSUM_CHECK_LAUNCH();
-  embed_scatter_tile_kernel<<<dim3(ntiles, D / 256), 256, 0, st>>>(dz_scratch, sid, order, cursor, V, dE, head, tail);
-  MMSUM_CHECK_LAUNCH();
-  embed_scatter_span_kernel<<<dim3(nblocks(rows, 16, 148 * 4), D / 256), 256, 0, st>>>(sid, cursor, V, head, tail, dE);
-  MMSUM_CHECK_LAUNCH();
-  embed_pos_bwd_kernel<true><<<dim3(D / 256, S), 256, 0, st>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, part_remb);
-  MMSUM_CHECK_LAUNCH();
-  if (rating_diff != nullptr)
+  if (dgamma != nullptr)
+    if (int rc = ordered_colsum(part_ln, nblk, 2 * D, D, dgamma, dbeta, st)) return rc;
+  if (dE != nullptr) {
+    embed_group_kernel<<<1, 1024, 0, st>>>(ids, rows, V, pad_id, cursor, order, sid);
+    MMSUM_CHECK_LAUNCH();
+    embed_scatter_tile_kernel<<<dim3(ntiles, D / 256), 256, 0, st>>>(dz_scratch, sid, order, cursor, V, dE, head, tail);
+    MMSUM_CHECK_LAUNCH();
+    embed_scatter_span_kernel<<<dim3(nblocks(rows, 16, 148 * 4), D / 256), 256, 0, st>>>(sid, cursor, V, head, tail, dE);
+    MMSUM_CHECK_LAUNCH();
+  }
+  if (dP != nullptr || want_remb) {
+    embed_pos_bwd_kernel<true><<<dim3(D / 256, S), 256, 0, st>>>(dz_scratch, rating_diff, dP, dremb, rows / S, S, part_remb);
+    MMSUM_CHECK_LAUNCH();
+  }
+  if (want_remb)
     if (int rc = ordered_colsum(part_remb, S, D, D, dremb, nullptr, st)) return rc;
   return 0;
+}
+
+extern "C" int mmsum_embed_ln_bwd_ordered(const void* dout, const void* dout2, const int32_t* ids, const float* E, const float* P,
+                                          const float* rating_diff, const float* remb, const float* gamma, const float* mean,
+                                          const float* rstd, float* dE, float* dP, float* dremb, float* dgamma, float* dbeta,
+                                          float* dz_scratch, int32_t rows, int32_t S, int32_t d_model, int32_t pad_id,
+                                          float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev, int32_t V,
+                                          float* workspace, int64_t workspace_elems, void* stream) {
+  if (!dE || !dP || !dgamma || !dbeta || (rating_diff != nullptr && !dremb)) return MMSUM_ERR_INVALID;
+  return embed_ln_bwd_ordered(dout, dout2, ids, E, P, rating_diff, remb, gamma, mean, rstd, dE, dP, dremb, dgamma, dbeta, dz_scratch,
+                              rows, S, d_model, pad_id, p_drop, seed, stream_id, step_dev, V, workspace, workspace_elems, stream);
+}
+
+extern "C" int mmsum_embed_ln_bwd_ordered_subset(const void* dout, const void* dout2, const int32_t* ids, const float* E,
+                                                 const float* P, const float* rating_diff, const float* remb, const float* gamma,
+                                                 const float* mean, const float* rstd, float* dE, float* dP, float* dremb,
+                                                 float* dgamma, float* dbeta, float* dz_scratch, int32_t rows, int32_t S,
+                                                 int32_t d_model, int32_t pad_id, float p_drop, uint64_t seed, uint32_t stream_id,
+                                                 const uint32_t* step_dev, int32_t V, float* workspace, int64_t workspace_elems,
+                                                 void* stream) {
+  return embed_ln_bwd_ordered(dout, dout2, ids, E, P, rating_diff, remb, gamma, mean, rstd, dE, dP, dremb, dgamma, dbeta, dz_scratch,
+                              rows, S, d_model, pad_id, p_drop, seed, stream_id, step_dev, V, workspace, workspace_elems, stream);
 }
 
 extern "C" int mmsum_add_ln_fwd(const void* res, const void* y, const float* gamma, const float* beta, void* out,
@@ -1145,12 +1190,27 @@ extern "C" int mmsum_add_ln_fwd(const void* res, const void* y, const float* gam
   return 0;
 }
 
+// dgamma = dbeta = NULL: the variant without the gamma / beta reduction (one kernel, nothing to order)
+static int add_ln_bwd_frozen(const void* d1, const void* d2, const void* res, const void* y, const float* gamma, const float* mean,
+                             const float* rstd, void* dres, void* dy, int32_t rows, float p_drop, uint64_t seed, uint32_t stream_id,
+                             const uint32_t* step_dev, void* stream) {
+  MMSUM_LAUNCH_PDL((add_ln_bwd_kernel<false, false>), nblocks(rows, 4 * 4, 148 * 3), 128, 0, STREAM(stream),
+      reinterpret_cast<const bf16*>(d1), reinterpret_cast<const bf16*>(d2), reinterpret_cast<const bf16*>(res),
+      reinterpret_cast<const bf16*>(y), gamma, mean, rstd, reinterpret_cast<bf16*>(dres), reinterpret_cast<bf16*>(dy),
+      nullptr, nullptr, rows, make_drop(p_drop, seed, stream_id, step_dev), nullptr);
+  MMSUM_CHECK_LAUNCH();
+  return 0;
+}
+
 extern "C" int mmsum_add_ln_bwd(const void* d1, const void* d2, const void* res, const void* y, const float* gamma,
                                 const float* mean, const float* rstd, void* dres, void* dy, float* dgamma, float* dbeta,
                                 int32_t rows, int32_t d_model, float p_drop, uint64_t seed, uint32_t stream_id, const uint32_t* step_dev,
                                 void* stream) {
   if (d_model != D || rows <= 0 || !d1 || !res || !y || !dres || !dy) return MMSUM_ERR_INVALID;
   if (p_drop > 0.f && dres == dy) return MMSUM_ERR_INVALID;
+  if ((dgamma == nullptr) != (dbeta == nullptr)) return MMSUM_ERR_INVALID;
+  if (dgamma == nullptr)
+    return add_ln_bwd_frozen(d1, d2, res, y, gamma, mean, rstd, dres, dy, rows, p_drop, seed, stream_id, step_dev, stream);
   static std::atomic<unsigned long long> attr{0};
   if (int rc = ensure_dyn_smem(add_ln_bwd_kernel<false>, 4 * 2 * VPL * 32 * 4, attr)) return rc;
   MMSUM_LAUNCH_PDL(add_ln_bwd_kernel<false>, nblocks(rows, 4 * 4, 148 * 3), 128, 4 * 2 * VPL * 32 * 4, STREAM(stream), 
@@ -1165,8 +1225,11 @@ extern "C" int mmsum_add_ln_bwd_ordered(const void* d1, const void* d2, const vo
                                         const float* mean, const float* rstd, void* dres, void* dy, float* dgamma, float* dbeta,
                                         int32_t rows, int32_t d_model, float p_drop, uint64_t seed, uint32_t stream_id,
                                         const uint32_t* step_dev, float* workspace, int64_t workspace_elems, void* stream) {
-  if (d_model != D || rows <= 0 || !d1 || !res || !y || !dres || !dy || !dgamma || !dbeta) return MMSUM_ERR_INVALID;
+  if (d_model != D || rows <= 0 || !d1 || !res || !y || !dres || !dy) return MMSUM_ERR_INVALID;
   if (p_drop > 0.f && dres == dy) return MMSUM_ERR_INVALID;
+  if ((dgamma == nullptr) != (dbeta == nullptr)) return MMSUM_ERR_INVALID;
+  if (dgamma == nullptr)      // no reduction left to order: the workspace is not read
+    return add_ln_bwd_frozen(d1, d2, res, y, gamma, mean, rstd, dres, dy, rows, p_drop, seed, stream_id, step_dev, stream);
   const int nblk = nblocks(rows, 4 * 4, 148 * 3);
   if (!workspace || workspace_elems < (int64_t)nblk * 2 * D) return MMSUM_ERR_INVALID;
   static std::atomic<unsigned long long> attr{0};

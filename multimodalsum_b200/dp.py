@@ -31,6 +31,7 @@ class GradAllReducer:
         self.lo = 0
         self.works = []
         self.n_buckets = 0
+        self.n_allreduce = 0                  # all-reduce calls (one per trainable sub-range of a bucket)
         cuda = engine.device.type == "cuda"
         self.comm_stream = torch.cuda.Stream() if cuda else None
         wire = wire_dtype or os.environ.get("MMSUM_DP_DTYPE", "bf16")
@@ -49,31 +50,44 @@ class GradAllReducer:
         last = hi >= eng.numel
         if hi - self.lo < self.bucket_elems and not last:
             return
-        if self.world() > 1:
-            bucket = eng.G32[self.lo:hi]
+        ranges = self._trainable_ranges(self.lo, hi)
+        if self.world() > 1 and ranges:
             if self.comm_stream is not None:
                 # gradients of this bucket are enqueued on the compute stream; the communication stream picks them up from
                 # there (one event object, re-recorded per bucket: the wait is enqueued before the next record)
                 self._ready_ev.record()
                 self.comm_stream.wait_event(self._ready_ev)
                 with torch.cuda.stream(self.comm_stream):
-                    if self.bf16_wire:
-                        if self.staging is None:
-                            self.staging = torch.empty(eng.numel, device=eng.device, dtype=torch.bfloat16)
-                        wire = self.staging[self.lo:hi]
-                        ops.cast_bf16(bucket, wire)
-                        dist.all_reduce(wire, op=dist.ReduceOp.AVG, group=self.pg)      # stream-ordered on comm_stream
-                        bucket.copy_(wire)
-                    else:
-                        dist.all_reduce(bucket, op=dist.ReduceOp.AVG, group=self.pg)
+                    for lo, r_hi in ranges:
+                        bucket = eng.G32[lo:r_hi]
+                        if self.bf16_wire:
+                            if self.staging is None:
+                                self.staging = torch.empty(eng.numel, device=eng.device, dtype=torch.bfloat16)
+                            wire = self.staging[lo:r_hi]
+                            ops.cast_bf16(bucket, wire)
+                            dist.all_reduce(wire, op=dist.ReduceOp.AVG, group=self.pg)      # stream-ordered on comm_stream
+                            bucket.copy_(wire)
+                        else:
+                            dist.all_reduce(bucket, op=dist.ReduceOp.AVG, group=self.pg)
                 self._pending = True
             else:                                          # gloo (CPU tests): no AVG, no streams
-                w = dist.all_reduce(bucket, op=dist.ReduceOp.SUM, group=self.pg, async_op=True)
-                self.works.append((w, bucket))
+                for lo, r_hi in ranges:
+                    bucket = eng.G32[lo:r_hi]
+                    w = dist.all_reduce(bucket, op=dist.ReduceOp.SUM, group=self.pg, async_op=True)
+                    self.works.append((w, bucket))
+            self.n_allreduce += len(ranges)
         self.n_buckets += 1
         self.lo = hi
         if last:
             self.finish()
+
+    def _trainable_ranges(self, lo, hi):
+        """The parts of arena range [lo, hi) that hold gradients of trainable parameters (adjacent ones merged): frozen ranges
+        are zero on every rank and are not exchanged."""
+        ranges = getattr(self.engine, "grad_ranges", None)
+        if ranges is None:
+            return [(lo, hi)]
+        return [(max(lo, a), min(hi, b)) for a, b in ranges() if a < hi and b > lo]
 
     def finish(self):
         """Make the compute stream wait for every outstanding bucket (no host sync on CUDA)."""

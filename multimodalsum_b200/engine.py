@@ -15,6 +15,7 @@ torch is used for memory (arenas, workspaces), streams and torch.distributed onl
 """
 import math
 import os
+import types
 import weakref
 
 import torch
@@ -67,6 +68,99 @@ def _arena_order(cfg: ModelConfig):
     names += [bm + "encoder.layernorm_embedding.weight", bm + "encoder.layernorm_embedding.bias",
               bm + "encoder.embed_positions.weight", bm + "shared.weight"]
     return names
+
+
+def backward_plan(cfg: ModelConfig, names, trainable):
+    """Which parts of the backward run when only the parameters in `trainable` want a gradient: autograd's rule, a gradient is
+    computed iff it reaches a trainable parameter.  A pure function of the configuration, the arena's parameter names and the
+    trainable set.
+      grads    parameters whose gradient the backward writes (the trainable ones the step reaches)
+      dgrad    activation gradients of the dgrad chain that are computed, by label: "dec.<l>.ffn.dH" (fc2 dgrad), "dec.<l>.ffn.in"
+               (d of the block input), "dec.<l>.cross.dU" / ".dO3" / ".dA3" / ".in", "dec.<l>.self.dctx" / ".in", the same for
+               "enc.<l>.", "head.in" (LM-head dgrad), "table.dtab_h", "table.dtabX"
+      mem      per memory modality: whether its rows of the memory gradient are needed (its producer has a trainable parameter)
+      dkv      per decoder layer: the modalities whose cross-attention dK/dV runs
+      dec_in / enc_in   whether the gradient into layer l's input is needed (index n_layers = the stack's output)"""
+    bm = "bart_model.model."
+    enc, dec, shared = bm + "encoder.", bm + "decoder.", bm + "shared.weight"
+    names = list(names)
+    tset = frozenset(trainable) & frozenset(names)
+    tr = lambda n: n in tset                                           # noqa: E731
+    anyp = lambda *pre: any(n.startswith(pre) for n in tset)            # noqa: E731
+    text, table, image = cfg.text_memory, cfg.table is not None, cfg.image
+    mods = [m for m, on in (("text", text), ("table", table), ("image", image)) if on]
+    mem = {"text": text and (anyp(enc) or tr(shared)), "table": table and anyp("table_encoder."),
+           "image": image and tr("img_encoder.linear.weight")}
+    mem_any = any(mem.values())
+    dgrad = set()
+
+    def ffn(tag, lp, need_in):
+        if tr(lp + "fc1.weight") or tr(lp + "fc1.bias") or need_in:
+            dgrad.add(tag + "ffn.dH")
+        if need_in:
+            dgrad.add(tag + "ffn.in")
+
+    def self_attn(tag, lp, need_in):
+        s = lp + "self_attn."
+        if anyp(s + "q_proj.", s + "k_proj.", s + "v_proj.") or need_in:
+            dgrad.add(tag + "self.dctx")
+        if need_in:
+            dgrad.add(tag + "self.in")
+
+    # decoder: layer l's input gradient is needed when anything trainable lies below it (memory producers included: the
+    # cross-attention dK/dV of the layers below needs the chain)
+    L_d = cfg.decoder_layers
+    dec_in = [tr(shared) or anyp(dec + "embed_positions.", dec + "rating_embeddings", dec + "layernorm_embedding.")]
+    for l in range(L_d):
+        dec_in.append(dec_in[l] or anyp(dec + "layers.%d." % l) or mem_any)
+    dkv = []
+    for l in range(L_d):
+        lp, tag = dec + "layers.%d." % l, "dec.%d." % l
+        c = lp + "encoder_attn."
+        if not dec_in[l + 1]:
+            dkv.append(())
+            continue
+        self_out = dec_in[l] or anyp(lp + "self_attn.", lp + "self_attn_layer_norm.")
+        cross_out = self_out or anyp(c, lp + "encoder_attn_layer_norm.") or mem_any
+        ffn(tag, lp, cross_out)
+        if cross_out:
+            kv = anyp(c + "k_proj.", c + "v_proj.")
+            want = tuple(m for m in mods if kv or mem[m])
+            dA3 = tr(c + "q_proj.weight") or tr(c + "q_proj.bias") or self_out or bool(want)
+            dO3 = tr(c + "out_proj.weight") or tr(c + "out_proj.bias") or dA3
+            if cfg.multimodal and (anyp(c + "alpha_proj.", c + "beta_proj.") or dO3):
+                dgrad.add(tag + "cross.dU")
+            dgrad.update(t for t, on in ((tag + "cross.dO3", dO3), (tag + "cross.dA3", dA3), (tag + "cross.in", self_out)) if on)
+            dkv.append(want if dA3 else ())
+        else:
+            dkv.append(())
+        if self_out:
+            self_attn(tag, lp, dec_in[l])
+    if dec_in[L_d]:
+        dgrad.add("head.in")
+    if mem["table"]:
+        t = "table_encoder."
+        emb = tr(t + "rating_embedding.weight") or tr(t + "hours_embedding.weight") or tr(t + "price_embedding.weight")
+        if anyp(t + "fc.") or emb:
+            dgrad.add("table.dtab_h")
+        if emb:
+            dgrad.add("table.dtabX")
+    # encoder: runs down to the lowest layer with something trainable at or below it (the embeddings count as below layer 0)
+    enc_in = []
+    if mem["text"]:
+        enc_in = [tr(shared) or anyp(enc + "embed_positions.", enc + "layernorm_embedding.")]
+        for l in range(cfg.encoder_layers):
+            enc_in.append(enc_in[l] or anyp(enc + "layers.%d." % l))
+        for l in range(cfg.encoder_layers):
+            lp, tag = enc + "layers.%d." % l, "enc.%d." % l
+            if enc_in[l + 1]:
+                self_out = enc_in[l] or anyp(lp + "self_attn.", lp + "self_attn_layer_norm.")
+                ffn(tag, lp, self_out)
+                if self_out:
+                    self_attn(tag, lp, enc_in[l])
+    grads = frozenset(n for n in tset if text or not n.startswith(enc))
+    return types.SimpleNamespace(trainable=tset, grads=grads, dgrad=frozenset(dgrad), mem=mem, dkv=tuple(dkv),
+                                 dec_in=tuple(dec_in), enc_in=tuple(enc_in), run=dec_in[L_d] or tr(shared))
 
 
 class _Pool:
@@ -139,6 +233,10 @@ class StepEngine:
         self.det_ws = None
         self.det_ws_side = None
         self._det_sized = set()
+        # the parameters that require grad, as read by the last forward, and the backward plan of that set (backward_plan)
+        self.trainable = frozenset()
+        self.plan = None
+        self._plans = {}
         self._graphs = {}
         self._graph_entry = None
         self._w16_fresh = False          # True only right after a fused optimizer wrote W16 itself
@@ -183,6 +281,9 @@ class StepEngine:
                 p.data = v
                 self.params[n] = p
         self.anchor = torch.zeros(1, device=dev, requires_grad=True)
+        self.trainable = frozenset(n for n, p in self.params.items() if p.requires_grad)
+        self._plans = {}
+        self._ln_sink = torch.empty(2, self.cfg.d_model, device=dev, dtype=torch.float32)  # gamma / beta of a half-frozen LayerNorm
         self.step_dev = torch.full((1,), self.step_count, device=dev, dtype=torch.int32)   # dropout step counter, incremented by every forward
         self.bound = True
         self._w16_fresh = False
@@ -251,6 +352,54 @@ class StepEngine:
 
     def mark_weights_dirty(self):
         self._w16_fresh = False
+
+    # ------------------------------------------------------------------ trainable set (requires_grad)
+    def _read_trainable(self):
+        """Read which parameters require grad (at every forward, like the deterministic switch) and select the backward plan of
+        that set.  A parameter that has just been frozen gets its arena range zeroed: nothing writes it afterwards, so the fused
+        clip and the data-parallel buckets see zeros there."""
+        t = frozenset(n for n, p in self.params.items() if p.requires_grad)
+        if t != self.trainable:
+            with torch.no_grad():
+                for n in self.trainable - t:
+                    self.g32(n).zero_()
+            self.trainable = t
+        plan = self._plans.get(t)
+        if plan is None:
+            plan = self._plans[t] = backward_plan(self.cfg, self.names, t)
+            plan.grad_ranges = self._merged_ranges(n for n in self.names if n in t)
+        self.plan = plan
+        return plan
+
+    def _merged_ranges(self, names):
+        out = []
+        for n in names:
+            lo = self.offsets[n]
+            hi = lo + (math.prod(self.shapes[n]) + ALIGN - 1) // ALIGN * ALIGN
+            if out and out[-1][1] == lo:
+                out[-1][1] = hi
+            else:
+                out.append([lo, hi])
+        return [tuple(r) for r in out]
+
+    def grad_ranges(self):
+        """Arena ranges [lo, hi) of the trainable parameters, adjacent ones merged, in arena order (data-parallel buckets)."""
+        return (self.plan or self._read_trainable()).grad_ranges
+
+    def step_anchor(self):
+        """The autograd input of a training step: detached when no parameter requires grad, so the loss does not either (as in
+        torch: its backward() then raises)."""
+        return self.anchor if any(p.requires_grad for p in self.params.values()) else self.anchor.detach()
+
+    def _point_grads(self):
+        """`.grad` of a trainable parameter is its arena view; a frozen parameter's is None."""
+        tset = self.plan.trainable
+        for n, p in self.params.items():
+            if n in tset:
+                if p.grad is None:
+                    p.grad = self.g32(n)
+            elif p.grad is not None:
+                p.grad = None
 
     # ------------------------------------------------------------------ workspaces
     def _frame_view(self, full, S_enc):
@@ -378,13 +527,14 @@ class StepEngine:
                                            dv_col=2 * D)
         return L.self_attn_args(self, qkv, out, lse, key_valid, w["N"], causal, fr, q_rows=(0 if fr == S else fr), **bwd)
 
-    def _cross_attn_args(self, w, qc, kv, out3, lse, dqc=None, dkv=None):
-        """Memory rows = [text B*R*S_enc (leave-one-out over the R reviews of a business) | table B*F | image]."""
+    def _cross_attn_args(self, w, qc, kv, out3, lse, dqc=None, dkv=None, no_dkv=None):
+        """Memory rows = [text B*R*S_enc (leave-one-out over the R reviews of a business) | table B*F | image].  no_dkv (backward):
+        per modality, whether its dK/dV is skipped."""
         D, B, R, F, n_img, Tt = self.cfg.d_model, w["B"], w["R"], w["F"], w["n_img"], w["Tt"]
         mods = ([(0, R, w["S_enc"])] if Tt > 0 else []) + ([(Tt, 1, F)] if F > 0 else []) + \
                ([(Tt + B * F, n_img, w["img_keys"])] if n_img > 0 else [])
         bwd = {} if dqc is None else dict(DELTA=w["delta"], dQ=dqc, lddq=D, dq_col=0, dKV=dkv, lddkv=dkv.stride(0), dk_col=0,
-                                          dv_col=D)
+                                          dv_col=D, no_dkv=no_dkv)
         return L.cross_attn_args(self, qc, kv, out3, lse, mods, w["mem_valid"], w["ent_valid"], w["inv_n"], w["N"], R,
                                  loo=Tt > 0, **bwd)
 
@@ -438,7 +588,8 @@ class StepEngine:
         S_in = batch.reviews.shape[-1] if batch.reviews is not None else 0
         frame = self._encoder_frame(batch, S_in) if self.cfg.text_memory else None
         self.det = torch.are_deterministic_algorithms_enabled()       # (a replay runs no forward(): the mode is read here too)
-        key = (self._batch_key(batch), bool(training), label_smoothing, frame, self.det)
+        plan = self._read_trainable()
+        key = (self._batch_key(batch), bool(training), label_smoothing, frame, plan.trainable, self.det)
         ent = self._graphs.get(key)
         if ent is None:
             if len(self._graphs) >= 4:
@@ -483,9 +634,7 @@ class StepEngine:
                 self.backward(ent["gout"], force_zero=True)
             ent["bwd"] = g
         ent["bwd"].replay()
-        for n, p in self.params.items():
-            if p.grad is None:
-                p.grad = self.g32(n)
+        self._point_grads()
 
     def forward(self, batch, label_smoothing=0.1, training=True, refresh=True):
         """batch: synth.Batch on the device.  Returns the scalar loss tensor (fp32, device)."""
@@ -506,6 +655,7 @@ class StepEngine:
         w = self._alloc(B, R, S, F, n_img, img_keys, S_enc)
         self.ws = w
         self.det = torch.are_deterministic_algorithms_enabled()
+        self._read_trainable()
         if self.det and training:
             self._size_ordered_workspaces()       # before any recorded graph of this shape can need it (backward re-checks)
         T, Tt, Te = w["T"], w["Tt"], w["Te"]
@@ -692,39 +842,84 @@ class StepEngine:
             hi = self.offsets[name_last] + (math.prod(self.shapes[name_last]) + ALIGN - 1) // ALIGN * ALIGN
             self.grad_ready_hook(hi)
 
-    def _ffn_block_bwd(self, w, a, lp, d1, d2, xin, mk, rk, l, kind, enc=False):
-        """Backward of x_out = LN(xin + drop(fc2(gelu(fc1(xin))))).  Returns the two addends of d xin."""
-        pool, pd = (w["pool_e"] if enc else w["pool"]), self.pd
+    def _ln_grads(self, ln):
+        """(dgamma, dbeta) outputs of LayerNorm `ln`: (None, None) when both are frozen (the kernel variant without the reduction);
+        a frozen half of a trainable pair writes into a sink instead of its arena range."""
+        gw, gb = ln + ".weight" in self.plan.grads, ln + ".bias" in self.plan.grads
+        if not gw and not gb:
+            return None, None
+        return (self.g32(ln + ".weight") if gw else self._ln_sink[0]), (self.g32(ln + ".bias") if gb else self._ln_sink[1])
+
+    def _fused_runs(self, names):
+        """Maximal runs [i0, i1) of adjacent members of a fused group (q|k|v, k|v: consecutive in the arena and in the columns of
+        their upstream gradient) whose gradient is computed: one GEMM / column sum per run, nothing written into a frozen member."""
+        runs = []
+        for i, n in enumerate(names):
+            if n in self.plan.grads:
+                if runs and runs[-1][1] == i:
+                    runs[-1][1] = i + 1
+                else:
+                    runs.append([i, i + 1])
+        return runs
+
+    def _fused_grads(self, dy, x, wnames, bnames):
+        """Bias column sums and weight gradients of a fused group over the column slices of dy that belong to trainable members."""
+        D = self.cfg.d_model
+        for i0, i1 in self._fused_runs(bnames):
+            self._bias_grad(dy[:, i0 * D:i1 * D], self.g32(bnames[i0], bnames[i1 - 1]))
+        for i0, i1 in self._fused_runs(wnames):
+            self._wgrad(dy[:, i0 * D:i1 * D], x, wnames[i0], wnames[i1 - 1])
+
+    def _ffn_block_bwd(self, w, a, lp, d1, d2, xin, mk, rk, l, kind, tag, enc=False):
+        """Backward of x_out = LN(xin + drop(fc2(gelu(fc1(xin))))).  Returns the two addends of d xin (None, None when the plan
+        does not need it)."""
+        pool, pd, P = (w["pool_e"] if enc else w["pool"]), self.pd, self.plan
+        need_in = tag + "ffn.in" in P.dgrad
         dres = pool.get()
         df = pool.get() if pd > 0 else dres
-        ops.add_ln_bwd(d1, d2, xin, a["f"], self.w32(lp + "final_layer_norm.weight"), a[mk], a[rk], dres, df,
-                       self.g32(lp + "final_layer_norm.weight"), self.g32(lp + "final_layer_norm.bias"), pd, self.seed,
+        gam, bet = self._ln_grads(lp + "final_layer_norm")
+        ops.add_ln_bwd(d1, d2, xin, a["f"], self.w32(lp + "final_layer_norm.weight"), a[mk], a[rk], dres, df, gam, bet, pd, self.seed,
                        self._sid(kind, l), step_dev=self.step_dev, workspace=self._ows())
         pool.put(d1, d2)
-        self._bias_grad(df, self.g32(lp + "fc2.bias"))
-        self._wgrad(df, a["a"], lp + "fc2.weight")
+        if lp + "fc2.bias" in P.grads:
+            self._bias_grad(df, self.g32(lp + "fc2.bias"))
+        if lp + "fc2.weight" in P.grads:
+            self._wgrad(df, a["a"], lp + "fc2.weight")
         dH = w["dH"][:xin.shape[0]]
-        ops.gemm(df, self.w16(lp + "fc2.weight"), dH, b_t=True, act=ops.ACT_GELU, aux=a["h"], aux_mode=ops.AUX_MUL)
+        if tag + "ffn.dH" in P.dgrad:
+            ops.gemm(df, self.w16(lp + "fc2.weight"), dH, b_t=True, act=ops.ACT_GELU, aux=a["h"], aux_mode=ops.AUX_MUL)
         if df is not dres:
             pool.put(df)
-        self._bias_grad(dH, self.g32(lp + "fc1.bias"))
-        self._wgrad(dH, xin, lp + "fc1.weight")
+        if lp + "fc1.bias" in P.grads:
+            self._bias_grad(dH, self.g32(lp + "fc1.bias"))
+        if lp + "fc1.weight" in P.grads:
+            self._wgrad(dH, xin, lp + "fc1.weight")
+        if not need_in:
+            pool.put(dres)
+            return None, None
         dx = pool.get()
         ops.gemm(dH, self.w16(lp + "fc1.weight"), dx, b_t=True)
         return dres, dx
 
-    def _self_block_bwd(self, w, a, lp, d1, d2, key_valid, causal, l, kind, enc=False):
-        """Backward of x1 = LN(x + drop(out_proj(attn(qkv(x))))).  Returns the two addends of d x."""
-        pool, pd, D = (w["pool_e"] if enc else w["pool"]), self.pd, self.cfg.d_model
+    def _self_block_bwd(self, w, a, lp, d1, d2, key_valid, causal, l, kind, tag, enc=False):
+        """Backward of x1 = LN(x + drop(out_proj(attn(qkv(x))))).  Returns the two addends of d x (None, None when the plan does
+        not need it)."""
+        pool, pd, P = (w["pool_e"] if enc else w["pool"]), self.pd, self.plan
         s = lp + "self_attn."
+        need_in = tag + "self.in" in P.dgrad
         dres = pool.get()
         do = pool.get() if pd > 0 else dres
-        ops.add_ln_bwd(d1, d2, a["x"], a["o"], self.w32(lp + "self_attn_layer_norm.weight"), a["m1"], a["r1"], dres, do,
-                       self.g32(lp + "self_attn_layer_norm.weight"), self.g32(lp + "self_attn_layer_norm.bias"), pd, self.seed,
-                       self._sid(kind, l), step_dev=self.step_dev, workspace=self._ows())
+        gam, bet = self._ln_grads(lp + "self_attn_layer_norm")
+        ops.add_ln_bwd(d1, d2, a["x"], a["o"], self.w32(lp + "self_attn_layer_norm.weight"), a["m1"], a["r1"], dres, do, gam, bet, pd,
+                       self.seed, self._sid(kind, l), step_dev=self.step_dev, workspace=self._ows())
         pool.put(d1, d2)
-        self._bias_grad(do, self.g32(s + "out_proj.bias"))
-        self._wgrad(do, a["ctx"], s + "out_proj.weight")
+        if s + "out_proj.bias" in P.grads:
+            self._bias_grad(do, self.g32(s + "out_proj.bias"))
+        if s + "out_proj.weight" in P.grads:
+            self._wgrad(do, a["ctx"], s + "out_proj.weight")
+        if tag + "self.dctx" not in P.dgrad:
+            pool.put(do, dres)
+            return None, None
         dctx = pool.get()
         ops.gemm(do, self.w16(s + "out_proj.weight"), dctx, b_t=True)
         if do is not dres:
@@ -732,14 +927,23 @@ class StepEngine:
         dqkv = w["dqkv"][:a["qkv"].shape[0]]
         ops.attn_bwd(self._self_attn_args(w, a["qkv"], dctx, a["lse"], key_valid, causal, dqkv=dqkv, frame=w["S_enc"] if enc else None))
         pool.put(dctx)
-        self._bias_grad(dqkv, self.g32(s + "q_proj.bias", s + "v_proj.bias"))
-        self._wgrad(dqkv, a["x"], s + "q_proj.weight", s + "v_proj.weight")
+        self._fused_grads(dqkv, a["x"], [s + "q_proj.weight", s + "k_proj.weight", s + "v_proj.weight"],
+                          [s + "q_proj.bias", s + "k_proj.bias", s + "v_proj.bias"])
+        if not need_in:
+            pool.put(dres)
+            return None, None
         dx = pool.get()
         ops.gemm(dqkv, self.w16(s + "q_proj.weight", s + "v_proj.weight"), dx, b_t=True)
         return dres, dx
 
+    def _mem_rows(self, w, m):
+        Tt, BF = w["Tt"], w["B"] * w["F"]
+        return {"text": (0, Tt), "table": (Tt, Tt + BF), "image": (Tt + BF, w["Tm"])}[m]
+
     def backward(self, grad_out=None, force_zero=False):
-        """Writes every parameter gradient into the fp32 gradient arena (+=) and points `.grad` at it."""
+        """Writes the gradient of every trainable parameter into the fp32 gradient arena (+=) and points its `.grad` at it.  Runs
+        the backward plan (backward_plan) of the trainable set the forward read: a frozen parameter's range is never written and
+        its `.grad` is None; what only frozen parameters need is not computed."""
         cfg, w = self.cfg, self.ws
         if w is None:
             raise RuntimeError("backward() without a forward()")
@@ -750,109 +954,164 @@ class StepEngine:
         pool, pd, seed = w["pool"], self.pd, self.seed
         bm = "bart_model.model."
         g = ops.gemm
+        P = self.plan
+        grads, dgrad = P.grads, P.dgrad
         if self.det:
             self._size_ordered_workspaces()
-        first = next(iter(self.params.values()))
-        if force_zero or first.grad is None:
+        first = next((p for n, p in self.params.items() if n in P.trainable), None)
+        if force_zero or (first is not None and first.grad is None):
             self.G32.zero_()
         # ---- loss + LM head
         logits = w["logits"]
-        ops.ce_fwd_bwd(logits, V, w["labels"], self.label_smoothing, 1.0 / T, grad_out, w["loss_rows"], None, 0.0, True,
-                       lse_rows=w["lse_rows"])
+        if P.run:
+            ops.ce_fwd_bwd(logits, V, w["labels"], self.label_smoothing, 1.0 / T, grad_out, w["loss_rows"], None, 0.0, True,
+                           lse_rows=w["lse_rows"])
         dl = logits[:, :V]
-        d1 = pool.get()
-        g(dl, self.w16(bm + "shared.weight"), d1, b_t=True)
+        d1 = d2 = None
+        if "head.in" in dgrad:
+            d1 = pool.get()
+            g(dl, self.w16(bm + "shared.weight"), d1, b_t=True)
         xfin = w["x_out"]
-        ops.gemm(dl, xfin, self.g32(bm + "shared.weight"), a_t=True, b_t=True, accumulate=True, workspace=self._ows())
-        d2 = None
+        if bm + "shared.weight" in grads:
+            ops.gemm(dl, xfin, self.g32(bm + "shared.weight"), a_t=True, b_t=True, accumulate=True, workspace=self._ows())
 
         # ---- decoder layers, last to first
         pre = bm + "decoder."
+        mem_any = any(P.mem.values())
         for l in reversed(range(cfg.decoder_layers)):
             a = w["dec"][l]
             lp = pre + "layers.%d." % l
             c = lp + "encoder_attn."
-            d1, d2 = self._ffn_block_bwd(w, a, lp, d1, d2, a["x2"], "m3", "r3", l, 6)
-            # cross block
-            dres = pool.get()
-            yc = a["yc"] if gates else a["O3"][0]
-            dyc = pool.get() if pd > 0 else dres
-            ops.add_ln_bwd(d1, d2, a["x1"], yc, self.w32(lp + "encoder_attn_layer_norm.weight"), a["m2"], a["r2"], dres, dyc,
-                           self.g32(lp + "encoder_attn_layer_norm.weight"), self.g32(lp + "encoder_attn_layer_norm.bias"),
-                           pd, seed, self._sid(5, l), step_dev=self.step_dev, workspace=self._ows())
-            pool.put(d1, d2)
-            nm = a["A3"].shape[0]
-            if gates:
-                dU, dO3 = w["dU"], w["dO3"]
-                ops.gate_bwd_u(dyc, a["O3"], a["AB"], dU, T, D)
-                self._bias_grad(dU[0], self.g32(c + "alpha_proj.bias"))
-                self._bias_grad(dU[1], self.g32(c + "beta_proj.bias"))
-                self._wgrad(dU[0], a["O3"][0], c + "alpha_proj.weight", col_slice=(0, D))
-                self._wgrad(dU[0], a["O3"][1], c + "alpha_proj.weight", col_slice=(D, 2 * D))
-                self._wgrad(dU[1], a["O3"][0], c + "beta_proj.weight", col_slice=(0, D))
-                self._wgrad(dU[1], a["O3"][2], c + "beta_proj.weight", col_slice=(D, 2 * D))
-                g(dU[0], self.w16(c + "alpha_proj.weight"), w["dca"], b_t=True)
-                g(dU[1], self.w16(c + "beta_proj.weight"), w["dcb"], b_t=True)
-                ops.gate_bwd_o(dyc, a["AB"], w["dca"], w["dcb"], dO3, T, D)
-                dO3f = dO3.view(nm * T, D)
-            else:
-                dO3f = dyc
-            self._bias_grad(dO3f, self.g32(c + "out_proj.bias"))
-            self._wgrad(dO3f, a["A3"].view(nm * T, D), c + "out_proj.weight")
-            dA3 = w["dA3"]
-            g(dO3f, self.w16(c + "out_proj.weight"), dA3.view(nm * T, D), b_t=True)
-            if dyc is not dres:
-                pool.put(dyc)
-            dqc = pool.get()
-            dkv = w["dkv_all"][:, l * 2 * D:(l + 1) * 2 * D]
-            ops.attn_bwd(self._cross_attn_args(w, a["qc"], a["kv"], dA3, a["lse_c"], dqc, dkv))
-            self._bias_grad(dqc, self.g32(c + "q_proj.bias"))
-            self._wgrad(dqc, a["x1"], c + "q_proj.weight")
-            dx1 = pool.get()
-            g(dqc, self.w16(c + "q_proj.weight"), dx1, b_t=True)
-            pool.put(dqc)
-            self._bias_grad(dkv, self.g32(c + "k_proj.bias", c + "v_proj.bias"))
-            self._wgrad(dkv, w["MEM"], c + "k_proj.weight", c + "v_proj.weight")
-            w["Wkv_cat"][l * 2 * D:(l + 1) * 2 * D].copy_(self.w16(c + "k_proj.weight", c + "v_proj.weight"))
-            # self block
-            d1, d2 = self._self_block_bwd(w, a, lp, dres, dx1, w["dec_valid"], True, l, 4)
+            tag = "dec.%d." % l
+            if not P.dec_in[l + 1]:
+                self._ready(lp + "self_attn_layer_norm.bias")
+                continue
+            d1, d2 = self._ffn_block_bwd(w, a, lp, d1, d2, a["x2"], "m3", "r3", l, 6, tag)
+            if tag + "ffn.in" in dgrad:
+                # cross block
+                dres = pool.get()
+                yc = a["yc"] if gates else a["O3"][0]
+                dyc = pool.get() if pd > 0 else dres
+                gam, bet = self._ln_grads(lp + "encoder_attn_layer_norm")
+                ops.add_ln_bwd(d1, d2, a["x1"], yc, self.w32(lp + "encoder_attn_layer_norm.weight"), a["m2"], a["r2"], dres, dyc,
+                               gam, bet, pd, seed, self._sid(5, l), step_dev=self.step_dev, workspace=self._ows())
+                pool.put(d1, d2)
+                nm = a["A3"].shape[0]
+                dO3_on, dA3_on = tag + "cross.dO3" in dgrad, tag + "cross.dA3" in dgrad
+                if gates:
+                    dU, dO3 = w["dU"], w["dO3"]
+                    if tag + "cross.dU" in dgrad:
+                        ops.gate_bwd_u(dyc, a["O3"], a["AB"], dU, T, D)
+                    if c + "alpha_proj.bias" in grads:
+                        self._bias_grad(dU[0], self.g32(c + "alpha_proj.bias"))
+                    if c + "beta_proj.bias" in grads:
+                        self._bias_grad(dU[1], self.g32(c + "beta_proj.bias"))
+                    if c + "alpha_proj.weight" in grads:
+                        self._wgrad(dU[0], a["O3"][0], c + "alpha_proj.weight", col_slice=(0, D))
+                        self._wgrad(dU[0], a["O3"][1], c + "alpha_proj.weight", col_slice=(D, 2 * D))
+                    if c + "beta_proj.weight" in grads:
+                        self._wgrad(dU[1], a["O3"][0], c + "beta_proj.weight", col_slice=(0, D))
+                        self._wgrad(dU[1], a["O3"][2], c + "beta_proj.weight", col_slice=(D, 2 * D))
+                    if dO3_on:
+                        g(dU[0], self.w16(c + "alpha_proj.weight"), w["dca"], b_t=True)
+                        g(dU[1], self.w16(c + "beta_proj.weight"), w["dcb"], b_t=True)
+                        ops.gate_bwd_o(dyc, a["AB"], w["dca"], w["dcb"], dO3, T, D)
+                    dO3f = dO3.view(nm * T, D)
+                else:
+                    dO3f = dyc
+                if c + "out_proj.bias" in grads:
+                    self._bias_grad(dO3f, self.g32(c + "out_proj.bias"))
+                if c + "out_proj.weight" in grads:
+                    self._wgrad(dO3f, a["A3"].view(nm * T, D), c + "out_proj.weight")
+                dA3 = w["dA3"]
+                if dA3_on:
+                    g(dO3f, self.w16(c + "out_proj.weight"), dA3.view(nm * T, D), b_t=True)
+                if dyc is not dres:
+                    pool.put(dyc)
+                need_x1 = tag + "cross.in" in dgrad
+                dx1 = None
+                if dA3_on:
+                    dqc = pool.get()
+                    dkv = w["dkv_all"][:, l * 2 * D:(l + 1) * 2 * D]
+                    mods = [m for m, on in (("text", Tt > 0), ("table", F > 0), ("image", n_img > 0)) if on]
+                    ops.attn_bwd(self._cross_attn_args(w, a["qc"], a["kv"], dA3, a["lse_c"], dqc, dkv,
+                                                       no_dkv=[m not in P.dkv[l] for m in mods]))
+                    if c + "q_proj.bias" in grads:
+                        self._bias_grad(dqc, self.g32(c + "q_proj.bias"))
+                    if c + "q_proj.weight" in grads:
+                        self._wgrad(dqc, a["x1"], c + "q_proj.weight")
+                    if need_x1:
+                        dx1 = pool.get()
+                        g(dqc, self.w16(c + "q_proj.weight"), dx1, b_t=True)
+                    pool.put(dqc)
+                    self._fused_grads(dkv, w["MEM"], [c + "k_proj.weight", c + "v_proj.weight"], [c + "k_proj.bias", c + "v_proj.bias"])
+                if mem_any:
+                    w["Wkv_cat"][l * 2 * D:(l + 1) * 2 * D].copy_(self.w16(c + "k_proj.weight", c + "v_proj.weight"))
+                if need_x1:
+                    # self block
+                    d1, d2 = self._self_block_bwd(w, a, lp, dres, dx1, w["dec_valid"], True, l, 4, tag)
+                else:
+                    pool.put(dres)
+                    d1, d2 = None, None
             self._ready(lp + "self_attn_layer_norm.bias")
         # decoder embedding
-        ops.embed_ln_bwd(d1, d2, w["dec_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"),
-                         w["rating_diff"], self.w32(pre + "rating_embeddings"), self.w32(pre + "layernorm_embedding.weight"),
-                         w["dec_m0"], w["dec_r0"], self.g32(bm + "shared.weight"), self.g32(pre + "embed_positions.weight"),
-                         self.g32(pre + "rating_embeddings"), self.g32(pre + "layernorm_embedding.weight"),
-                         self.g32(pre + "layernorm_embedding.bias"), w["dz32"], T, S, cfg.pad_token_id, pd, seed, self._sid(3, 0), step_dev=self.step_dev,
-                         workspace=self._ows())
-        pool.put(d1, d2)
+        if P.dec_in[0]:
+            opt = lambda n: self.g32(n) if n in grads else None        # noqa: E731
+            gam, bet = self._ln_grads(pre + "layernorm_embedding")
+            ops.embed_ln_bwd(d1, d2, w["dec_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"),
+                             w["rating_diff"], self.w32(pre + "rating_embeddings"), self.w32(pre + "layernorm_embedding.weight"),
+                             w["dec_m0"], w["dec_r0"], opt(bm + "shared.weight"), opt(pre + "embed_positions.weight"),
+                             opt(pre + "rating_embeddings"), gam, bet, w["dz32"], T, S, cfg.pad_token_id, pd, seed, self._sid(3, 0),
+                             step_dev=self.step_dev, workspace=self._ows())
+            pool.put(d1, d2)
         self._ready(pre + "embed_positions.weight")
 
-        # ---- memory gradients: table, image, text
+        # ---- memory gradients: table, image, text (only the rows of modalities whose producer has a trainable parameter)
         dMEM = w["dMEM16"]
-        g(w["dkv_all"], w["Wkv_cat"], dMEM, b_t=True)
+        runs = []
+        for m in ("text", "table", "image"):
+            if P.mem[m]:
+                r0, r1 = self._mem_rows(w, m)
+                if runs and runs[-1][1] == r0:
+                    runs[-1][1] = r1
+                else:
+                    runs.append([r0, r1])
+        for r0, r1 in runs:
+            g(w["dkv_all"][r0:r1], w["Wkv_cat"], dMEM[r0:r1], b_t=True)
         if F > 0:
             t = "table_encoder."
-            dtab = dMEM[Tt:Tt + B * F]
-            self._wgrad(dtab, w["tab_h"], t + "linear.weight")
-            g(dtab, self.w16(t + "linear.weight"), w["dtab_h"], b_t=True, act=ops.ACT_RELU, aux=w["tab_h"], aux_mode=ops.AUX_MUL_DACT)
-            self._bias_grad(w["dtab_h"], self.g32(t + "fc.bias"))
-            self._wgrad(w["dtab_h"], w["tabX"], t + "fc.weight")
-            g(w["dtab_h"], self.w16(t + "fc.weight"), w["dtabX"], b_t=True)
-            batch = w["batch"]
-            if cfg.table == "yelp":
-                ops.table_bits_bwd(w["dtabX"], batch.field_value[4], self.g32(t + "rating_embedding.weight"), B, F, 39, 1, 4)
-                ops.table_bits_bwd(w["dtabX"], batch.field_value[5], self.g32(t + "hours_embedding.weight"), B, F, 40, 7, 4)
-            else:
-                ops.table_bits_bwd(w["dtabX"], batch.field_value[0], self.g32(t + "price_embedding.weight"), B, F, 0, 1, 11)
-                ops.table_bits_bwd(w["dtabX"], batch.field_value[1], self.g32(t + "rating_embedding.weight"), B, F, 1, 1, 4)
+            if P.mem["table"]:
+                dtab = dMEM[Tt:Tt + B * F]
+                if t + "linear.weight" in grads:
+                    self._wgrad(dtab, w["tab_h"], t + "linear.weight")
+                if "table.dtab_h" in dgrad:
+                    g(dtab, self.w16(t + "linear.weight"), w["dtab_h"], b_t=True, act=ops.ACT_RELU, aux=w["tab_h"],
+                      aux_mode=ops.AUX_MUL_DACT)
+                if t + "fc.bias" in grads:
+                    self._bias_grad(w["dtab_h"], self.g32(t + "fc.bias"))
+                if t + "fc.weight" in grads:
+                    self._wgrad(w["dtab_h"], w["tabX"], t + "fc.weight")
+                if "table.dtabX" in dgrad:
+                    g(w["dtab_h"], self.w16(t + "fc.weight"), w["dtabX"], b_t=True)
+                batch = w["batch"]
+                if cfg.table == "yelp":
+                    bits = ((batch.field_value[4], t + "rating_embedding.weight", 39, 1, 4),
+                            (batch.field_value[5], t + "hours_embedding.weight", 40, 7, 4))
+                else:
+                    bits = ((batch.field_value[0], t + "price_embedding.weight", 0, 1, 11),
+                            (batch.field_value[1], t + "rating_embedding.weight", 1, 1, 4))
+                for v, n, f0, nrows, nb in bits:
+                    if n in grads:
+                        ops.table_bits_bwd(w["dtabX"], v, self.g32(n), B, F, f0, nrows, nb)
             if n_img == 0:
                 self._ready(t + ("hours_embedding.weight" if cfg.table == "yelp" else "price_embedding.weight"))
         if n_img > 0:
-            self._wgrad(dMEM[Tt + B * F:], w["img_in"], "img_encoder.linear.weight")
+            if "img_encoder.linear.weight" in grads:
+                self._wgrad(dMEM[Tt + B * F:], w["img_in"], "img_encoder.linear.weight")
             self._ready("img_encoder.linear.weight")
 
-        # ---- encoder layers, last to first (the img / table stages have no text memory: encoder gradients stay zero)
-        if Tt > 0:
+        # ---- encoder layers, last to first, down to the lowest one the plan needs (the img / table stages have no text memory)
+        if Tt > 0 and P.mem["text"]:
             pre = bm + "encoder."
             Te, S_enc, pool = w["Te"], w["S_enc"], w["pool_e"]
             d1 = pool.get()
@@ -861,16 +1120,19 @@ class StepEngine:
             for l in reversed(range(cfg.encoder_layers)):
                 a = w["enc"][l]
                 lp = pre + "layers.%d." % l
-                d1, d2 = self._ffn_block_bwd(w, a, lp, d1, d2, a["x1"], "m2", "r2", l, 2, enc=True)
-                d1, d2 = self._self_block_bwd(w, a, lp, d1, d2, w["enc_valid"], False, l, 1, enc=True)
+                if P.enc_in[l + 1]:
+                    tag = "enc.%d." % l
+                    d1, d2 = self._ffn_block_bwd(w, a, lp, d1, d2, a["x1"], "m2", "r2", l, 2, tag, enc=True)
+                    if tag + "ffn.in" in dgrad:
+                        d1, d2 = self._self_block_bwd(w, a, lp, d1, d2, w["enc_valid"], False, l, 1, tag, enc=True)
                 self._ready(lp + "self_attn_layer_norm.bias")
-            ops.embed_ln_bwd(d1, d2, w["enc_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"), None, None,
-                             self.w32(pre + "layernorm_embedding.weight"), w["enc_m0"], w["enc_r0"], self.g32(bm + "shared.weight"),
-                             self.g32(pre + "embed_positions.weight"), None, self.g32(pre + "layernorm_embedding.weight"),
-                             self.g32(pre + "layernorm_embedding.bias"), w["dz32"], Te, S_enc, cfg.pad_token_id, pd, seed, self._sid(0, 0), step_dev=self.step_dev,
-                             workspace=self._ows())
-            pool.put(d1, d2)
+            if P.enc_in[0]:
+                opt = lambda n: self.g32(n) if n in grads else None    # noqa: E731
+                gam, bet = self._ln_grads(pre + "layernorm_embedding")
+                ops.embed_ln_bwd(d1, d2, w["enc_ids"], self.w32(bm + "shared.weight"), self.w32(pre + "embed_positions.weight"), None,
+                                 None, self.w32(pre + "layernorm_embedding.weight"), w["enc_m0"], w["enc_r0"],
+                                 opt(bm + "shared.weight"), opt(pre + "embed_positions.weight"), None, gam, bet, w["dz32"], Te, S_enc,
+                                 cfg.pad_token_id, pd, seed, self._sid(0, 0), step_dev=self.step_dev, workspace=self._ows())
+                pool.put(d1, d2)
         self._ready(bm + "shared.weight")
-        for n, p in self.params.items():
-            if p.grad is None:
-                p.grad = self.g32(n)
+        self._point_grads()

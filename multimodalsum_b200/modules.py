@@ -427,7 +427,7 @@ class MultimodalSum(nn.Module, _EngineRoot):
         batch = Batch(_ids(reviews), _ids(reviews_mask), reviews_rating.float().contiguous(), _ids(field),
                       [_ids(v) for v in field_value], img if img.dtype == torch.bfloat16 else img.float(),
                       img_mask.to(torch.bool).contiguous(), max_review_len=max_review_len)
-        loss = _StepFn.apply(eng.anchor, self, batch, self.label_smoothing)
+        loss = _StepFn.apply(eng.step_anchor(), self, batch, self.label_smoothing)
         return (loss,)
 
     @torch.no_grad()
@@ -470,7 +470,7 @@ class TextSupervised(nn.Module, _EngineRoot):
         if max_review_len is None:
             max_review_len = getattr(reviews_mask, "max_review_len", None)      # attached by prefetch.text_data_prefetcher
         batch = Batch(_ids(reviews), _ids(reviews_mask), reviews_rating.float().contiguous(), max_review_len=max_review_len)
-        loss = _StepFn.apply(eng.anchor, self, batch, self.label_smoothing)
+        loss = _StepFn.apply(eng.step_anchor(), self, batch, self.label_smoothing)
         return (loss,)
 
 
@@ -504,7 +504,7 @@ class ImgSupervised(nn.Module, _EngineRoot):
         _check_device(input_imgs.device, mask, labels)
         batch = Batch(None, None, None, img=input_imgs if input_imgs.dtype == torch.bfloat16 else input_imgs.float(),
                       img_mask=mask.to(torch.bool).contiguous(), labels=_ids(labels))
-        return (_StepFn.apply(eng.anchor, self, batch, self.label_smoothing),)
+        return (_StepFn.apply(eng.step_anchor(), self, batch, self.label_smoothing),)
 
 
 class TableSupervised(nn.Module, _EngineRoot):
@@ -533,4 +533,4 @@ class TableSupervised(nn.Module, _EngineRoot):
         eng = self._ensure_engine(field.device)
         _check_device(field.device, labels, *field_value)
         batch = Batch(None, None, None, field=_ids(field), field_value=[_ids(v) for v in field_value], labels=_ids(labels))
-        return (_StepFn.apply(eng.anchor, self, batch, self.label_smoothing),)
+        return (_StepFn.apply(eng.step_anchor(), self, batch, self.label_smoothing),)

@@ -187,19 +187,31 @@ def _embed_ln_fwd(ids, E, P, rating_diff, remb, gamma, beta, out, mean, rstd, ro
 
 def embed_ln_bwd(dout, dout2, ids, E, P, rating_diff, remb, gamma, mean, rstd, dE, dP, dremb, dgamma, dbeta, dz, rows, S,
                  pad_id, p_drop, seed, sid, step_dev=None, workspace=None):
-    """workspace (fp32, >= embed_ln_bwd_workspace(rows, S, E.shape[0]) elements): the ordered variant (bitwise reproducible)."""
+    """workspace (fp32, >= embed_ln_bwd_workspace(rows, S, E.shape[0]) elements): the ordered variant (bitwise reproducible).
+    Each of dE, dP, dremb and the pair dgamma / dbeta may be None (frozen): not computed; with all of them None nothing runs."""
+    want_remb = rating_diff is not None and dremb is not None
+    if dE is None and dP is None and dgamma is None and not want_remb:
+        return
+    full = dE is not None and dP is not None and dgamma is not None and (rating_diff is None or dremb is not None)
     if workspace is not None:
         ORDERED_CALLS["embed_ln_bwd"] += 1
-        _timed("embed_ln_bwd_ordered", rows * E.shape[1] * 12.0, lambda: check(_lib.lib().mmsum_embed_ln_bwd_ordered(
+        n = 6 if rating_diff is not None else 5
+        fn, name = _lib.lib().mmsum_embed_ln_bwd_ordered, "mmsum_embed_ln_bwd_ordered"
+        if not full:
+            fn, name = _lib.lib().mmsum_embed_ln_bwd_ordered_subset, "mmsum_embed_ln_bwd_ordered_subset"
+            n -= (3 if dE is None else 0) + (1 if dgamma is None else 0) + (1 if dP is None and not want_remb else 0) + \
+                (1 if rating_diff is not None and dremb is None else 0)
+        _timed("embed_ln_bwd_ordered", rows * E.shape[1] * 12.0, lambda: check(fn(
             _ptr(dout), _ptr(dout2), _ptr(ids), _ptr(E), _ptr(P), _ptr(rating_diff), _ptr(remb), _ptr(gamma), _ptr(mean),
             _ptr(rstd), _ptr(dE), _ptr(dP), _ptr(dremb), _ptr(dgamma), _ptr(dbeta), _ptr(dz), rows, S, E.shape[1], pad_id,
             C.c_float(p_drop), C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), E.shape[0], _ptr(workspace),
-            C.c_int64(workspace.numel()), _stream()), "mmsum_embed_ln_bwd_ordered", 6 if rating_diff is not None else 5))
+            C.c_int64(workspace.numel()), _stream()), name, n))
         return
     check(_lib.lib().mmsum_embed_ln_bwd(_ptr(dout), _ptr(dout2), _ptr(ids), _ptr(E), _ptr(P), _ptr(rating_diff), _ptr(remb),
                                         _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dE), _ptr(dP), _ptr(dremb), _ptr(dgamma),
                                         _ptr(dbeta), _ptr(dz), rows, S, E.shape[1], pad_id, C.c_float(p_drop),
-                                        C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), _stream()), "mmsum_embed_ln_bwd", 2)
+                                        C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), _stream()), "mmsum_embed_ln_bwd",
+          2 if dP is not None or want_remb else 1)
 
 
 def add_ln_fwd(res, y, gamma, beta, out, mean, rstd, p_drop, seed, sid, step_dev=None):
@@ -214,7 +226,8 @@ def _add_ln_fwd(res, y, gamma, beta, out, mean, rstd, p_drop, seed, sid, step_de
 
 
 def add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_drop, seed, sid, step_dev=None, workspace=None):
-    """workspace (fp32, >= ADD_LN_BWD_WORKSPACE elements): the ordered variant (bitwise reproducible)."""
+    """workspace (fp32, >= ADD_LN_BWD_WORKSPACE elements): the ordered variant (bitwise reproducible).  dgamma = dbeta = None
+    (a frozen LayerNorm): the variant without the gamma / beta reduction."""
     rows, d = res.shape
     n_mats = 3 + (1 if d2 is not None else 0) + 1 + (1 if dy.data_ptr() != dres.data_ptr() else 0)   # d1 (+d2), res, y in; dres (+dy) out
     if workspace is not None:
@@ -222,7 +235,7 @@ def add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_dro
         _timed("add_ln_bwd_ordered", float(n_mats) * rows * d * 2, lambda: check(_lib.lib().mmsum_add_ln_bwd_ordered(
             _ptr(d1), _ptr(d2), _ptr(res), _ptr(y), _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dres), _ptr(dy), _ptr(dgamma),
             _ptr(dbeta), rows, d, C.c_float(p_drop), C.c_uint64(seed), C.c_uint32(sid), _ptr(step_dev), _ptr(workspace),
-            C.c_int64(workspace.numel()), _stream()), "mmsum_add_ln_bwd_ordered", 2))
+            C.c_int64(workspace.numel()), _stream()), "mmsum_add_ln_bwd_ordered", 2 if dgamma is not None else 1))
         return
     _timed("add_ln_bwd", float(n_mats) * rows * d * 2, lambda: _add_ln_bwd(d1, d2, res, y, gamma, mean, rstd, dres, dy, dgamma, dbeta, p_drop, seed, sid, step_dev))
 
@@ -291,8 +304,10 @@ def _ce_fwd_bwd(logits, V, target, eps, gscale, gscale_dev, loss_rows, loss_out,
 
 
 def attn_args(**kw):
+    """no_dkv (optional, one flag per modality): the backward skips that modality's dK/dV (see MmsumAttnMod)."""
     a = _lib.AttnArgs()
     mods = kw.pop("mods")
+    no_dkv = kw.pop("no_dkv", None)
     for k, v in kw.items():
         if isinstance(v, torch.Tensor):
             v = v.data_ptr()
@@ -301,6 +316,7 @@ def attn_args(**kw):
     for i, m in enumerate(mods):
         a.mods[i].kv_row_base, a.mods[i].o_off, a.mods[i].E, a.mods[i].Sk, a.mods[i].loo, a.mods[i].ent_base = m[:6]
         a.mods[i].ent_stride = m[6] if len(m) > 6 else 0
+        a.mods[i].no_dkv = int(bool(no_dkv[i])) if no_dkv is not None else 0
     return a
 
 
@@ -320,9 +336,11 @@ def attn_fwd(a):
 
 
 def attn_bwd(a):
-    # backward = 2.5 x forward algorithmic FLOPs (S, dP, dQ, dK, dV products; SURVEY App. H); two kernels (dQ, then dK/dV)
+    # backward = 2.5 x forward algorithmic FLOPs (S, dP, dQ, dK, dV products; SURVEY App. H); two kernels (dQ, then dK/dV; the
+    # second is not launched when no modality wants dK/dV)
     kind = "attn_self_bwd" if a.n_mod == 1 and a.mods[0].E == 1 else "attn_cross_bwd"
-    _timed(kind, 2.5 * attn_flops(a), lambda: check(_lib.lib().mmsum_attn_bwd(C.byref(a), _stream()), "mmsum_attn_bwd", 2))
+    n = 1 if all(a.mods[i].no_dkv for i in range(a.n_mod)) else 2
+    _timed(kind, 2.5 * attn_flops(a), lambda: check(_lib.lib().mmsum_attn_bwd(C.byref(a), _stream()), "mmsum_attn_bwd", n))
 
 
 def debug_poison():

@@ -14,7 +14,10 @@ from .engine import ALIGN
 
 class FusedAdamW:
     """param_groups: [{'params': [Parameter...], 'weight_decay': float}, ...] exactly as the reference builds them.
-    Parameters that appear in no group are never updated (this is how quirk Q1 manifests in the reference)."""
+    Parameters that appear in no group are never updated (this is how quirk Q1 manifests in the reference).  A frozen parameter
+    (requires_grad=False when the engine's last forward ran) is skipped as torch / transformers AdamW skip a None grad: no update,
+    no weight decay, moments unchanged.  The step count is shared, so a parameter of the groups whose trainability changes after
+    the first step raises ValueError."""
 
     def __init__(self, engine, param_groups, lr=1e-5, betas=(0.9, 0.999), eps=1e-6, weight_decay=0.0, correct_bias=True,
                  max_grad_norm=None):
@@ -33,6 +36,7 @@ class FusedAdamW:
         flags = torch.zeros(n // ALIGN, dtype=torch.uint8)
         by_id = {id(p): name for name, p in engine.params.items()}
         wds = set()
+        self._names = []
         for g in self.param_groups:
             wd = float(g.get("weight_decay", weight_decay))
             for p in g["params"]:
@@ -42,13 +46,35 @@ class FusedAdamW:
                 lo = engine.offsets[name] // ALIGN
                 hi = lo + (math.prod(engine.shapes[name]) + ALIGN - 1) // ALIGN
                 flags[lo:hi] = 1 | (2 if wd > 0 else 0)
+                self._names.append(name)
                 if wd > 0:
                     wds.add(wd)
         if len(wds) > 1:
             raise ValueError("one non-zero weight_decay value supported")
         self.weight_decay = wds.pop() if wds else 0.0
-        self.flags = flags.to(dev)
+        self._group_flags = flags
+        self._trainable = None                # the engine's trainable set the device flags were computed for
         self.step_count = 0
+        self._sync_flags()
+
+    def _sync_flags(self):
+        """Clear the update flags of frozen parameters (recomputed when the engine's trainable set changes)."""
+        eng = self.engine
+        t = eng.trainable
+        if t == self._trainable:
+            return
+        if self._trainable is not None and self.step_count > 0:
+            changed = sorted(n for n in self._names if (n in t) != (n in self._trainable))
+            if changed:
+                raise ValueError("requires_grad of %s changed after the first step; the fused optimizer keeps one step count for "
+                                 "all its parameters (build a new optimizer, or use a torch optimizer)" % changed[:3])
+        flags = self._group_flags.clone()
+        for name in self._names:
+            if name not in t:
+                lo = eng.offsets[name] // ALIGN
+                flags[lo:lo + (math.prod(eng.shapes[name]) + ALIGN - 1) // ALIGN] = 0
+        self.flags = flags.to(eng.device)
+        self._trainable = t
 
     def zero_grad(self, set_to_none=True):
         for p in self.engine.params.values():
@@ -64,6 +90,7 @@ class FusedAdamW:
             if len(lrs) > 1:
                 raise ValueError("parameter groups with different learning rates are not supported by the fused step")
             lr = lrs.pop() if lrs else self.lr
+        self._sync_flags()
         self.step_count += 1
         b1, b2 = self.betas
         step_size = lr
@@ -97,7 +124,7 @@ class FusedAdamW:
             for p in g["params"]:
                 name = by_id[id(p)]
                 o, n = eng.offsets[name], math.prod(eng.shapes[name])
-                if self.step_count > 0:
+                if self.step_count > 0 and name in self._trainable:      # a frozen parameter was never updated: no state
                     state[idx] = {"step": self.step_count, "exp_avg": self.m[o:o + n].view(eng.shapes[name]).detach().cpu().clone(),
                                   "exp_avg_sq": self.v[o:o + n].view(eng.shapes[name]).detach().cpu().clone()}
                 ids.append(idx)
